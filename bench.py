@@ -9,6 +9,7 @@ fixed, no data-path collective).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # product (CUDA, libort_b200.so)
     python bench.py --impl reference [...]                         # the reference's own CPU sse_trace
+    python bench.py [...] --dump-outputs DIR                       # also write the last timed step's outputs (sampled)
 
 One JSON line on stdout (rank 0).  `value`: device-resident throughput (outputs stay in HBM; L2 is
 flushed before every step).  `parity`: the timed frames against the CPU checker, in the same run.
@@ -435,6 +436,19 @@ def run_product(args):
     parity = None
     if args.launch == "streams" and not args.no_cpu:
         parity = parity_of_timed_frames(ort, tree, n_up, ctx, mg, world, rank, outs, NS, len(step_cams), cams, frame_rows, torch, dist)
+    if args.dump_outputs and rank == 0:
+        # the timed loop's output buffers still hold the last step: every frame with the batched launch, else frame k of the
+        # step in buffer k % NS for the last k of each residue (with N > 1, this rank's strip rows of those frames)
+        n_step = len(step_cams)
+        held = list(enumerate(batch_outs)) if args.launch == "batch" else \
+            [(max(k for k in range(n_step) if k % NS == j), outs[j]) for j in range(min(NS, n_step))]
+
+        def take(buf):
+            def rows(idx):
+                sel = torch.from_numpy(idx).cuda()
+                return buf[0][sel].cpu().numpy().view(np.uint32), buf[1][sel].cpu().numpy(), buf[2][sel].cpu().numpy()
+            return rows
+        dump_outputs(args.dump_outputs, [(f"frame{k}_pose{POSE_NAMES[k % len(cams)]}", take(buf)) for k, buf in held], n_local)
 
     # per-launch view of the same work: serialised launches, each timed alone
     serial_launches(1, True)
@@ -825,6 +839,28 @@ def sample_rays(sample_tiles: int):
     return out
 
 
+DUMP_BYTES = 60 << 20          # --dump-outputs writes at most this much: 16 B per sampled ray and frame
+
+
+def dump_outputs(out_dir, frames, n_rays):
+    """--dump-outputs: the outputs a caller of the timed path receives -- voxel id, face, hit time t -- for a fixed, seeded
+    sample of the n_rays rays of each frame (the same ray indices in every frame and every run), as
+    out_dir/<frame>_{voxel,face,t}.npy: voxel as float64 (exact for any uint32), face and t as float32 (t bit for bit).
+    A ray that leaves the volume without a hit (face 6) has t = +inf; the file holds -1 there, never a hit time, so that a
+    correct build writes only finite values.  Any other non-finite t is written as it is.
+    frames: [(name, take)], take(idx) -> (voxel, face, t) of the rays at the sorted indices idx."""
+    n = min(n_rays, DUMP_BYTES // (16 * len(frames)))
+    idx = np.sort(np.random.RandomState(0).choice(n_rays, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, take in frames:
+        v, f, t = take(idx)
+        np.save(os.path.join(out_dir, f"{name}_voxel.npy"), np.asarray(v, np.uint32).astype(np.float64))
+        f, t = np.asarray(f, np.uint8), np.asarray(t, np.float32)
+        np.save(os.path.join(out_dir, f"{name}_face.npy"), f.astype(np.float32))
+        np.save(os.path.join(out_dir, f"{name}_t.npy"), np.where((f == 6) & (t == np.inf), np.float32(-1.0), t))
+    log(f"--dump-outputs: {len(frames)} frame(s), {n} of {n_rays} rays each, written to {out_dir}")
+
+
 CPU_LAYOUT = ("compact level-ordered node array (the product's flatten) imported into the reference's nodes[]: 44 MiB contiguous instead of "
               "1.44 M nodes hashed over a 512 MiB table -- this favours the CPU arm; the traced function is the reference's own sse_trace")
 
@@ -866,15 +902,17 @@ def run_reference(args):
     n = sum(d.shape[0] for _, d in rays)
 
     def step():
-        for o, d in rays:
-            fn(o, d, cores)
+        return [fn(o, d, cores) for o, d in rays]
 
     for _ in range(max(1, min(args.warmup, 2))):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        last = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(f"frame{k}_pose{p}", lambda idx, r=r: tuple(a[idx] for a in r))
+                                         for k, (p, r) in enumerate(zip(POSE_NAMES, last))], last[0][0].size)
     value = n * args.steps / dt / 1e6
     sample = f"all rays of a step: the 3 poses' full 4K frames ({n} rays per step), {cores} threads"
     emit({
@@ -927,7 +965,12 @@ def main():
     ap.add_argument("--as-rank", default=None, metavar="R/N", help="with --quick on one GPU: trace the share rank R of an N-GPU job would")
     ap.add_argument("--variant", type=int, default=None, help="kernel variant (ort_set_option 'variant')")
     ap.add_argument("--opt", action="append", default=[], help="key=value passed to ort_set_option")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the last step's outputs (voxel, face, t) of a fixed, seeded sample of each "
+                         "frame's rays as DIR/<frame>_<output>.npy, at most 60 MiB in all, so that two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     TILE_ROWS = args.tile_rows
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":

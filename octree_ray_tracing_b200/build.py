@@ -66,10 +66,9 @@ def _compile(lib: str, defines, log_name: str, verbose: bool) -> None:
     cmd = [nvcc()] + NVCC_FLAGS + list(defines) + [os.path.join(CSRC, s) for s in SOURCES] + ["-o", lib]
     out = subprocess.run(cmd, capture_output=True, text=True)
     log = out.stdout + out.stderr
-    # the log is tracked (ptxas -v: registers, spills, stack per kernel); compile times would only make it churn
-    stable = "\n".join(line for line in log.splitlines() if "Compile time" not in line)
+    # the last build's ptxas -v report (registers, spills, stack per kernel); a build product, kept out of git
     with open(os.path.join(HERE, log_name), "w") as f:
-        f.write(" ".join(cmd) + "\n" + stable + "\n")
+        f.write(" ".join(cmd) + "\n" + log + "\n")
     if verbose or out.returncode:
         print(log)
     if out.returncode:

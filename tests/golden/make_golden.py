@@ -3,11 +3,13 @@
 
     python tests/golden/make_golden.py
 
-Each file holds inputs (a DAG as the reference's own table produced it, rays) and the outputs of the
+Each file holds inputs (a DAG as the reference's own table produced it, camera poses) and the outputs of the
 reference's own och::h_octree::sse_trace (och_h_octree.h:292-447) on this (Intel) host.  Nothing of
 ours is on the producing path except the fixture recursion in ref_wrap.cpp, which drives the
-reference's own register_node/set/simplex_n.
+reference's own register_node/set/simplex_n.  The incoherent and edge-case rays are not stored: golden_rays()
+draws them again from their seed, and the file keeps their sha256 so that a different draw is caught.
 """
+import hashlib
 import os
 import sys
 
@@ -84,6 +86,30 @@ def edge_rays(rs, n_each=2000):
     return np.concatenate(o).astype(np.float32), np.concatenate(d).astype(np.float32)
 
 
+RAY_SETS = ("d6_tunnels", "d8_tunnels")         # drawn in this order from one RandomState(12345)
+RAY_KEYS = ("rand_o", "rand_d", "edge_o", "edge_d")
+
+
+def golden_rays(name):
+    """The incoherent ("rand") and edge-case ("edge") rays of golden file `name`, drawn again from their seed."""
+    rs = np.random.RandomState(12345)
+    for set_name in RAY_SETS:
+        n = 40000
+        o = np.stack([rs.uniform(1.05, 1.95, n), rs.uniform(1.05, 1.95, n), rs.uniform(1.35, 1.95, n)], 1).astype(np.float32)
+        d = rs.normal(size=(n, 3)); d /= np.linalg.norm(d, axis=1, keepdims=True); d = d.astype(np.float32)
+        eo, ed = edge_rays(rs)
+        if set_name == name:
+            return dict(rand_o=o, rand_d=d, edge_o=eo, edge_d=ed)
+    raise KeyError(name)
+
+
+def rays_sha256(rays):
+    h = hashlib.sha256()
+    for k in RAY_KEYS:
+        h.update(np.ascontiguousarray(rays[k]).tobytes())
+    return h.hexdigest()
+
+
 def digest(vox, face, t):
     """FNV-1a-64 over (voxel u32, face u8, t bits u32) per ray, in ray order."""
     rec = np.zeros(vox.size, dtype=[("v", "<u4"), ("f", "u1"), ("t", "<u4")])
@@ -96,7 +122,6 @@ def digest(vox, face, t):
 
 def main():
     assert oc.have_ref(), "oracle/_ref/libochref.so missing: run make -C oracle in the authoring container"
-    rs = np.random.RandomState(12345)
 
     for name, (L, D, tunnels, W, H) in {"d6_tunnels": (16, 6, True, 160, 90), "d8_tunnels": (19, 8, True, 320, 180)}.items():
         hmap = oc.ref_heightmap(D)
@@ -121,16 +146,12 @@ def main():
             data[f"pose{pn}_vox"] = v1.astype(np.uint8)
             data[f"pose{pn}_face"] = f1
             data[f"pose{pn}_t"] = t1
-        # incoherent rays
-        n = 40000
-        o = np.stack([rs.uniform(1.05, 1.95, n), rs.uniform(1.05, 1.95, n), rs.uniform(1.35, 1.95, n)], 1).astype(np.float32)
-        d = rs.normal(size=(n, 3)); d /= np.linalg.norm(d, axis=1, keepdims=True); d = d.astype(np.float32)
-        v, f, t = T.trace(o, d)
-        data.update(rand_o=o, rand_d=d, rand_vox=v.astype(np.uint8), rand_face=f, rand_t=t)
-        # edge cases
-        o, d = edge_rays(rs)
-        v, f, t = T.trace(o, d)
-        data.update(edge_o=o, edge_d=d, edge_vox=v.astype(np.uint8), edge_face=f, edge_t=t)
+        # incoherent rays and edge cases
+        rays = golden_rays(name)
+        data["rays_sha256"] = rays_sha256(rays)
+        for k in ("rand", "edge"):
+            v, f, t = T.trace(rays[f"{k}_o"], rays[f"{k}_d"])
+            data.update({f"{k}_vox": v.astype(np.uint8), f"{k}_face": f, f"{k}_t": t})
         np.savez_compressed(os.path.join(OUT, f"{name}.npz"), **data)
         print(name, "nodes", nodes8.shape[0], "fill", T.fillcnt, {k: int((data[f'pose{k}_vox'] != 0).sum()) for k in POSES},
               "rand hits", int((data['rand_vox'] != 0).sum()), "edge faces", np.bincount(f, minlength=9).tolist())

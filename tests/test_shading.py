@@ -1,8 +1,11 @@
 """Shading epilogue (SURVEY 8f-4): voxels.txt parsing and the fused colour lookup of trace_pixel."""
+import json
 import os
 
 import numpy as np
 import pytest
+
+from conftest import GOLDEN, ROOT
 
 
 def test_parse_voxels_format_and_errors(ort):
@@ -10,8 +13,13 @@ def test_parse_voxels_format_and_errors(ort):
     cols, names = h.parse_voxels(h.DEMO_VOXELS)
     assert names == ["Stone", "Grass", "Dark Grass", "Dirt"] and cols.shape == (4, 6)
     assert cols[0, 0] == 0xFF5D4444          # "44445D" -> r=0x44 g=0x44 b=0x5D, alpha 0xFF, packed like olc::Pixel::n
-    ref_file = "/root/reference/Octree_Ray_Tracing/voxels.txt"
-    if os.path.exists(ref_file):             # authoring container only: the embedded palette is the reference's asset
+    # the reference's palette (voxels.txt): stored under tests/golden, and live where oracle/_ref is built from its sources
+    pal = json.load(open(os.path.join(GOLDEN, "voxels_palette.json")))
+    rgb = np.array([[int(c, 16) for c in row] for row in pal["faces_rrggbb"]], np.uint32)
+    want = 0xFF000000 | (rgb & 0xFF) << 16 | (rgb & 0xFF00) | (rgb >> 16)       # RRGGBB -> r | g<<8 | b<<16 | a<<24
+    assert names == pal["names"] and np.array_equal(cols, want)
+    ref_file = os.path.join(ROOT, "oracle", "_ref", "voxels.txt")
+    if os.path.exists(ref_file):
         c2, n2 = h.parse_voxels(open(ref_file).read())
         assert n2 == names and np.array_equal(c2, cols)
     for bad in ("Stone: 44445D 4E4E5B", "X: 12345G 000000 000000 000000 000000 000000", ": 000000 000000 000000 000000 000000 000000",
