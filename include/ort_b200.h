@@ -94,6 +94,22 @@ int ort_upload_delta(ort_ctx* ctx, const uint32_t* ids, const uint32_t* nodes8, 
  * ort_upload_delta afterwards addresses rows as id = row + 1 (its root argument is ignored in this layout). */
 int ort_upload_pool(ort_ctx* ctx, const uint32_t* nodes8, size_t n_nodes);
 
+/* Build the DAG of a dense voxel grid on ctx's GPU and install it as the device mirror, like ort_upload_full.
+ * voxels: nx*ny*nz unsigned elements of elem_bytes (1 or 4), index (z*ny + y)*nx + x = voxel (x, y, z); 0 = empty, cells
+ * outside the grid are empty.  Host or device pointer (a device source must be complete: synchronise its producer).
+ * The mirror afterwards holds exactly what ort_tree_flatten returns for a table holding these voxels: root id 1 (0 and
+ * n = 0 for an empty grid), level_offsets (optional, depth+1 entries) as ort_tree_flatten's.  ctx depth <= 11.
+ * ORT_ERR_INVALID for bad arguments, ORT_ERR_CAPACITY for a DAG beyond the 2^29 - 1 compact ids, ORT_ERR_CUDA when
+ * device memory runs out; after any failure the previous mirror is still installed.  A device source of 4-byte
+ * elements must be 4-byte aligned. */
+int ort_build_voxels(ort_ctx* ctx, const void* voxels, int elem_bytes, int nx, int ny, int nz,
+                     size_t* n_nodes, uint32_t* level_offsets);
+/* Copy n rows of the device mirror, starting at compact id first (1-based), to nodes8 (host or device). */
+int ort_read_nodes(ort_ctx* ctx, uint32_t first, size_t n, uint32_t* nodes8);
+/* Device bytes the last successful ort_build_voxels allocated: its temporaries plus a new mirror if it had to grow one
+ * (nothing is freed before the build ends, so this is its peak on top of what the context held). */
+uint64_t ort_build_bytes(const ort_ctx* ctx);
+
 /* Replaces: N calls of sse_trace(ox,oy,oz,dx,dy,dz, direction&, uint32_t&, float&) const
  * (och_h_octree.h:292-447).  o3: origins, 3 floats each, o_stride = 3, or ONE shared origin with
  * o_stride = 0.  d3: n directions.  Outputs per ray: voxel = hit_voxel, face = hit_direction,
@@ -326,6 +342,12 @@ const uint32_t* ort_tree_refcounts(const ort_tree* tree);
  * next flatten/sync.  level_offsets (optional, depth+1 entries) receives the first id of each
  * level (entry depth = n+1).  Pure host code. */
 size_t   ort_tree_flatten(ort_tree* tree, const uint32_t** nodes8, uint32_t* root, uint32_t* level_offsets);
+/* Register a compact level-ordered DAG (as ort_tree_flatten / ort_read_nodes give it) in an EMPTY table: nodes interned
+ * bottom-up, reference counts = instance counts (as the fixture builder assigns them), fillcnt / nodecnt accordingly;
+ * the next ort_tree_sync is a full upload.  Host pointer, or device pointer when the tree is attached to a context (the
+ * copy runs on that context's stream; a tree without a context makes no CUDA call).  ORT_ERR_INVALID for a non-empty table or a
+ * malformed DAG (child id out of range or at the wrong level, an all-zero reachable row); ORT_ERR_TABLE_FULL as set(). */
+int      ort_tree_import(ort_tree* tree, const uint32_t* nodes8, size_t n, uint32_t root);
 
 /* Bind a device context: subsequent ort_tree_sync() calls mirror the table into it. */
 int      ort_tree_attach(ort_tree* tree, ort_ctx* ctx);

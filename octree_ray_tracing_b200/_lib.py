@@ -37,6 +37,9 @@ _SIGS = {
     "ort_upload_full": (C.c_int, [_vp, _vp, C.c_size_t, C.c_uint32]),
     "ort_upload_delta": (C.c_int, [_vp, _vp, _vp, C.c_size_t, C.c_uint32]),
     "ort_upload_pool": (C.c_int, [_vp, _vp, C.c_size_t]),
+    "ort_build_voxels": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t), _vp]),
+    "ort_read_nodes": (C.c_int, [_vp, C.c_uint32, C.c_size_t, _vp]),
+    "ort_build_bytes": (C.c_uint64, [_vp]),
     "ort_trace_rays": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_size_t, _vp, _vp, _vp, _vp]),
     "ort_trace_frame": (C.c_int, [_vp, _vp, _vp, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, _vp]),
     "ort_trace_frame_async": (C.c_int, [_vp, _vp, _vp, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, _vp]),
@@ -85,6 +88,7 @@ _SIGS = {
     "ort_tree_cashes": (C.POINTER(C.c_uint8), [_vp]),
     "ort_tree_refcounts": (_u32p, [_vp]),
     "ort_tree_flatten": (C.c_size_t, [_vp, C.POINTER(_u32p), _u32p, _vp]),
+    "ort_tree_import": (C.c_int, [_vp, _vp, C.c_size_t, C.c_uint32]),
     "ort_tree_attach": (C.c_int, [_vp, _vp]),
     "ort_tree_sync": (C.c_int, [_vp]),
     "ort_tree_sync_stats": (None, [_vp, C.POINTER(C.c_uint64), C.POINTER(C.c_int)]),

@@ -21,7 +21,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libort_b200.so")
 LIB_EXP = os.path.join(HERE, "libort_b200_exp.so")
 SOURCES = ["ort_device.cu", "ort_host_tree.cpp", "ort_host_octree.cpp", "ort_fixture.cpp"]
-HEADERS = ["ort_internal.h", "ort_trace.cuh", "ort_beam.cuh", "ort_kernels.cuh", "ort_mg.cuh", "ort_noise.h", "ort_rcp_table.h", os.path.join("..", "..", "include", "ort_b200.h")]
+HEADERS = ["ort_internal.h", "ort_trace.cuh", "ort_beam.cuh", "ort_kernels.cuh", "ort_build.cuh", "ort_mg.cuh", "ort_noise.h", "ort_rcp_table.h", os.path.join("..", "..", "include", "ort_b200.h")]
 HEADERS_EXP = ["ort_experiments.cuh", "ort_trace_experiments.cuh"]
 
 NVCC_FLAGS = [

@@ -113,6 +113,7 @@ struct ort_ctx
 	uint64_t beam_seen_seq = 0;
 	bool frame_call_nested = false;
 	uint64_t beam_builds = 0;
+	uint64_t build_bytes = 0;           // device bytes the last successful ort_build_voxels allocated (its peak)
 
 	unsigned long long* d_counters = nullptr; // work counters of the persistent kernels: a ring, one per launch (kCounterRing)
 	unsigned next_counter = 0;
@@ -250,6 +251,7 @@ inline void beam_invalidate(ort_ctx* c)
 }  // namespace
 
 #include "ort_kernels.cuh"
+#include "ort_build.cuh"
 
 namespace {
 
@@ -815,6 +817,255 @@ int ort_upload_delta(ort_ctx* c, const uint32_t* ids, const uint32_t* nodes8, si
 	if (changed) beam_invalidate(c);            // (an empty delta -- a per-frame sync without edits -- leaves the grids alone)
 	return ORT_OK;
 }
+
+// ------------------------------------------------------------------------------------------------
+// DAG of a dense voxel grid (ort_build.cuh, DESIGN section 13)
+// ------------------------------------------------------------------------------------------------
+
+}  // extern "C"
+
+namespace {
+
+// device allocations of one build, released however the build ends; `bytes` counts them (nothing is freed before the
+// end, so that is the build's peak)
+struct BuildTemps
+{
+	std::vector<void*> ptrs;
+	uint64_t bytes = 0;
+	~BuildTemps() { for (void* p : ptrs) cudaFree(p); }
+	template<class T> cudaError_t alloc(T** p, size_t count)
+	{
+		void* q = nullptr;
+		const size_t b = count ? count * sizeof(T) : sizeof(T);
+		const cudaError_t e = cudaMalloc(&q, b);
+		if (e == cudaSuccess) { ptrs.push_back(q); bytes += b; }
+		*p = static_cast<T*>(q);
+		return e;
+	}
+};
+
+inline unsigned blocks_for(size_t n, unsigned threads = 256) { return static_cast<unsigned>((n + threads - 1) / threads); }
+
+inline size_t pow2_at_least(size_t v)
+{
+	size_t p = 64;
+	while (p < v) p <<= 1;
+	return p;
+}
+
+int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, uint32_t ny, uint32_t nz, size_t* n_out, uint32_t* level_offsets)
+{
+	const int D = c->depth;
+	cudaStream_t st = c->stream;
+	BuildTemps tmp;
+
+	// the input, on this device
+	const void* src = voxels;
+	{
+		cudaPointerAttributes a;
+		const bool dev = cudaPointerGetAttributes(&a, voxels) == cudaSuccess && (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged);
+		cudaGetLastError();
+		if (dev && a.type == cudaMemoryTypeDevice && a.device != c->device)
+			return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: the voxels live on device %d, the context on device %d", a.device, c->device);
+		if (dev && (reinterpret_cast<uintptr_t>(voxels) & static_cast<uintptr_t>(elem_bytes - 1)))
+			return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: a device source of %d-byte elements must be %d-byte aligned", elem_bytes, elem_bytes);
+		if (!dev)
+		{
+			const size_t bytes = static_cast<size_t>(nx) * ny * nz * elem_bytes;
+			void* d = nullptr;
+			ORT_CUDA(c, tmp.alloc(reinterpret_cast<uint8_t**>(&d), bytes));
+			ORT_CUDA(c, cudaMemcpyAsync(d, voxels, bytes, cudaMemcpyDefault, st));
+			src = d;
+		}
+	}
+	const ort::BuildInput in{ src, elem_bytes, nx, ny, nz };
+
+	// level grids, clipped to the input's extent: level l has cells of side 2^(D-l+1) voxels
+	ort::BuildLevel lv[ort::kBuildMaxDepth + 2] = {};
+	size_t cap[ort::kBuildMaxDepth + 2] = {};
+	{
+		uint32_t gx = (nx + 1) / 2, gy = (ny + 1) / 2, gz = (nz + 1) / 2;
+		for (int l = D; l >= 1; --l)
+		{
+			lv[l].gx = gx; lv[l].gy = gy; lv[l].gz = gz;
+			ORT_CUDA(c, tmp.alloc(&lv[l].ids, static_cast<size_t>(gx) * gy * gz));
+			gx = (gx + 1) / 2; gy = (gy + 1) / 2; gz = (gz + 1) / 2;
+		}
+	}
+	unsigned long long* d_cnt = nullptr;                       // [0] leaf non-empty, [l] non-empty of level l, [D+1+l] distinct
+	ORT_CUDA(c, tmp.alloc(&d_cnt, 2 * (D + 1)));
+	ORT_CUDA(c, cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long) * 2 * (D + 1), st));
+	unsigned long long h_cnt[2 * (ort::kBuildMaxDepth + 1)] = {};
+
+	// bottom-up: a level's distinct contents are at most its non-empty cells, which are at most the level below's
+	ort::build_count_leaf_kernel<<<blocks_for(static_cast<size_t>(lv[D].gx) * lv[D].gy * lv[D].gz), 256, 0, st>>>(in, lv[D], d_cnt);
+	++c->launches;
+	ORT_CUDA(c, cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+	ORT_CUDA(c, cudaStreamSynchronize(st));
+	size_t bound = static_cast<size_t>(h_cnt[0]);
+	for (int l = D; l >= 1; --l)
+	{
+		const size_t cells = static_cast<size_t>(lv[l].gx) * lv[l].gy * lv[l].gz;
+		cap[l] = pow2_at_least(2 * std::min(bound, cells));      // load factor <= 1/2
+		ORT_CUDA(c, tmp.alloc(&lv[l].table, cap[l]));
+		lv[l].mask = static_cast<uint32_t>(cap[l] - 1);
+		ORT_CUDA(c, cudaMemsetAsync(lv[l].table, 0xFF, cap[l] * 4, st));
+		ort::build_insert_kernel<<<blocks_for(cells), 256, 0, st>>>(l == D, in, lv[l], l == D ? lv[l] : lv[l + 1], d_cnt + l);
+		ort::build_count_table_kernel<<<blocks_for(cap[l]), 256, 0, st>>>(lv[l].table, cap[l], d_cnt + D + 1 + l);
+		c->launches += 2;
+		ORT_CUDA(c, cudaGetLastError());
+		ORT_CUDA(c, cudaMemcpyAsync(h_cnt + l, d_cnt + l, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+		ORT_CUDA(c, cudaStreamSynchronize(st));
+		bound = static_cast<size_t>(h_cnt[l]);
+	}
+	ORT_CUDA(c, cudaMemcpyAsync(h_cnt + D + 1, d_cnt + D + 1, sizeof(unsigned long long) * (D + 1), cudaMemcpyDeviceToHost, st));
+	ORT_CUDA(c, cudaStreamSynchronize(st));
+
+	// final ids: level l holds ids base[l] .. base[l] + n[l] - 1
+	size_t n_lvl[ort::kBuildMaxDepth + 2] = {}, base[ort::kBuildMaxDepth + 2] = {};
+	size_t total = 0;
+	for (int l = 1; l <= D; ++l)
+	{
+		n_lvl[l] = static_cast<size_t>(h_cnt[D + 1 + l]);
+		base[l] = 1 + total;
+		total += n_lvl[l];
+	}
+	if (total > ort::kIdMask)
+		return ort_fail(c, ORT_ERR_CAPACITY, "ort_build_voxels: the grid's DAG has %zu nodes, more than the %u compact ids allow", total, ort::kIdMask);
+
+	// the output rows: straight into a new mirror when the current one is too small, else a temporary copied over
+	uint32_t* out = nullptr;
+	size_t out_cap = 0;
+	struct NewMirror { uint32_t* p = nullptr; ~NewMirror() { cudaFree(p); } } fresh;
+	if (total > c->cap_nodes)
+	{
+		out_cap = std::min<size_t>(total + total / 4 + 4096, ort::kIdMask);      // head-room for the deltas that follow, as ort_upload_full
+		ORT_CUDA(c, cudaMalloc(&fresh.p, out_cap * 32));
+		out = fresh.p;
+	}
+	else if (total)
+		ORT_CUDA(c, tmp.alloc(&out, total * 8));
+
+	if (total)
+	{
+		// top-down: scratch sized for the widest level
+		size_t max_slots = 0, max_cap = 0;
+		for (int l = 1; l < D; ++l) { max_slots = std::max(max_slots, 8 * n_lvl[l]); max_cap = std::max(max_cap, cap[l + 1]); }
+		uint32_t *ch = nullptr, *pos = nullptr, *first = nullptr, *scratch = nullptr;
+		uint32_t* frontier[ort::kBuildMaxDepth + 2] = {};
+		for (int l = 1; l <= D; ++l) ORT_CUDA(c, tmp.alloc(&frontier[l], n_lvl[l]));
+		if (max_slots)
+		{
+			ORT_CUDA(c, tmp.alloc(&ch, max_slots));
+			ORT_CUDA(c, tmp.alloc(&pos, max_slots));
+			ORT_CUDA(c, tmp.alloc(&first, max_cap));
+			ORT_CUDA(c, tmp.alloc(&scratch, ort::scan_scratch_words(max_slots)));
+		}
+		ORT_CUDA(c, cudaMemcpyAsync(frontier[1], lv[1].ids, 4, cudaMemcpyDeviceToDevice, st));     // the root cell's temporary id
+		for (int l = 1; l < D; ++l)
+		{
+			const size_t slots = 8 * n_lvl[l];
+			ORT_CUDA(c, cudaMemsetAsync(first, 0xFF, cap[l + 1] * 4, st));
+			ort::build_children_kernel<<<blocks_for(slots), 256, 0, st>>>(frontier[l], slots, lv[l], lv[l + 1], ch, first);
+			ort::build_flags_kernel<<<blocks_for(slots), 256, 0, st>>>(ch, first, slots, pos);
+			c->launches += 2;
+			ort::scan_exclusive(pos, slots, scratch, st, c->launches);
+			ort::build_rows_kernel<<<blocks_for(slots), 256, 0, st>>>(ch, first, pos, slots, static_cast<uint32_t>(base[l + 1]),
+			                                                          out + 8 * (base[l] - 1), frontier[l + 1]);
+			++c->launches;
+			ORT_CUDA(c, cudaGetLastError());
+		}
+		ort::build_leaf_rows_kernel<<<blocks_for(n_lvl[D]), 256, 0, st>>>(frontier[D], n_lvl[D], in, lv[D], out + 8 * (base[D] - 1));
+		++c->launches;
+		ORT_CUDA(c, cudaGetLastError());
+	}
+	ORT_CUDA(c, cudaStreamSynchronize(st));
+
+	// install, as ort_upload_full does: every launch in flight reads the array that is replaced
+	ORT_CUDA(c, cudaDeviceSynchronize());
+	if (out_cap)
+	{
+		cudaFree(c->d_nodes);
+		c->d_nodes = out;
+		c->cap_nodes = static_cast<uint32_t>(out_cap);
+		fresh.p = nullptr;                                         // (owned by the context now)
+	}
+	else if (total)
+	{
+		ORT_CUDA(c, cudaMemcpyAsync(c->d_nodes, out, total * 32, cudaMemcpyDeviceToDevice, st));
+		ORT_CUDA(c, cudaStreamSynchronize(st));
+	}
+	c->n_nodes = static_cast<uint32_t>(total);
+	c->root = total ? 1u : 0u;
+	c->index_base = 1;
+	c->has_root = total != 0;
+	c->miss_t = __builtin_inff();
+	beam_invalidate(c);
+	c->build_bytes = tmp.bytes + out_cap * 32;
+	if (n_out) *n_out = total;
+	if (level_offsets)
+	{
+		for (int l = 1; l <= D; ++l) level_offsets[l - 1] = static_cast<uint32_t>(base[l]);
+		level_offsets[D] = static_cast<uint32_t>(total + 1);
+	}
+	return ORT_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ort_build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, int nx, int ny, int nz, size_t* n_nodes, uint32_t* level_offsets)
+{
+	enter(c);
+	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: null context");
+	if (c->depth > ort::kBuildMaxDepth)
+		return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: context depth %d; the builder takes depth <= %d", c->depth, ort::kBuildMaxDepth);
+	const int dim = 1 << c->depth;
+	if (!voxels || (elem_bytes != 1 && elem_bytes != 4) || nx < 1 || ny < 1 || nz < 1 || nx > dim || ny > dim || nz > dim)
+		return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: bad arguments (voxels=%p elem_bytes=%d extent %d x %d x %d, 1..%d per axis)",
+		                voxels, elem_bytes, nx, ny, nz, dim);
+	DeviceGuard g(c->device);
+	const int rc = build_voxels(c, voxels, elem_bytes, static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz), n_nodes, level_offsets);
+	if (rc != ORT_OK) cudaGetLastError();       // (an allocation that failed leaves its error behind for the next check)
+	return rc;
+}
+
+int ort_read_nodes(ort_ctx* c, uint32_t first, size_t n, uint32_t* nodes8)
+{
+	enter(c);
+	if (!c || (n && (!nodes8 || first == 0 || static_cast<size_t>(first) - 1 + n > c->n_nodes)))
+		return ort_fail(c, ORT_ERR_INVALID, "ort_read_nodes: bad arguments (first=%u n=%zu, %u rows in the mirror)", first, n, c ? c->n_nodes : 0u);
+	if (!n) return ORT_OK;
+	DeviceGuard g(c->device);
+	ORT_CUDA(c, cudaMemcpyAsync(nodes8, c->d_nodes + 8 * (static_cast<size_t>(first) - 1), n * 32, cudaMemcpyDefault, c->stream));
+	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
+	return ORT_OK;
+}
+
+uint64_t ort_build_bytes(const ort_ctx* c) { return c ? c->build_bytes : 0; }
+
+}  // extern "C"
+
+// Host copy of a buffer that may live on a device (ort_tree_import), made on the context's stream: the buffer itself
+// when it is host memory or there is no context (a tree without one makes no CUDA call), nullptr when the copy fails.
+const void* ort_host_view(ort_ctx* c, const void* p, size_t bytes, std::vector<uint8_t>& keep)
+{
+	if (!c || !p) return p;
+	DeviceGuard g(c->device);
+	cudaPointerAttributes a;
+	if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return p; }
+	if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) return p;
+	keep.resize(bytes);
+	if (cudaMemcpyAsync(keep.data(), p, bytes, cudaMemcpyDefault, c->stream) != cudaSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess)
+	{
+		cudaGetLastError();
+		return nullptr;
+	}
+	return keep.data();
+}
+
+extern "C" {
 
 // ------------------------------------------------------------------------------------------------
 // trace

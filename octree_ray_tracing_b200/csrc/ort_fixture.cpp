@@ -334,7 +334,7 @@ uint32_t build_parallel(const Builder& b, ort_tree* tree, int nthreads, bool& fa
 
 // refcount(node) = number of instances of the node in the fully expanded tree = what one
 // register_node call per instance (the reference's builders) would have produced.
-static void assign_instance_counts(ort_tree* t, int nthreads)
+void assign_instance_counts(ort_tree* t, int nthreads)
 {
 	if (!t->root) return;
 	struct Acc

@@ -1033,6 +1033,78 @@ int ort_tree_load(ort_tree* t, const char* path)
 	return ORT_OK;
 }
 
+// A compact level-ordered DAG (ort_tree_flatten / ort_read_nodes) into an empty table.  A device buffer is read through
+// the attached context; a tree without one takes host memory only and makes no CUDA call.  The input is checked in full
+// before the table is written: a walk from the root for exactly `depth` levels (so a cyclic input cannot hang it) in
+// which every child id must lie in [1, n] and beyond every id of its parent's level, and no reachable row may be empty.
+int ort_tree_import(ort_tree* t, const uint32_t* nodes8, size_t n, uint32_t root)
+{
+	if (!t) return ort_fail(nullptr, ORT_ERR_INVALID, "ort_tree_import: null tree");
+	if (t->root != 0 || t->fillcnt != 0)
+		return ort_fail(nullptr, ORT_ERR_INVALID, "ort_tree_import: the table is not empty (root %u, %u live nodes)", t->root, t->fillcnt);
+	if (n == 0)
+		return root == 0 ? ORT_OK : ort_fail(nullptr, ORT_ERR_INVALID, "ort_tree_import: root %u of an empty DAG", root);
+	if (!nodes8 || root == 0 || root > n || n > UINT32_MAX)
+		return ort_fail(nullptr, ORT_ERR_INVALID, "ort_tree_import: bad arguments (n=%zu root=%u)", n, root);
+	std::vector<uint8_t> keep;
+	const uint32_t* rows = static_cast<const uint32_t*>(ort_host_view(t->ctx, nodes8, n * 32, keep));
+	if (!rows) return ort_fail(nullptr, ORT_ERR_INVALID, "ort_tree_import: cannot read the device buffer");
+
+	const int depth = t->depth;
+	std::vector<std::vector<uint32_t>> level(depth + 1);      // level[l]: ids reached at level l, in discovery order
+	std::vector<uint8_t> seen(n, 0);
+	level[1].push_back(root);
+	seen[root - 1] = 1;
+	for (int l = 1; l <= depth; ++l)
+	{
+		const uint32_t top = *std::max_element(level[l].begin(), level[l].end());
+		for (const uint32_t id : level[l])
+		{
+			const uint32_t* r = rows + 8 * static_cast<size_t>(id - 1);
+			if (!(r[0] | r[1] | r[2] | r[3] | r[4] | r[5] | r[6] | r[7]))
+				return ort_fail(nullptr, ORT_ERR_INVALID, "ort_tree_import: node %u (level %d) is reachable and has no children", id, l);
+			if (l == depth) continue;
+			for (int c = 0; c < 8; ++c)
+			{
+				const uint32_t ch = r[c];
+				if (!ch) continue;
+				if (ch > n)
+					return ort_fail(nullptr, ORT_ERR_INVALID, "ort_tree_import: node %u child %d = %u is out of range (n = %zu)", id, c, ch, n);
+				if (ch <= top)
+					return ort_fail(nullptr, ORT_ERR_INVALID, "ort_tree_import: node %u (level %d) child %d = %u points to its own level or above", id, l, c, ch);
+				if (!seen[ch - 1]) { seen[ch - 1] = 1; level[l + 1].push_back(ch); }
+			}
+		}
+	}
+
+	// bottom-up: children are in the table before their parents
+	std::vector<uint32_t> slot_of(n + 1, 0), created;
+	for (int l = depth; l >= 1; --l)
+		for (const uint32_t id : level[l])
+		{
+			uint32_t row[8];
+			std::memcpy(row, rows + 8 * static_cast<size_t>(id - 1), 32);
+			if (l != depth)
+				for (int c = 0; c < 8; ++c) if (row[c]) row[c] = slot_of[row[c]];
+			const uint32_t before = t->fillcnt;
+			const uint32_t s = t->intern_node(row);
+			if (!s)
+			{
+				// table full (flag set, as set() leaves it): take back what this call inserted
+				for (const uint32_t k : created) t->tags[k - 1] = 0xFF;
+				t->fillcnt = 0;
+				t->invalidate_mirror();
+				return ort_fail(nullptr, ORT_ERR_TABLE_FULL, "ort_tree_import: the table is full");
+			}
+			if (t->fillcnt != before) created.push_back(s);
+			slot_of[id] = s;
+		}
+	t->root = slot_of[root];
+	assign_instance_counts(t, static_cast<int>(std::max(1u, std::thread::hardware_concurrency())));
+	t->invalidate_mirror();
+	return ORT_OK;
+}
+
 size_t ort_tree_flatten(ort_tree* t, const uint32_t** nodes8, uint32_t* root, uint32_t* level_offsets)
 {
 	const size_t n = t->flatten(level_offsets);

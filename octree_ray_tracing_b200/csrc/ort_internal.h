@@ -17,6 +17,10 @@ void* ort_zalloc(size_t bytes);
 void  ort_zfree(void* p, size_t bytes);
 void  ort_prefault(void* const* ptrs, const size_t* bytes, int n_ranges, int nthreads);
 
+// `p` itself when it is host memory or ctx is null (no CUDA call is made then), else a host copy of its `bytes` kept in
+// `keep`, made on ctx's stream; nullptr when that copy fails.
+const void* ort_host_view(ort_ctx* ctx, const void* p, size_t bytes, std::vector<uint8_t>& keep);
+
 // Host node store.  Field meanings follow och::h_octree (och_h_octree.h:70-99).
 struct ort_tree
 {
@@ -96,3 +100,7 @@ private:
 	uint32_t delta_visit(uint32_t slot, int level);
 	uint32_t& id_ref(uint32_t slot, int level, bool assign);
 };
+
+// Adds to every node reachable from t->root its number of instances in the fully expanded tree (what one register_node
+// call per instance would have counted), and their sum to nodecnt.  For DAGs interned with intern_node (ort_fixture.cpp).
+void assign_instance_counts(ort_tree* t, int nthreads);

@@ -114,6 +114,44 @@ class TraceContext:
         assert a.shape[0] == i.size
         self._ck(self.L.ort_upload_delta(self.h, _p(i), _p(a), i.size, root))
 
+    def upload_voxels(self, grid):
+        """Build the DAG of a dense voxel grid on this context's GPU and install it as the mirror (ort_build_voxels).
+        grid: C-contiguous 3-D numpy array or torch tensor (CPU or CUDA) of shape (nz, ny, nx), dtype uint8, int32 or
+        uint32 (read as unsigned); grid[z, y, x] is voxel (x, y, z), 0 = empty.  Returns (n_nodes, level_offsets):
+        the mirror then holds what HOctree.flatten() gives for a table holding these voxels."""
+        if isinstance(grid, np.ndarray):
+            if grid.dtype not in (np.uint8, np.int32, np.uint32):
+                raise TypeError(f"upload_voxels: dtype {grid.dtype} (uint8, int32 or uint32 required)")
+            if grid.ndim != 3 or not grid.flags.c_contiguous:
+                raise ValueError("upload_voxels: a C-contiguous 3-D array of shape (nz, ny, nx) is required")
+            elem = grid.dtype.itemsize
+        elif hasattr(grid, "data_ptr"):
+            import torch
+            if grid.dtype not in (torch.uint8, torch.int32, torch.uint32):
+                raise TypeError(f"upload_voxels: dtype {grid.dtype} (uint8, int32 or uint32 required)")
+            if grid.dim() != 3 or not grid.is_contiguous():
+                raise ValueError("upload_voxels: a contiguous 3-D tensor of shape (nz, ny, nx) is required")
+            if grid.is_cuda:
+                if grid.device.index != self.device:
+                    raise ValueError(f"upload_voxels: the tensor is on {grid.device}, the context on cuda:{self.device}")
+                torch.cuda.current_stream(grid.device).synchronize()      # the builder reads it on its own stream
+            elem = grid.element_size()
+        else:
+            raise TypeError(f"upload_voxels: numpy array or torch tensor required, got {type(grid).__name__}")
+        nz, ny, nx = (int(s) for s in grid.shape)
+        n = C.c_size_t(0)
+        lo = np.zeros(self.depth + 1, np.uint32)
+        self._ck(self.L.ort_build_voxels(self.h, _p(grid), elem, nx, ny, nz, C.byref(n), _p(lo)))
+        return n.value, lo
+
+    def read_nodes(self, first: int = 1, n: int | None = None) -> np.ndarray:
+        """Rows first .. first + n - 1 (compact ids, 1-based) of the device mirror as an (n, 8) uint32 array."""
+        if n is None:
+            n = max(0, self.node_count - first + 1)
+        out = np.zeros((n, 8), np.uint32)
+        self._ck(self.L.ort_read_nodes(self.h, first, n, _p(out)))
+        return out
+
     def set_option(self, key: str, value: int):
         self._ck(self.L.ort_set_option(self.h, key.encode(), value))
 
@@ -154,6 +192,11 @@ class TraceContext:
         out = np.zeros((n, n, n), np.uint8)
         self._ck(self.L.ort_beam_grid(self.h, level, _p(out)))
         return out
+
+    @property
+    def build_bytes(self) -> int:
+        """Device bytes the last successful upload_voxels allocated (its peak on top of what the context held)."""
+        return self.L.ort_build_bytes(self.h)
 
     @property
     def beam_builds(self) -> int:
@@ -353,6 +396,40 @@ class HOctree:
         n = self.L.ort_tree_flatten(self.h, C.byref(p), C.byref(root), _p(lo))
         arr = np.ctypeslib.as_array(p, shape=(n, 8)).copy() if n else np.zeros((0, 8), np.uint32)
         return arr, root.value, lo
+
+    def import_dag(self, nodes8, root: int):
+        """Register a compact level-ordered DAG (as flatten() / TraceContext.read_nodes give it) in this EMPTY table;
+        reference counts become instance counts, so set / fill_box / sync continue from it (ort_tree_import)."""
+        if hasattr(nodes8, "data_ptr"):
+            if nodes8.element_size() != 4 or not nodes8.is_contiguous():
+                raise ValueError("import_dag: a contiguous 32-bit tensor of n x 8 node words is required")
+            if nodes8.is_cuda and self.ctx is None:
+                raise ValueError("import_dag: a CUDA tensor needs an attached device context (the copy runs on its stream)")
+            if nodes8.is_cuda:
+                import torch
+                torch.cuda.current_stream(nodes8.device).synchronize()
+            n = nodes8.numel() // 8
+        else:
+            nodes8 = np.ascontiguousarray(nodes8, np.uint32).reshape(-1, 8)
+            n = nodes8.shape[0]
+        check(self.L.ort_tree_import(self.h, _p(nodes8), n, root))
+
+    def load_voxels(self, grid):
+        """Build a dense voxel grid's DAG on the attached context's GPU (TraceContext.upload_voxels), import it into
+        this empty table and sync.  Returns (n_nodes, level_offsets)."""
+        if self.ctx is None:
+            raise OrtError(6, "load_voxels: no device context attached (the builder runs on the GPU)")
+        if self.get_root() or self.get_fillcnt():
+            raise OrtError(1, f"load_voxels: the table is not empty (root {self.get_root()}, {self.get_fillcnt()} live nodes)")
+        n, lo = self.ctx.upload_voxels(grid)
+        try:
+            self.import_dag(self.ctx.read_nodes(1, n), self.ctx.root)
+            self.sync()
+        except BaseException:
+            # the context now holds the grid, not this table: the next sync must be a full upload of the table
+            self.attach(self.ctx)
+            raise
+        return n, lo
 
     def take_delta(self):
         """(ids or None, nodes8, root, is_full): the pending device update, consumed."""
