@@ -263,9 +263,11 @@ uint64_t ort_launch_count(const ort_ctx* ctx);
  * cube unhindered end as a MISS without a round -- same outputs bit for bit, fewer PUSH rounds; 0 = every ray walks from
  * its origin like och_h_octree.h:292-447), "beam_after" (default 2: a DAG version gets its grid once it has been traced
  * that many times without one, so that a loop which edits the DAG every other frame never pays for grids it cannot use;
- * 0 = build at the first frame), "beam_level" (force a coarser grid level, measurement), "count_beam"
+ * 0 = build at the first frame; where the pixels are fine enough, tiles of DAGs of depth 8 and more then refine their start
+ * on a level-8 grid built with it), "beam_level" (force a coarser grid level and no refinement, measurement), "count_beam"
  * (launches that return PUSH counts normally walk from the origin so that the counts are the reference's; 1 = they
- * use the beam start too and count the loads actually issued).
+ * use the beam start of the launch's level and count the loads issued then; 2 = they refine on level 8 too, as the
+ * frame launches without counts do).
  * Band schedule: "band_order" (1 = default: a frame launch of a view that has been traced before -- same camera, same
  * rows -- schedules its 16-row bands by what they cost last time, most expensive first, so that the long rays of a view
  * start early; 0 = the "band_rotate" rule only).  Outputs never depend on it. */
@@ -273,12 +275,13 @@ int ort_set_option(ort_ctx* ctx, const char* key, int value);
 
 /* Introspection of the beam start.  ort_beam_level: the grid level (3..7) frame launches of this camera geometry would
  * use on ctx, 0 = they run without a beam start (pixels too coarse for the coarsest grid, rot not a rotation, option
- * off, ...).  ort_beam_grid: the level-`level` grid of the DAG currently on the device, (2^level)^3 bytes to host
+ * off, ...); tiles may refine on level 8 beyond it.  ort_beam_grid: the level-`level` grid (1..8) of the DAG currently on the device, (2^level)^3 bytes to host
  * memory, index (z * N + y) * N + x: 0 = some cell among the 27 around this one holds a voxel, j > 0 = the level-j cell
  * around this one has no such cell.  Both are for tests and tools; tracing needs neither. */
 int ort_beam_level(ort_ctx* ctx, const float pos[3], const float rot[9], float fov_factor, int W, int H);
 int ort_beam_grid(ort_ctx* ctx, int level, uint8_t* skip_out);
-/* number of beam grids built on ctx since creation (one per DAG version and level in use) */
+/* number of beam grid builds on ctx since creation (one per DAG version and level in use; a launch's level and the level-8
+ * grid of its refinement, built together, count as one) */
 uint64_t ort_beam_builds(const ort_ctx* ctx);
 /* number of band schedules applied on ctx since creation (option "band_order", default 1: a frame launch records what each
  * 16-row band cost, the next launches of the same view -- same camera, same rows -- schedule the most expensive bands

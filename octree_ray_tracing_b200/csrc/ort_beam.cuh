@@ -42,14 +42,26 @@
 //     a 16th of a cell into a neighbour it runs along; the cells it can miss that way are clipped by less than the slack
 //     (0.3 s).  tau = tau_c (1 - 2^-12) - 2^-17.
 //
+//     The condition on t_max is stronger than the argument needs: it uses the bound only at the times t < tau_c, and
+//     there every ray of the tile stays within R t <= R tau_c of the central ray.  t_max was only ever an upper bound of
+//     tau_c.  So a tile may march on from its level-k stop t_k on the finer level-8 grid (beam_tile_start, refinement) and
+//     stop at t_8: for t < t_k the level-k march answers as before (R t <= R t_max fits level k), for t_k <= t < t_8 every
+//     ray is within R t_8 of the central ray, inside one of the 27 level-8 cells around the central ray's cell, as long as
+//     R t_8 + slack <= 0.7 2^-8.  That is checked per tile at t_8, where the march stops (the beam only widens with t), as
+//     t_8 <= t_fine = (0.7 2^-8 - slack) / R, rounded down on the host.  A tile that fails it keeps t_k.  A march that
+//     leaves the cube stops at the sample that is more than a level-8 cell outside, and the same check at that time lets
+//     its tile see nothing (+inf, item 3 with level-8 cells).
+//
 // (3) Tiles that see nothing.  When the central ray has left the cube by more than a cell without meeting a marked cell,
 //     every ray of the tile has left it too: tau = +inf.  If all rays of the tile are certain to be lean-tier rays
 //     (beam_tile_start), the trace kernel writes 32 MISSes and is done -- no camera ray, no reciprocals.
 //
 // What this buys is measured in profiles/ (r2_final_beam_ncu_full.md, r2_bench_n1.json) and argued in DESIGN.md 4b; what it
 // costs is one byte grid per DAG version and level in use (built lazily: occupancy, dilation, k - 1 pyramid levels, skip
-// levels; 8^k bytes) and one march per tile (a separate launch, one thread per tile).
-// Tested claim by claim: tests/test_beam.py (this header compiled for the host) and tests/test_gpu_beam.py.
+// levels; 8^k bytes; the level-8 grid of the refinement is built with the launch's level) and one march per tile (a
+// separate launch, one thread per tile).
+// Tested claim by claim: tests/test_beam.py (this header compiled for the host) and tests/test_gpu_beam.py; the level-8
+// refinement in tests/test_beam_refine.py and tests/test_gpu_beam_refine.py.
 #pragma once
 
 #include <cmath>
@@ -59,7 +71,8 @@
 namespace ort {
 
 constexpr int kBeamMinLevel = 3;      // below this the grid says nothing (8 cells per axis)
-constexpr int kBeamMaxLevel = 7;      // 128^3 bytes = 2 MiB
+constexpr int kBeamMaxLevel = 7;      // 128^3 bytes = 2 MiB: the finest level a whole launch is bounded with
+constexpr int kBeamFineLevel = 8;     // 256^3 bytes = 16 MiB: the grid tiles refine their start on (item 2)
 constexpr int kBeamMaxSteps = 64;       // a march that needs more ends early: its tile starts where the march stood
 
 struct BeamGrid
@@ -78,6 +91,20 @@ inline int beam_level_for(double tile_radius, int depth, double t_max = 1.75)
 		if (t_max * tile_radius + 3e-5 <= 0.7 / static_cast<double>(1 << k))
 			return k;
 	return 0;
+}
+
+// Refinement of a launch at level k (host side): t_fine, the latest stop time of the level-8 march at which a tile's beam
+// still fits a level-8 cell, rounded down to a float; 0 = no refinement.  Only launches at level kBeamMaxLevel get it: a
+// coarser launch level means R t_max > 0.7 2^-7, so the level-8 bound would hold over less than about half of the
+// longest stay in the cube, too little to pay for the 16 MiB grid.
+inline float beam_fine_t_limit(double tile_radius, int depth, int k)
+{
+	if (k != kBeamMaxLevel || depth < kBeamFineLevel || !(tile_radius > 0.0)) return 0.0f;
+	const double cell = 1.0 / static_cast<double>(1 << kBeamFineLevel), t = (0.7 * cell - 3e-5) / tile_radius;
+	if (!(t >= cell)) return 0.0f;
+	float f = static_cast<float>(t);
+	if (static_cast<double>(f) > t) f = std::nextafter(f, 0.0f);
+	return f;
 }
 
 // Longest stay in the cube [1,2]^3 of a ray from (ox, oy, oz) inside it: the distance to the farthest corner, widened
@@ -128,27 +155,32 @@ inline double rcp_table_rel_error(const uint32_t* tab, int log2n)
 	return worst;
 }
 
-// First parameter at which the ray o + t d (|d| = 1, o inside the cube) is inside a dilated-occupied cell of the grid, made
-// conservative; 0 when it starts in one; +inf when the whole tile has left the cube with nothing in sight.  Outside
-// the cube the grid continues as one ring of virtual cells that inherit the flag of the boundary cell next to them (the
-// inside cells around a virtual cell are among the 27 around that boundary cell): the tile's other rays may still be
-// inside while the central ray is up to one cell out, and not once it is further.
-__device__ __forceinline__ float beam_march(const BeamGrid g, float ox, float oy, float oz, float dx, float dy, float dz, int* steps = nullptr)
+// March of the ray o + t d (|d| = 1, o inside the cube) from t on (0: from the origin) to the first parameter at which it
+// is inside a dilated-occupied cell of the grid.  Returns that parameter, or with `left` set the time of the first sample
+// that lies more than a cell outside the cube with nothing met before; 0 when the march cannot start (NaN, the origin
+// outside); a time later than t_end as soon as it is clear that the march stops after t_end (the caller only wants to
+// know whether it stops by then).  Outside the cube the grid continues as one ring of virtual cells that inherit the flag
+// of the boundary cell next to them (the inside cells around a virtual cell are among the 27 around that boundary cell):
+// the tile's other rays may still be inside while the central ray is up to one cell out, and not once it is further.
+__device__ __forceinline__ float beam_march(const BeamGrid g, float ox, float oy, float oz, float dx, float dy, float dz, float t, float t_end, bool& left, int* steps)
 {
 	const int N = 1 << g.k;
 	const float fN = static_cast<float>(N), cell = 1.0f / fN;
 	const float inf = __uint_as_float(0x7F800000u);
 	const float ix_ = dx != 0.0f ? __fdiv_rn(1.0f, dx) : inf, iy_ = dy != 0.0f ? __fdiv_rn(1.0f, dy) : inf, iz_ = dz != 0.0f ? __fdiv_rn(1.0f, dz) : inf;
 	const float delta = 0x1p-19f;
-	float t = 0.0f;
+	left = false;
 	for (int it = 0; it < kBeamMaxSteps; ++it)
 	{
-		const float ts = it ? __fadd_rn(t, delta) : 0.0f;
+		const float ts = t > 0.0f ? __fadd_rn(t, delta) : 0.0f;
 		const float qx = __fmul_rn(__fsub_rn(__fmaf_rn(ts, dx, ox), 1.0f), fN), qy = __fmul_rn(__fsub_rn(__fmaf_rn(ts, dy, oy), 1.0f), fN),
 		            qz = __fmul_rn(__fsub_rn(__fmaf_rn(ts, dz, oz), 1.0f), fN);                      // position in cells
 		const float lim = __fadd_rn(fN, 1.0f);
 		if (!(qx >= -1.0f && qx < lim && qy >= -1.0f && qy < lim && qz >= -1.0f && qz < lim))
-			return it ? inf : 0.0f;                        // more than a cell outside (NaN: no beam start)
+		{
+			left = t > 0.0f;                               // more than a cell outside (at the origin: NaN, no beam start)
+			return left ? ts : 0.0f;
+		}
 		const int cx = static_cast<int>(floorf(qx)), cy = static_cast<int>(floorf(qy)), cz = static_cast<int>(floorf(qz));      // -1 .. N
 		const int bx = min(max(cx, 0), N - 1), by = min(max(cy, 0), N - 1), bz = min(max(cz, 0), N - 1);
 		const int s = g.skip[(static_cast<size_t>(bz) * N + by) * N + bx];
@@ -174,10 +206,10 @@ __device__ __forceinline__ float beam_march(const BeamGrid g, float ox, float oy
 		te = fminf(te, ey > t ? ey : __fmaf_rn(drift, fabsf(iy_), t));
 		te = fminf(te, ez > t ? ez : __fmaf_rn(drift, fabsf(iz_), t));
 		t = te > t ? te : __fadd_rn(t, delta);             // always forward
+		if (t > t_end) break;
 	}
 	// inside a dilated-occupied cell from t on (or out of steps): nothing before t
-	const float tau = __fsub_rn(__fmul_rn(t, 1.0f - 0x1p-12f), 0x1p-17f);
-	return tau > 0.0f ? tau : 0.0f;
+	return t;
 }
 
 // A tile whose march ends with +inf has nothing in sight; if, on top of that, every ray of the tile is certain to be in
@@ -189,9 +221,11 @@ __device__ __forceinline__ float beam_march(const BeamGrid g, float ox, float oy
 constexpr uint32_t kBeamAllMissBits = 0x7F800000u;        // +inf
 constexpr float kBeamNoneInSight = 3.0e38f;
 
-// start time of the 8 x 4 pixel tile whose first pixel is (x0, y0) of the frame: the ray through the tile's centre.
-// min_comp <= 0: never certify.
-__device__ __forceinline__ float beam_tile_start(const BeamGrid g, const Camera& c, int x0, int y0, float min_comp = 0.0f, int* steps = nullptr)
+// start time of the 8 x 4 pixel tile whose first pixel is (x0, y0) of the frame: the ray through the tile's centre, marched
+// on the launch's grid g and then, if the stop time is not later than fine_t (> 0: refinement on), on the level-8 grid
+// `fine` -- kept where that march also stops by fine_t.  min_comp <= 0: never certify.  steps: grid lookups (statistics).
+__device__ __forceinline__ float beam_tile_start(const BeamGrid g, const Camera& c, int x0, int y0, float min_comp = 0.0f, int* steps = nullptr,
+                                                 const BeamGrid fine = BeamGrid{ nullptr, 0 }, float fine_t = 0.0f)
 {
 	const float xc = static_cast<float>(x0) + 3.5f, yc = static_cast<float>(y0) + 1.5f;
 	const float u = __fmul_rn(c.aspect, __fsub_rn(__fmul_rn(c.vfx, xc), 1.0f));
@@ -202,11 +236,25 @@ __device__ __forceinline__ float beam_tile_start(const BeamGrid g, const Camera&
 	const float s = __fadd_rn(__fadd_rn(__fmul_rn(ru, ru), __fmul_rn(rv, rv)), __fmul_rn(rw, rw));
 	const float rm = __fdiv_rn(1.0f, __fsqrt_rn(s));
 	const float dx = __fmul_rn(rw, rm), dy = __fmul_rn(ru, rm), dz = __fmul_rn(-rv, rm);
-	const float tau = beam_march(g, c.ox, c.oy, c.oz, dx, dy, dz, steps);
-	if (__float_as_uint(tau) != kBeamAllMissBits)
-		return tau;
+	bool left;
+	float t = beam_march(g, c.ox, c.oy, c.oz, dx, dy, dz, 0.0f, __uint_as_float(0x7F800000u), left, steps);
+	if (!left && fine_t > 0.0f && t <= fine_t)
+	{
+		bool left_fine;
+		const float tf = beam_march(fine, c.ox, c.oy, c.oz, dx, dy, dz, t, fine_t, left_fine, steps);
+		if (tf <= fine_t)
+		{
+			t = tf;
+			left = left_fine;
+		}
+	}
+	if (!left)
+	{
+		const float tau = __fsub_rn(__fmul_rn(t, 1.0f - 0x1p-12f), 0x1p-17f);
+		return tau > 0.0f ? tau : 0.0f;
+	}
 	const bool certain = min_comp > 0.0f && fminf(fabsf(dx), fminf(fabsf(dy), fabsf(dz))) >= min_comp;
-	return certain ? tau : kBeamNoneInSight;
+	return certain ? __uint_as_float(kBeamAllMissBits) : kBeamNoneInSight;
 }
 
 // significant bits of a float's mantissa (1 for a power of two, 24 at most)

@@ -91,10 +91,10 @@ struct ort_ctx
 
 	// beam start (ort_beam.cuh): per level k one byte grid of the current DAG, built on demand by the first frame launch
 	// that needs it.  Two buffers per level, used in turn, so that launches still reading the grid of the previous DAG
-	// version (on other streams) are not overwritten by a rebuild.
-	uint8_t* d_beam_skip[8][2] = {};
-	int      beam_gen[8] = {};          // buffer of level k in use
-	bool     beam_valid[8] = {};        // grid of level k describes the current DAG
+	// version (on other streams) are not overwritten by a rebuild.  Level kBeamFineLevel is the refinement's grid.
+	uint8_t* d_beam_skip[9][2] = {};    // levels 0 .. ort::kBeamFineLevel
+	int      beam_gen[9] = {};          // buffer of level k in use
+	bool     beam_valid[9] = {};        // grid of level k describes the current DAG
 	uint8_t* d_beam_tmp = nullptr;      // occupancy + pyramid scratch of a build (largest level)
 	cudaEvent_t ev_beam = nullptr;      // last grid build done (builds share the scratch; launches on other streams wait for their grid)
 	bool     beam_built_once = false;
@@ -105,8 +105,8 @@ struct ort_ctx
 	int opt_band_order = 1;             // 1: frame launches schedule their bands by the costs recorded for the same view (BandMap)
 	uint64_t band_schedules = 0;        // schedules applied so far
 	int opt_beam = 1;                   // 1: camera frames of the lean tier start at their tile's beam bound
-	int opt_beam_level = 0;             // 0: the finest level the tile size allows; else forced (measurement)
-	int opt_count_beam = 0;             // 1: launches that return PUSH counts use the beam start too (counts = loads actually issued)
+	int opt_beam_level = 0;             // 0: the finest level the tile size allows, tiles refining on level 8; else forced, no refinement (measurement)
+	int opt_count_beam = 0;             // 1: launches that return PUSH counts use the beam start too (the launch's level alone); 2: with the level-8 refinement
 	int opt_beam_after = 2;             // frame launches a DAG version must have seen before a grid is built for it (edit loops: see beam_level_for_launch)
 	int beam_dag_age = 0;               // frame calls that have met the current DAG version (saturating)
 	uint64_t frame_call_seq = 0;        // public frame calls so far (a host-buffer frame is one call, however many chunk launches it makes)
@@ -244,7 +244,7 @@ void band_map_release(BandMap& m)
 // the DAG changed: every beam grid is out of date (rebuilt by the next frame launch that wants one)
 inline void beam_invalidate(ort_ctx* c)
 {
-	for (int k = 0; k < 8; ++k) c->beam_valid[k] = false;
+	for (bool& v : c->beam_valid) v = false;
 	c->beam_dag_age = 0;
 }
 
@@ -252,6 +252,8 @@ inline void beam_invalidate(ort_ctx* c)
 
 #include "ort_kernels.cuh"
 #include "ort_build.cuh"
+
+static_assert(ort::kBeamFineLevel == 8, "ort_ctx holds the beam grids of levels 0 .. 8");
 
 namespace {
 
@@ -312,6 +314,15 @@ int beam_level_for_launch(ort_ctx* c, const ort::Camera& cam, const ort::FrameRo
 	return c->beam_dag_age > c->opt_beam_after ? k : 0;
 }
 
+// Refinement of a launch that runs with the level-k grid (ort_beam.cuh, item 2): the time limit of its tiles' level-8
+// march, or 0 when it has none (a forced level, a launch level below 7, a DAG shallower than 8, a launch that returns PUSH
+// counts unless option count_beam is 2: with count_beam 1 the counts stay those of the launch-level start alone).
+float beam_fine_limit(const ort_ctx* c, const ort::Camera& cam, int k, bool counting)
+{
+	if (c->opt_beam_level >= ort::kBeamMinLevel || (counting && c->opt_count_beam < 2)) return 0.0f;
+	return ort::beam_fine_t_limit(ort::beam_tile_radius(cam, c->rcp_eps), c->depth, k);
+}
+
 // the same for the experiment kernels that bring their own walker (ORT_EXPERIMENTS builds): the selected variant is not
 // the product's, everything else decides as above
 int beam_level_any_variant(ort_ctx* c, const ort::Camera& cam, const ort::FrameRows& fr, bool counting)
@@ -323,40 +334,55 @@ int beam_level_any_variant(ort_ctx* c, const ort::Camera& cam, const ort::FrameR
 	return k;
 }
 
-// Make the level-k grid describe the current DAG; on return the launch stream is ordered after the build.
-int beam_ensure_grid(ort_ctx* c, int k)
+// Build the level-k grid of the current DAG into its spare buffer (on the launch stream, after the previous build).
+int beam_build_grid(ort_ctx* c, int k)
 {
 	const size_t cells = static_cast<size_t>(1) << (3 * k);
-	if (!c->beam_valid[k])
+	if (!c->d_beam_tmp)
 	{
-		if (!c->d_beam_tmp)
+		// occupancy of the finest level + the pyramid levels 1 .. kBeamFineLevel
+		size_t bytes = static_cast<size_t>(1) << (3 * ort::kBeamFineLevel);
+		for (int j = 1; j <= ort::kBeamFineLevel; ++j) bytes += static_cast<size_t>(1) << (3 * j);
+		ORT_CUDA(c, cudaMalloc(&c->d_beam_tmp, bytes));
+	}
+	const int gen = c->beam_gen[k] ^ 1;
+	if (!c->d_beam_skip[k][gen]) ORT_CUDA(c, cudaMalloc(&c->d_beam_skip[k][gen], cells));
+	// builds share the scratch: one after the other, whatever streams ask for them
+	if (c->beam_built_once) ORT_CUDA(c, cudaStreamWaitEvent(c->stream, c->ev_beam, 0));
+	uint8_t* occ = c->d_beam_tmp;
+	uint8_t* pyr = c->d_beam_tmp + (static_cast<size_t>(1) << (3 * ort::kBeamFineLevel));
+	size_t off[ort::kBeamFineLevel + 2] = {};
+	for (int j = 1; j <= k; ++j) off[j + 1] = off[j] + (static_cast<size_t>(1) << (3 * j));      // level j at off[j]
+	const ort::Dag dag = make_dag(c);
+	const unsigned blocks = static_cast<unsigned>((cells + 255) / 256);
+	ort::beam_occupancy_kernel<<<blocks, 256, 0, c->stream>>>(dag.nodes_m1, dag.root, k, occ);
+	ort::beam_dilate_kernel<<<blocks, 256, 0, c->stream>>>(occ, k, pyr + off[k]);
+	for (int j = k - 1; j >= 1; --j)
+		ort::beam_reduce_kernel<<<static_cast<unsigned>(((static_cast<size_t>(1) << (3 * j)) + 255) / 256), 256, 0, c->stream>>>(pyr + off[j + 1], j, pyr + off[j]);
+	ort::beam_skip_kernel<<<blocks, 256, 0, c->stream>>>(pyr, k, c->d_beam_skip[k][gen]);
+	c->launches += 3 + (k - 1);
+	ORT_CUDA(c, cudaGetLastError());
+	ORT_CUDA(c, cudaEventRecord(c->ev_beam, c->stream));
+	c->beam_built_once = true;
+	c->beam_gen[k] = gen;
+	c->beam_valid[k] = true;
+	return ORT_OK;
+}
+
+// Make the level-k grid (and with `fine` the refinement's level-8 grid) describe the current DAG; on return the launch
+// stream is ordered after the build.  The grids one call builds count as one build (ort_beam_builds).
+int beam_ensure_grid(ort_ctx* c, int k, bool fine = false)
+{
+	bool built = false;
+	for (const int level : { k, fine ? ort::kBeamFineLevel : k })
+		if (!c->beam_valid[level])
 		{
-			// occupancy of the finest level + the pyramid levels 1 .. kBeamMaxLevel
-			size_t bytes = static_cast<size_t>(1) << (3 * ort::kBeamMaxLevel);
-			for (int j = 1; j <= ort::kBeamMaxLevel; ++j) bytes += static_cast<size_t>(1) << (3 * j);
-			ORT_CUDA(c, cudaMalloc(&c->d_beam_tmp, bytes));
+			const int rc = beam_build_grid(c, level);
+			if (rc != ORT_OK) return rc;
+			built = true;
 		}
-		const int gen = c->beam_gen[k] ^ 1;
-		if (!c->d_beam_skip[k][gen]) ORT_CUDA(c, cudaMalloc(&c->d_beam_skip[k][gen], cells));
-		// builds share the scratch: one after the other, whatever streams ask for them
-		if (c->beam_built_once) ORT_CUDA(c, cudaStreamWaitEvent(c->stream, c->ev_beam, 0));
-		uint8_t* occ = c->d_beam_tmp;
-		uint8_t* pyr = c->d_beam_tmp + (static_cast<size_t>(1) << (3 * ort::kBeamMaxLevel));
-		size_t off[ort::kBeamMaxLevel + 2] = {};
-		for (int j = 1; j <= k; ++j) off[j + 1] = off[j] + (static_cast<size_t>(1) << (3 * j));      // level j at off[j]
-		const ort::Dag dag = make_dag(c);
-		const unsigned blocks = static_cast<unsigned>((cells + 255) / 256);
-		ort::beam_occupancy_kernel<<<blocks, 256, 0, c->stream>>>(dag.nodes_m1, dag.root, k, occ);
-		ort::beam_dilate_kernel<<<blocks, 256, 0, c->stream>>>(occ, k, pyr + off[k]);
-		for (int j = k - 1; j >= 1; --j)
-			ort::beam_reduce_kernel<<<static_cast<unsigned>(((static_cast<size_t>(1) << (3 * j)) + 255) / 256), 256, 0, c->stream>>>(pyr + off[j + 1], j, pyr + off[j]);
-		ort::beam_skip_kernel<<<blocks, 256, 0, c->stream>>>(pyr, k, c->d_beam_skip[k][gen]);
-		c->launches += 3 + (k - 1);
-		ORT_CUDA(c, cudaGetLastError());
-		ORT_CUDA(c, cudaEventRecord(c->ev_beam, c->stream));
-		c->beam_built_once = true;
-		c->beam_gen[k] = gen;
-		c->beam_valid[k] = true;
+	if (built)
+	{
 		++c->beam_builds;
 		return ORT_OK;
 	}
@@ -366,13 +392,16 @@ int beam_ensure_grid(ort_ctx* c, int k)
 }
 
 // the march over the tiles of one frame launch; `tile_word` = the output array that carries the start times
-int beam_launch_march(ort_ctx* c, int k, const ort::Camera& cam, const ort::FrameRows& fr, float* tile_word)
+int beam_launch_march(ort_ctx* c, int k, const ort::Camera& cam, const ort::FrameRows& fr, float* tile_word, bool counting)
 {
-	const int rc = beam_ensure_grid(c, k);
+	const float fine_t = beam_fine_limit(c, cam, k, counting);
+	const int rc = beam_ensure_grid(c, k, fine_t > 0.0f);
 	if (rc != ORT_OK) return rc;
 	const unsigned tiles = static_cast<unsigned>(((fr.W + 7) / 8) * ((fr.rows + 3) / 4));
 	const float min_comp = ort::beam_certify_min_comp(cam, ort::beam_tile_radius(cam, c->rcp_eps), c->rcp_sig_bits);
-	ort::beam_start_kernel<<<(tiles + 127) / 128, 128, 0, c->stream>>>(ort::BeamGrid{ c->d_beam_skip[k][c->beam_gen[k]], k }, cam, fr, min_comp, tile_word);
+	const int kf = ort::kBeamFineLevel;
+	ort::beam_start_kernel<<<(tiles + 127) / 128, 128, 0, c->stream>>>(ort::BeamGrid{ c->d_beam_skip[k][c->beam_gen[k]], k },
+	                                                                   ort::BeamGrid{ c->d_beam_skip[kf][c->beam_gen[kf]], kf }, fine_t, cam, fr, min_comp, tile_word);
 	++c->launches;
 	ORT_CUDA(c, cudaGetLastError());
 	return ORT_OK;
@@ -649,7 +678,7 @@ int ort_destroy(ort_ctx* c)
 	cudaFree(c->d_stage);
 	for (BandMap& m : c->band_maps) band_map_release(m);
 	cudaFree(c->d_beam_tmp);
-	for (int k = 0; k < 8; ++k) { cudaFree(c->d_beam_skip[k][0]); cudaFree(c->d_beam_skip[k][1]); }
+	for (int k = 0; k <= ort::kBeamFineLevel; ++k) { cudaFree(c->d_beam_skip[k][0]); cudaFree(c->d_beam_skip[k][1]); }
 	if (c->ev_beam) cudaEventDestroy(c->ev_beam);
 	for (int i = 0; i < 2; ++i)
 	{
@@ -1225,7 +1254,7 @@ int ort_trace_frame_async(ort_ctx* c, const float pos[3], const float rot[9], fl
 	const int bk = beam_level_for_launch(c, cam, fr, npush != nullptr);
 	if (bk)
 	{
-		const int rc = beam_launch_march(c, bk, cam, fr, t);
+		const int rc = beam_launch_march(c, bk, cam, fr, t, npush != nullptr);
 		if (rc != ORT_OK) return rc;
 	}
 	// band schedule of this view (launches of 8 bands and more; the frame kernels of the product walks)
@@ -1298,6 +1327,7 @@ int ort_trace_frames_async(ort_ctx* c, const ort_frame_job* jobs, int n_jobs)
 			d.fr = ort::FrameRows{ j.W, j.H, j.y0, j.rows, j.tile_rows, j.tile_step, 0, rotate, ort::tile_shift_of(j.tile_rows) };
 			d.voxel = j.voxel; d.face = j.face; d.t = j.t; d.npush = j.npush;
 			d.beam_k = 0;
+			d.beam_fine_t = 0.0f;
 			gx = std::max(gx, static_cast<unsigned>((j.W + 15) / 16));
 			gy = std::max(gy, static_cast<unsigned>((j.rows + 15) / 16));
 		}
@@ -1312,6 +1342,7 @@ int ort_trace_frames_async(ort_ctx* c, const ort_frame_job* jobs, int n_jobs)
 			ort::FrameJob& d = batch.job[k];
 			d.beam_k = beam_level_for_launch(c, d.cam, d.fr, count);
 			d.beam_min_comp = ort::beam_certify_min_comp(d.cam, ort::beam_tile_radius(d.cam, c->rcp_eps), c->rcp_sig_bits);
+			d.beam_fine_t = beam_fine_limit(c, d.cam, d.beam_k, count);
 			beam = d.beam_k != 0;
 			max_tiles = std::max(max_tiles, static_cast<unsigned>(((d.fr.W + 7) / 8) * ((d.fr.rows + 3) / 4)));
 		}
@@ -1320,17 +1351,19 @@ int ort_trace_frames_async(ort_ctx* c, const ort_frame_job* jobs, int n_jobs)
 			ort::BeamGridSet grids{};
 			for (int k = 0; k < n; ++k)
 			{
-				const int bk = batch.job[k].beam_k;
-				const int rc = beam_ensure_grid(c, bk);
+				const int bk = batch.job[k].beam_k, kf = ort::kBeamFineLevel;
+				const bool fine = batch.job[k].beam_fine_t > 0.0f;
+				const int rc = beam_ensure_grid(c, bk, fine);
 				if (rc != ORT_OK) return rc;
 				grids.skip[bk] = c->d_beam_skip[bk][c->beam_gen[bk]];
+				if (fine) grids.skip[kf] = c->d_beam_skip[kf][c->beam_gen[kf]];
 			}
 			ort::beam_start_batch_kernel<<<dim3((max_tiles + 127) / 128, static_cast<unsigned>(n)), 128, 0, c->stream>>>(grids, batch);
 			++c->launches;
 			ORT_CUDA(c, cudaGetLastError());
 		}
 		else
-			for (int k = 0; k < n; ++k) batch.job[k].beam_k = 0;
+			for (int k = 0; k < n; ++k) { batch.job[k].beam_k = 0; batch.job[k].beam_fine_t = 0.0f; }
 		const dim3 bgrid(gx, gy, static_cast<unsigned>(n));
 #define ORT_LAUNCH_BATCH(V, C, B) ort::trace_frames_kernel<V, C, B><<<bgrid, 256, (V) == ort::kLean ? smem : 0, c->stream>>>(dag, batch)
 		switch (walk_variant(c))
@@ -1614,7 +1647,7 @@ static int launch_frame_rgba(ort_ctx* c, const float pos[3], const float rot[9],
 	const int bk = beam_level_for_launch(c, cam, fr, false);
 	if (bk)
 	{
-		const int rc = beam_launch_march(c, bk, cam, fr, reinterpret_cast<float*>(d_rgba));
+		const int rc = beam_launch_march(c, bk, cam, fr, reinterpret_cast<float*>(d_rgba), false);
 		if (rc != ORT_OK) return rc;
 	}
 	switch (walk_variant(c))
@@ -1797,8 +1830,8 @@ int ort_beam_level(ort_ctx* c, const float pos[3], const float rot[9], float fov
 int ort_beam_grid(ort_ctx* c, int level, uint8_t* skip_out)
 {
 	enter(c);
-	if (!c || !skip_out || level < 1 || level > ort::kBeamMaxLevel || level > c->depth)
-		return ort_fail(c, ORT_ERR_INVALID, "ort_beam_grid: level must be 1..min(depth, %d)", ort::kBeamMaxLevel);
+	if (!c || !skip_out || level < 1 || level > ort::kBeamFineLevel || level > c->depth)
+		return ort_fail(c, ORT_ERR_INVALID, "ort_beam_grid: level must be 1..min(depth, %d)", ort::kBeamFineLevel);
 	if (!c->has_root)
 		return ort_fail(c, ORT_ERR_INVALID, "ort_beam_grid: no DAG on the device");
 	DeviceGuard g(c->device);

@@ -578,7 +578,7 @@ static int launch_frame_experiment(ort_ctx* c, const ort::Dag& g, const ort::Cam
 		const size_t smem = ort::lean_smem_bytes(g.depth);
 		if (bk)
 		{
-			const int rc = beam_launch_march(c, bk, cam, fr, t);
+			const int rc = beam_launch_march(c, bk, cam, fr, t, npush != nullptr);
 			if (rc != ORT_OK) return ORT_ERR_CUDA;
 #define ORT_BEAM_KERNEL(W, L) (npush ? ort::trace_frame_walker_beam_kernel<W, true, L> : ort::trace_frame_walker_beam_kernel<W, false, L>)
 			// 28-31: the product's walker and loop with the guard as a slow-path call / without a guard / other register budgets

@@ -242,14 +242,15 @@ trace_frame_kernel(const Dag g, Camera cam, FrameRows fr,
 // The march of the beam start (ort_beam.cuh), one thread per 8 x 4 pixel tile of the rows a frame launch traces: the tile's
 // start time goes into the output word of its first pixel -- `t` for the voxel / face / t kernels, the pixel for the
 // shaded kernel -- where the trace kernel picks it up.
+// fine / fine_t: the level-8 grid and the time limit of the refinement (fine_t = 0: none).
 __global__ void __launch_bounds__(128)
-beam_start_kernel(const BeamGrid grid, Camera cam, FrameRows fr, float min_comp, float* __restrict__ tile_word)
+beam_start_kernel(const BeamGrid grid, const BeamGrid fine, float fine_t, Camera cam, FrameRows fr, float min_comp, float* __restrict__ tile_word)
 {
 	const int tiles_x = (fr.W + 7) >> 3, tiles_y = (fr.rows + 3) >> 2;
 	const int i = blockIdx.x * blockDim.x + threadIdx.x;
 	if (i >= tiles_x * tiles_y) return;
 	const int x0 = (i % tiles_x) * 8, r0 = (i / tiles_x) * 4;
-	tile_word[static_cast<size_t>(r0) * fr.W + x0] = beam_tile_start(grid, cam, x0, frame_row(fr, r0), min_comp);
+	tile_word[static_cast<size_t>(r0) * fr.W + x0] = beam_tile_start(grid, cam, x0, frame_row(fr, r0), min_comp, nullptr, fine, fine_t);
 }
 
 // Several frame jobs in ONE launch (blockIdx.z = job): strips of different frames, or the views of a multi-camera
@@ -267,6 +268,7 @@ struct FrameJob
 	uint16_t* npush;    // may be null
 	int       beam_k;   // level of the beam grid this job's tile starts come from (0: the job runs without)
 	float     beam_min_comp;   // beam_certify_min_comp() of the job's camera
+	float     beam_fine_t;     // beam_fine_t_limit() of the job's camera: its tiles refine their start on the level-8 grid (0: not)
 };
 
 struct FrameJobBatch
@@ -308,10 +310,11 @@ trace_frames_kernel(const Dag g, const __grid_constant__ FrameJobBatch batch)
 	if (COUNT && jb.npush) jb.npush[i] = static_cast<uint16_t>(min(h.npush, 65535u));
 }
 
-// the march for every job of a batch (blockIdx.y = job); grids[k] = the context's grid of level k
+// the march for every job of a batch (blockIdx.y = job); grids[k] = the context's grid of level k (kBeamFineLevel: the
+// refinement's, where some job refines)
 struct BeamGridSet
 {
-	const uint8_t* skip[kBeamMaxLevel + 1];
+	const uint8_t* skip[kBeamFineLevel + 1];
 };
 
 __global__ void __launch_bounds__(128)
@@ -324,7 +327,8 @@ beam_start_batch_kernel(const BeamGridSet grids, const __grid_constant__ FrameJo
 	const int i = blockIdx.x * blockDim.x + threadIdx.x;
 	if (i >= tiles_x * tiles_y) return;
 	const int x0 = (i % tiles_x) * 8, r0 = (i / tiles_x) * 4;
-	jb.t[static_cast<size_t>(r0) * fr.W + x0] = beam_tile_start(BeamGrid{ grids.skip[jb.beam_k], jb.beam_k }, jb.cam, x0, frame_row(fr, r0), jb.beam_min_comp);
+	jb.t[static_cast<size_t>(r0) * fr.W + x0] = beam_tile_start(BeamGrid{ grids.skip[jb.beam_k], jb.beam_k }, jb.cam, x0, frame_row(fr, r0), jb.beam_min_comp, nullptr,
+	                                                               BeamGrid{ grids.skip[kBeamFineLevel], kBeamFineLevel }, jb.beam_fine_t);
 }
 
 // Shading epilogue (tree_camera::trace_pixel, test_och_h_octree.cpp:76-84) fused into the frame kernel: the hit is

@@ -79,32 +79,34 @@ void beam_walk(const uint32_t* nodes8, uint32_t root, int depth, const float* o,
 }
 
 // Entry parameter of the first occupied cell of a (dilated) level-k bitmap along the ray o + t * d (world coordinates,
-// cube [1,2)^3), plain 3-D DDA in double precision; +inf when the ray leaves the cube first.  occ: (2^k)^3 bytes, index
-// (z * N + y) * N + x.
-void beam_dda(const uint8_t* occ, int k, const float* o, const double* d, size_t n, double* t_entry)
+// cube [1,2)^3) from t0[r] on (NULL: from 0), plain 3-D DDA in double precision; +inf when the ray leaves the cube first,
+// and then t_exit[r] (if not NULL) = the parameter at which it leaves.  occ: (2^k)^3 bytes, index (z * N + y) * N + x.
+void beam_dda(const uint8_t* occ, int k, const float* o, const double* d, const double* t0, size_t n, double* t_entry, double* t_exit)
 {
 	const int N = 1 << k;
 	for (size_t r = 0; r < n; ++r)
 	{
 		int c[3], step[3];
 		double tnext[3], dt[3];
+		const double ts = t0 ? t0[r] : 0.0;
 		for (int a = 0; a < 3; ++a)
 		{
-			const double p = ((double)o[a] - 1.0) * N;
+			const double da = d[3 * r + a];
+			const double p = ((double)o[a] + ts * da - 1.0) * N;
 			c[a] = (int)floor(p);
 			if (c[a] < 0) c[a] = 0;
 			if (c[a] >= N) c[a] = N - 1;
-			const double da = d[3 * r + a];
 			step[a] = da > 0 ? 1 : -1;
 			if (da == 0.0) { tnext[a] = INFINITY; dt[a] = INFINITY; }
 			else
 			{
 				const double edge = da > 0 ? (c[a] + 1) : c[a];
-				tnext[a] = (edge - p) / (da * N);
+				tnext[a] = ts + (edge - p) / (da * N);
 				dt[a] = 1.0 / (fabs(da) * N);
 			}
 		}
-		double t = 0.0;
+		double t = ts;
+		if (t_exit) t_exit[r] = INFINITY;
 		for (;;)
 		{
 			if (occ[((size_t)c[2] * N + c[1]) * N + c[0]]) { t_entry[r] = t; break; }
@@ -112,7 +114,7 @@ void beam_dda(const uint8_t* occ, int k, const float* o, const double* d, size_t
 			t = tnext[a];
 			c[a] += step[a];
 			tnext[a] += dt[a];
-			if (c[a] < 0 || c[a] >= N) { t_entry[r] = INFINITY; break; }
+			if (c[a] < 0 || c[a] >= N) { t_entry[r] = INFINITY; if (t_exit) t_exit[r] = t; break; }
 		}
 	}
 }

@@ -3,6 +3,7 @@ how many PUSH rounds of the reference walk lie before a tile-wide conservative s
 level-k occupancy grid, and at which level the walk would be re-entered.  python tools/beam/beam_model.py [k] [tile_w tile_h]"""
 import ctypes as C
 import os
+import re
 import subprocess
 import sys
 
@@ -16,6 +17,7 @@ from oracle import oracle as oc
 
 K = int(sys.argv[1]) if len(sys.argv) > 1 else 6
 TW, TH = (int(sys.argv[2]), int(sys.argv[3])) if len(sys.argv) > 3 else (8, 4)
+FINE = int(sys.argv[4]) if len(sys.argv) > 4 else 0
 DEPTH, W, H = 12, 3840, 2160
 so = "/tmp/libbeam_model.so"
 subprocess.check_call(["gcc", "-O2", "-shared", "-fPIC", "-ffp-contract=off", "-o", so, os.path.join(ROOT, "tools/beam/beam_model.c"), "-lm"])
@@ -27,26 +29,43 @@ harness.build_terrain(tree)
 nodes8, root, _ = tree.flatten()
 nodes8 = np.ascontiguousarray(nodes8, np.uint32)
 
-# occupancy of level k: ids[z, y, x] of the level-l cells, expanded level by level
-ids = np.array([[[root]]], np.uint32)
-for l in range(K):
-    n = ids.shape[0]
-    nxt = np.zeros((2 * n, 2 * n, 2 * n), np.uint32)
-    ch = np.where(ids[..., None] != 0, nodes8[np.maximum(ids, 1) - 1], 0)          # (n, n, n, 8)
-    for s in range(8):
-        nxt[(s >> 2 & 1)::2, (s >> 1 & 1)::2, (s & 1)::2] = ch[..., s]
-    ids = nxt
-occ = ids != 0
+
+def dilated_grid(k):
+    """occupancy of level k (ids[z, y, x] of the level-l cells, expanded level by level), dilated by one cell"""
+    ids = np.array([[[root]]], np.uint32)
+    for l in range(k):
+        n = ids.shape[0]
+        nxt = np.zeros((2 * n, 2 * n, 2 * n), np.uint32)
+        ch = np.where(ids[..., None] != 0, nodes8[np.maximum(ids, 1) - 1], 0)          # (n, n, n, 8)
+        for s in range(8):
+            nxt[(s >> 2 & 1)::2, (s >> 1 & 1)::2, (s & 1)::2] = ch[..., s]
+        ids = nxt
+    occ = ids != 0
+    N = 1 << k
+    print(f"level {k}: {occ.sum()} of {N**3} cells occupied")
+    dil = np.zeros_like(occ)
+    pad = np.pad(occ, 1)
+    for dz in range(3):
+        for dy in range(3):
+            for dx in range(3):
+                dil |= pad[dz:dz + N, dy:dy + N, dx:dx + N]
+    print(f"dilated: {dil.sum()} cells")
+    return np.ascontiguousarray(dil, np.uint8)
+
+
+def rcp_eps():
+    """largest relative error of the library's reciprocal table (ort::rcp_table_rel_error)"""
+    txt = open(os.path.join(ROOT, "octree_ray_tracing_b200", "csrc", "ort_rcp_table.h")).read()
+    tab = np.array([int(x, 16) for x in re.findall(r"0x([0-9a-f]{8})u", txt)], np.uint32).view(np.float32).astype(np.float64)
+    n = len(tab)
+    lo, hi = 1.0 + np.arange(n) / n, 1.0 + np.arange(1, n + 1) / n
+    return float(np.maximum(np.abs(tab * lo - 1.0), np.abs(tab * hi - 1.0)).max())
+
+
+dil8 = dilated_grid(K)
 N = 1 << K
-print(f"level {K}: {occ.sum()} of {N**3} cells occupied")
-dil = np.zeros_like(occ)
-pad = np.pad(occ, 1)
-for dz in range(3):
-    for dy in range(3):
-        for dx in range(3):
-            dil |= pad[dz:dz + N, dy:dy + N, dx:dx + N]
-print(f"dilated: {dil.sum()} cells")
-dil8 = np.ascontiguousarray(dil, np.uint8)
+fine = dilated_grid(FINE) if FINE else None
+EPS = rcp_eps()
 
 step = 4       # every step-th tile in x and y
 for name in "ABC":
@@ -57,6 +76,10 @@ for name in "ABC":
     miss_free = 0
     worst = 0.0
     lv_hist = np.zeros(16, np.int64)
+    refined = tiles = 0
+    # the library's tile radius R (ort::beam_tile_radius): 3.5 x 1.5 pixels from the tile's centre, the table's error
+    du, dv = 3.5 * (W / H) * (2.0 / W), 1.5 * (2.0 / H)
+    R = 1.01 * np.hypot(du, dv) / fov + EPS + 1e-6
     for ty in range(0, H // TH, step):
         rows = oc.gen_rays(rot, fov, W, H, ty * TH, ty * TH + TH).reshape(TH, W, 3)
         txs = np.arange(0, W // TW, step)
@@ -65,7 +88,18 @@ for name in "ABC":
         dc /= np.linalg.norm(dc, axis=1, keepdims=True)
         dev = np.linalg.norm(d.astype(np.float64) / np.linalg.norm(d.astype(np.float64), axis=2, keepdims=True) - dc[:, None, :], axis=2).max(axis=1)
         te = np.zeros(len(txs), np.float64)
-        L.beam_dda(p(dil8), K, p(o), p(np.ascontiguousarray(dc)), C.c_size_t(len(txs)), p(te))
+        dc = np.ascontiguousarray(dc)
+        L.beam_dda(p(dil8), K, p(o), p(dc), None, C.c_size_t(len(txs)), p(te), None)
+        fin = np.isfinite(te)
+        tiles += len(txs)
+        if FINE:
+            tf = np.zeros(len(txs), np.float64)
+            tx_ = np.zeros(len(txs), np.float64)
+            L.beam_dda(p(fine), FINE, p(o), p(dc), p(np.ascontiguousarray(np.where(fin, te, 0.0))), C.c_size_t(len(txs)), p(tf), p(tx_))
+            stop = np.where(np.isfinite(tf), tf, tx_)
+            ok = fin & (R * stop + 3e-5 <= 0.7 * 2.0 ** -FINE)
+            te = np.where(ok, tf, te)
+            refined += int(ok.sum())
         fin = np.isfinite(te)
         worst = max(worst, float((np.where(fin, te, 1.8) * (dev + 4e-4)).max() * N))       # beam radius at t0 in level-k cells (must stay < 1)
         t0 = np.repeat((te * (1 - 1e-3)).astype(np.float32), TW * TH)
@@ -82,4 +116,5 @@ for name in "ABC":
         tot_r += int(rounds.sum()); tot_after += int(new.sum()); tot_n += n
         np.add.at(lv_hist, at_l[found], 1)
     print(f"pose {name}: rounds/ray {tot_r / tot_n:.2f} -> {tot_after / tot_n:.2f} ({tot_after / tot_r:.3f}); rays that become a MISS without a round: {miss_free / tot_n:.3f}; "
-          f"beam radius at t0 <= {worst:.2f} level-{K} cells; re-entry level histogram {lv_hist[1:13].tolist()}")
+          f"beam radius at t0 <= {worst:.2f} level-{K} cells; re-entry level histogram {lv_hist[1:13].tolist()}"
+          + (f"; tiles refined on level {FINE}: {refined / tiles:.3f} (R = {R:.3g}, up to t = {(0.7 * 2.0 ** -FINE - 3e-5) / R:.3f})" if FINE else ""))
