@@ -110,6 +110,25 @@ int ort_read_nodes(ort_ctx* ctx, uint32_t first, size_t n, uint32_t* nodes8);
  * (nothing is freed before the build ends, so this is its peak on top of what the context held). */
 uint64_t ort_build_bytes(const ort_ctx* ctx);
 
+/* Replaces: n calls of at(x, y, z) (och_h_octree.h:239-258; och::octree::at, och_octree.cpp:141-160) on the DAG
+ * currently on ctx's device, in either layout (h_octree compact ids or och::octree pool rows).  xyz: n triples x, y, z;
+ * out[i] = the voxel at triple i, bit for bit what at() returns on a table holding the mirrored DAG.  Coordinate rule
+ * (at()'s): each coordinate is cast to uint16 and only its low `depth` bits choose the cell, so negative coordinates and
+ * coordinates >= 2^depth (or >= 65536) wrap around the cube.  A context that holds no tree (never uploaded to, or an
+ * h_octree mirror with root 0) reads 0 everywhere; a pool mirror is walked from row 0.  A child id past the mirror's
+ * rows reads as empty: the walk never loads outside them.
+ * Pointers may be host (pageable or pinned) or device memory, in any mix; device buffers must be 4-byte aligned.  With
+ * both on the device the call only enqueues on ort_stream(ctx); otherwise it returns when out holds the result (host
+ * buffers go through device staging in chunks of at most 64 MiB).  n == 0 does nothing.  ORT_ERR_INVALID for a null
+ * context, a null buffer with n > 0 or a misaligned device buffer. */
+int ort_voxels_at(ort_ctx* ctx, const int32_t* xyz, size_t n, uint32_t* out);
+/* The voxels of the box [x0, x0+nx) x [y0, y0+ny) x [z0, z0+nz) of the device DAG, as uint32.
+ * Index (z*ny + y)*nx + x relative to the box origin, the layout ort_build_voxels reads.  The box does not wrap: it
+ * needs 0 <= x0, nx >= 1 and x0 + nx <= 2^depth on each axis, else ORT_ERR_INVALID and nothing is written.  Same
+ * content rules, pointers and completion as ort_voxels_at; a host output is staged in chunks of whole output rows of at
+ * most 64 MiB, so a large box never needs a device buffer of its size. */
+int ort_read_voxels(ort_ctx* ctx, int x0, int y0, int z0, int nx, int ny, int nz, uint32_t* out);
+
 /* Replaces: N calls of sse_trace(ox,oy,oz,dx,dy,dz, direction&, uint32_t&, float&) const
  * (och_h_octree.h:292-447).  o3: origins, 3 floats each, o_stride = 3, or ONE shared origin with
  * o_stride = 0.  d3: n directions.  Outputs per ray: voxel = hit_voxel, face = hit_direction,

@@ -252,6 +252,7 @@ inline void beam_invalidate(ort_ctx* c)
 
 #include "ort_kernels.cuh"
 #include "ort_build.cuh"
+#include "ort_query.cuh"
 
 static_assert(ort::kBeamFineLevel == 8, "ort_ctx holds the beam grids of levels 0 .. 8");
 
@@ -1073,6 +1074,172 @@ int ort_read_nodes(ort_ctx* c, uint32_t first, size_t n, uint32_t* nodes8)
 }
 
 uint64_t ort_build_bytes(const ort_ctx* c) { return c ? c->build_bytes : 0; }
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// voxels read back from the device DAG (ort_query.cuh, DESIGN section 14)
+// ------------------------------------------------------------------------------------------------
+
+namespace {
+
+constexpr size_t kQueryStageBytes = size_t(64) << 20;       // one staging slot of a host-buffer query
+
+ort::QueryDag query_dag(const ort_ctx* c)
+{
+	const ort::Dag d = make_dag(c);
+	return ort::QueryDag{ d.nodes_m1, d.root, c->has_root ? c->n_nodes + c->index_base : 0u, c->depth };
+}
+
+// The next staging slot of a host-buffer query: ordered on c->stream after whatever an earlier call (a deferred frame
+// among them) still reads from it or copies out of it.
+int query_slot(ort_ctx* c, char** base)
+{
+	const int slot = c->next_slot;
+	c->next_slot ^= 1;
+	if (c->slot_used[slot])
+	{
+		ORT_CUDA(c, cudaStreamWaitEvent(c->stream, c->ev_chunk[slot], 0));
+		ORT_CUDA(c, cudaStreamWaitEvent(c->stream, c->ev_copied[slot], 0));
+	}
+	*base = stage_slot(c, slot);
+	return slot;
+}
+
+// After the slot's kernel on c->stream: copy its `bytes` of results to `host` on copy_stream (bytes 0: nothing to copy)
+// and mark the slot busy until then.
+int query_slot_done(ort_ctx* c, int slot, void* host, const void* staged, size_t bytes)
+{
+	ORT_CUDA(c, cudaEventRecord(c->ev_chunk[slot], c->stream));
+	ORT_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_chunk[slot], 0));
+	if (bytes) ORT_CUDA(c, cudaMemcpyAsync(host, staged, bytes, cudaMemcpyDeviceToHost, c->copy_stream));
+	ORT_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
+	c->slot_used[slot] = true;
+	return ORT_OK;
+}
+
+int launch_voxels_at(ort_ctx* c, const int32_t* d_xyz, size_t n, uint32_t* d_out)
+{
+	const unsigned blocks = static_cast<unsigned>(std::min<size_t>((n + 255) / 256, static_cast<size_t>(c->sm_count) * 8));
+	ort::voxels_at_kernel<<<blocks, 256, 0, c->stream>>>(query_dag(c), d_xyz, n, d_out);
+	++c->launches;
+	ORT_CUDA(c, cudaGetLastError());
+	return ORT_OK;
+}
+
+// the box b (inside the cube) into d_out, densely
+int launch_read_voxels(ort_ctx* c, const ort::QueryBox& b, uint32_t* d_out)
+{
+	const uint32_t cx0 = b.x0 >> 1, ncx = ((b.x0 + b.nx - 1) >> 1) - cx0 + 1;
+	const uint32_t cy0 = b.y0 >> 1, ncy = ((b.y0 + b.ny - 1) >> 1) - cy0 + 1;
+	const uint32_t cz0 = b.z0 >> 1, ncz = ((b.z0 + b.nz - 1) >> 1) - cz0 + 1;
+	const uint32_t rows = ncy * ncz;
+	uint32_t bx = 1;
+	while (bx < ncx && bx < 256) bx <<= 1;
+	const uint32_t by = 256 / bx, gx = (ncx + bx - 1) / bx;
+	const uint32_t want = static_cast<uint32_t>(c->sm_count) * 8 / gx + 1;        // about 8 blocks of 256 per SM in all
+	const uint32_t gy = std::min<uint32_t>(std::min<uint32_t>((rows + by - 1) / by, want), 65535u);
+	ort::read_voxels_kernel<<<dim3(gx, gy), dim3(bx, by), 0, c->stream>>>(query_dag(c), b, d_out, cx0, ncx, cy0, ncy, cz0, rows);
+	++c->launches;
+	ORT_CUDA(c, cudaGetLastError());
+	return ORT_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ort_voxels_at(ort_ctx* c, const int32_t* xyz, size_t n, uint32_t* out)
+{
+	enter(c);
+	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_voxels_at: null context");
+	if (!n) return ORT_OK;
+	if (!xyz || !out) return ort_fail(c, ORT_ERR_INVALID, "ort_voxels_at: null buffer");
+	DeviceGuard g(c->device);
+	const bool in_dev = is_device_ptr(xyz), out_dev = is_device_ptr(out);
+	if ((in_dev && (reinterpret_cast<uintptr_t>(xyz) & 3u)) || (out_dev && (reinterpret_cast<uintptr_t>(out) & 3u)))
+		return ort_fail(c, ORT_ERR_INVALID, "ort_voxels_at: device buffers must be 4-byte aligned");
+	if (in_dev && out_dev) return launch_voxels_at(c, xyz, n, out);          // enqueue only
+
+	// host buffers: chunks of at most kQueryStageBytes of points and results per staging slot
+	const size_t cn = std::min(n, kQueryStageBytes / 16);
+	const size_t off_out = align_up(cn * 12, 256);
+	int rc = ensure_dstage(c, 2 * align_up(off_out + cn * 4, 256));
+	if (rc != ORT_OK) return rc;
+	for (size_t first = 0; first < n; first += cn)
+	{
+		const size_t m = std::min(cn, n - first);
+		char* base = nullptr;
+		const int slot = query_slot(c, &base);
+		const int32_t* d_xyz = xyz + 3 * first;
+		if (!in_dev)
+		{
+			ORT_CUDA(c, cudaMemcpyAsync(base, d_xyz, m * 12, cudaMemcpyHostToDevice, c->stream));
+			d_xyz = reinterpret_cast<const int32_t*>(base);
+		}
+		uint32_t* d_out = out_dev ? out + first : reinterpret_cast<uint32_t*>(base + off_out);
+		if ((rc = launch_voxels_at(c, d_xyz, m, d_out)) != ORT_OK) return rc;
+		if ((rc = query_slot_done(c, slot, out + first, d_out, out_dev ? 0 : m * 4)) != ORT_OK) return rc;
+	}
+	ORT_CUDA(c, cudaStreamSynchronize(c->copy_stream));
+	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
+	return ORT_OK;
+}
+
+int ort_read_voxels(ort_ctx* c, int x0, int y0, int z0, int nx, int ny, int nz, uint32_t* out)
+{
+	enter(c);
+	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_read_voxels: null context");
+	const long long dim = 1ll << c->depth;
+	const auto axis_ok = [dim](int o, int e) { return o >= 0 && e >= 1 && static_cast<long long>(o) + e <= dim; };
+	if (!axis_ok(x0, nx) || !axis_ok(y0, ny) || !axis_ok(z0, nz))
+		return ort_fail(c, ORT_ERR_INVALID, "ort_read_voxels: box origin (%d, %d, %d) extent (%d, %d, %d) is not inside the cube of %lld voxels a side",
+		                x0, y0, z0, nx, ny, nz, dim);
+	if (!out) return ort_fail(c, ORT_ERR_INVALID, "ort_read_voxels: null buffer");
+	DeviceGuard g(c->device);
+	const bool out_dev = is_device_ptr(out);
+	if (out_dev && (reinterpret_cast<uintptr_t>(out) & 3u))
+		return ort_fail(c, ORT_ERR_INVALID, "ort_read_voxels: a device output must be 4-byte aligned");
+	const ort::QueryBox box{ static_cast<uint32_t>(x0), static_cast<uint32_t>(y0), static_cast<uint32_t>(z0),
+	                         static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz) };
+	if (out_dev) return launch_read_voxels(c, box, out);                      // enqueue only
+
+	// host output: whole output rows (nx voxels) through the staging slots, at most kQueryStageBytes at a time -- whole
+	// z slices when one fits, else runs of rows of one slice; each chunk is a sub-box whose output is contiguous
+	const size_t row_bytes = static_cast<size_t>(nx) * 4;
+	const size_t chunk_rows = std::max<size_t>(1, kQueryStageBytes / row_bytes);
+	const size_t slice_rows = static_cast<size_t>(ny);
+	const size_t total_rows = slice_rows * static_cast<size_t>(nz);
+	int rc = ensure_dstage(c, 2 * align_up(std::min(chunk_rows, total_rows) * row_bytes, 256));
+	if (rc != ORT_OK) return rc;
+	for (size_t r0 = 0; r0 < total_rows;)
+	{
+		const uint32_t z = static_cast<uint32_t>(r0 / slice_rows), y = static_cast<uint32_t>(r0 % slice_rows);
+		ort::QueryBox sub = box;
+		if (y == 0 && chunk_rows >= slice_rows)
+		{
+			sub.z0 = box.z0 + z;
+			sub.nz = static_cast<uint32_t>(std::min<size_t>(chunk_rows / slice_rows, box.nz - z));
+		}
+		else
+		{
+			sub.y0 = box.y0 + y;
+			sub.ny = static_cast<uint32_t>(std::min<size_t>(chunk_rows, slice_rows - y));
+			sub.z0 = box.z0 + z;
+			sub.nz = 1;
+		}
+		const size_t m = static_cast<size_t>(sub.ny) * sub.nz;
+		char* base = nullptr;
+		const int slot = query_slot(c, &base);
+		uint32_t* d_out = reinterpret_cast<uint32_t*>(base);
+		if ((rc = launch_read_voxels(c, sub, d_out)) != ORT_OK) return rc;
+		if ((rc = query_slot_done(c, slot, out + r0 * nx, d_out, m * row_bytes)) != ORT_OK) return rc;
+		r0 += m;
+	}
+	ORT_CUDA(c, cudaStreamSynchronize(c->copy_stream));
+	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
+	return ORT_OK;
+}
 
 }  // extern "C"
 

@@ -152,6 +152,77 @@ class TraceContext:
         self._ck(self.L.ort_read_nodes(self.h, first, n, _p(out)))
         return out
 
+    def _query_out(self, out, n: int, shape, like_torch, device, what: str):
+        """The output buffer of a voxel query: `out` checked (numpy uint32 / int32 array, or a CPU, pinned or CUDA tensor
+        of that dtype on this context's GPU, C-contiguous, `n` elements), or a new one: a torch.uint32 tensor on `device`
+        when the input was a tensor (like_torch), else a numpy uint32 array.  Returns (buffer, is_cuda)."""
+        if out is None:
+            if like_torch:
+                import torch
+                return torch.empty(shape, dtype=torch.uint32, device=device), device.type == "cuda"
+            return np.empty(shape, np.uint32), False
+        if isinstance(out, np.ndarray):
+            if out.dtype not in (np.uint32, np.int32):
+                raise TypeError(f"{what}: out dtype {out.dtype} (uint32 or int32 required)")
+            if out.size != n or not out.flags.c_contiguous or not out.flags.writeable:
+                raise ValueError(f"{what}: out must be a writeable C-contiguous array of {n} elements")
+            return out, False
+        if hasattr(out, "data_ptr"):
+            import torch
+            if out.dtype not in (torch.uint32, torch.int32):
+                raise TypeError(f"{what}: out dtype {out.dtype} (uint32 or int32 required)")
+            if out.numel() != n or not out.is_contiguous():
+                raise ValueError(f"{what}: out must be a contiguous tensor of {n} elements")
+            if out.is_cuda and out.device.index != self.device:
+                raise ValueError(f"{what}: out is on {out.device}, the context on cuda:{self.device}")
+            return out, out.is_cuda
+        raise TypeError(f"{what}: out must be a numpy array or a torch tensor, got {type(out).__name__}")
+
+    def voxels_at(self, xyz, out=None):
+        """at(x, y, z) for every row of xyz on this context's GPU (ort_voxels_at).  xyz: (n, 3) integers x, y, z -- a numpy
+        array of any integer dtype (converted to int32), or a contiguous int32 torch tensor on the CPU or this GPU.
+        Coordinates wrap as at()'s do (low `depth` bits).  Returns n uint32 values: numpy for numpy input, a torch.uint32
+        tensor on the input's device for a tensor, or `out`."""
+        if isinstance(xyz, np.ndarray) or not hasattr(xyz, "data_ptr"):
+            a = np.asarray(xyz)
+            if a.dtype.kind not in "iu":
+                raise TypeError(f"voxels_at: integer coordinates required, got {a.dtype}")
+            if a.ndim != 2 or a.shape[1] != 3:
+                raise ValueError("voxels_at: an (n, 3) array of x, y, z is required")
+            xyz, in_cuda, device = np.ascontiguousarray(a.astype(np.int32, copy=False)), False, None
+        else:
+            import torch
+            if xyz.dtype != torch.int32:
+                raise TypeError(f"voxels_at: dtype {xyz.dtype} (int32 required)")
+            if xyz.dim() != 2 or xyz.shape[1] != 3 or not xyz.is_contiguous():
+                raise ValueError("voxels_at: a contiguous (n, 3) tensor of x, y, z is required")
+            if xyz.is_cuda and xyz.device.index != self.device:
+                raise ValueError(f"voxels_at: the tensor is on {xyz.device}, the context on cuda:{self.device}")
+            in_cuda, device = xyz.is_cuda, xyz.device
+        n = int(xyz.shape[0])
+        out, out_cuda = self._query_out(out, n, (n,), device is not None, device, "voxels_at")
+        self._run_query(in_cuda, out_cuda, lambda: self.L.ort_voxels_at(self.h, _p(xyz), n, _p(out)))
+        return out
+
+    def read_voxels(self, origin, extent, out=None):
+        """The box [x0, x0+nx) x [y0, y0+ny) x [z0, z0+nz) of the DAG on this context's GPU (ort_read_voxels) as an
+        (nz, ny, nx) uint32 grid indexed [z, y, x] -- numpy by default, or `out`: a numpy array or a CPU, pinned or CUDA
+        tensor of uint32 or int32.  The box must lie inside the cube.  The result can go straight back to upload_voxels."""
+        x0, y0, z0 = (int(v) for v in origin)
+        nx, ny, nz = (int(v) for v in extent)
+        shape = (max(nz, 0), max(ny, 0), max(nx, 0))           # (a bad box is refused by the library)
+        out, out_cuda = self._query_out(out, shape[0] * shape[1] * shape[2], shape, False, None, "read_voxels")
+        self._run_query(False, out_cuda, lambda: self.L.ort_read_voxels(self.h, x0, y0, z0, nx, ny, nz, _p(out)))
+        return out
+
+    def _run_query(self, in_cuda: bool, out_cuda: bool, call):
+        if in_cuda or out_cuda:
+            import torch
+            torch.cuda.current_stream(self.device).synchronize()      # the query runs on the context's stream
+        self._ck(call())
+        if out_cuda:
+            self.sync()                                                # a device-only call was only enqueued
+
     def set_option(self, key: str, value: int):
         self._ck(self.L.ort_set_option(self.h, key.encode(), value))
 
@@ -467,6 +538,16 @@ class HOctree:
         rot, fov = camera_coeffs(yaw, pitch)
         return self.ctx.trace_frame(pos, rot, fov, W, H, **kw)
 
+    def voxels_at(self, xyz, out=None):
+        """at() for every row of xyz, read from the GPU mirror after a sync (TraceContext.voxels_at)."""
+        self.sync()
+        return self.ctx.voxels_at(xyz, out)
+
+    def read_voxels(self, origin, extent, out=None):
+        """A box of voxels as an (nz, ny, nx) grid, read from the GPU mirror after a sync (TraceContext.read_voxels)."""
+        self.sync()
+        return self.ctx.read_voxels(origin, extent, out)
+
 
 class Octree:
     """och::octree(depth, table_capacity) (och_octree.h:10-69): plain pointer octree over a node pool, GPU tracer.
@@ -544,3 +625,13 @@ class Octree:
         self.sync()
         rot, fov = camera_coeffs(yaw, pitch)
         return self.ctx.trace_frame(pos, rot, fov, W, H, **kw)
+
+    def voxels_at(self, xyz, out=None):
+        """at() for every row of xyz, read from the GPU mirror after a sync (TraceContext.voxels_at)."""
+        self.sync()
+        return self.ctx.voxels_at(xyz, out)
+
+    def read_voxels(self, origin, extent, out=None):
+        """A box of voxels as an (nz, ny, nx) grid, read from the GPU mirror after a sync (TraceContext.read_voxels)."""
+        self.sync()
+        return self.ctx.read_voxels(origin, extent, out)

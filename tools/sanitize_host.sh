@@ -29,7 +29,7 @@ export LD_PRELOAD="$(gcc -print-file-name=libasan.so) $(gcc -print-file-name=lib
 export ASAN_OPTIONS=detect_leaks=0:halt_on_error=1 UBSAN_OPTIONS=print_stacktrace=1:halt_on_error=0
 export ORT_EMU_SANITIZE=1      # the host emulation of the device walkers too: their parent stacks are plain local arrays
 python -m pytest tests/test_host_tree.py tests/test_octree.py tests/test_shading.py tests/test_capi_symbols.py \
-       tests/test_fuzz_random_dags.py tests/test_multi_gpu_cpu.py tests/test_host_emu.py tests/test_beam.py -q -s -m "not gpu" 2>&1 | tee sanitize.log | tail -3
+       tests/test_fuzz_random_dags.py tests/test_multi_gpu_cpu.py tests/test_host_emu.py tests/test_beam.py tests/test_voxel_query.py -q -s -m "not gpu" 2>&1 | tee sanitize.log | tail -3
 if grep -q "runtime error\|AddressSanitizer" sanitize.log; then
 	grep "runtime error\|AddressSanitizer" sanitize.log | sort | uniq -c | sort -rn | head -20
 	exit 1
