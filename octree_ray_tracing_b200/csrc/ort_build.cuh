@@ -270,6 +270,7 @@ __global__ void scan_add_kernel(uint32_t* a, size_t n, const uint32_t* offs)
 	if (i < n) a[i] += offs[i / kScanTile];
 }
 
+#ifndef ORT_HOST_EMU          // (the host emulation, tests/host_emu/emu_build.cpp, compiles the device code above only)
 // scratch words scan_exclusive needs for n items
 inline size_t scan_scratch_words(size_t n)
 {
@@ -290,5 +291,6 @@ inline void scan_exclusive(uint32_t* a, size_t n, uint32_t* scratch, cudaStream_
 	scan_add_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(a, n, scratch);
 	++launches;
 }
+#endif
 
 }  // namespace ort
