@@ -104,10 +104,25 @@ int ort_upload_pool(ort_ctx* ctx, const uint32_t* nodes8, size_t n_nodes);
  * elements must be 4-byte aligned. */
 int ort_build_voxels(ort_ctx* ctx, const void* voxels, int elem_bytes, int nx, int ny, int nz,
                      size_t* n_nodes, uint32_t* level_offsets);
+/* Write the box [x0, x0+nx) x [y0, y0+ny) x [z0, z0+nz) of voxels into the DAG on ctx's GPU and install the result as
+ * the mirror.  voxels: nx*ny*nz elements of elem_bytes (1 or 4), voxel (x, y, z) of the box at index
+ * ((z-z0)*ny + (y-y0))*nx + (x-x0) -- the layout ort_read_voxels writes and ort_build_voxels reads; 0 erases.  Every
+ * voxel outside the box keeps the value ort_voxels_at returned before the call.  The mirror afterwards holds exactly
+ * what ort_tree_flatten returns for a table holding the resulting voxels (root id 1, or 0 and n = 0 when the scene became
+ * empty; level_offsets, optional, depth+1 entries, as ort_build_voxels'), whatever form the previous mirror had: built,
+ * fully uploaded, after deltas with unreachable rows, or never uploaded to.  The box does not wrap: 0 <= x0, 1 <= nx <=
+ * 2048 and x0 + nx <= 2^depth on each axis; context depth 1..16.  Host (pageable or pinned) or device source; a device
+ * source must be complete and, for 4-byte elements, 4-byte aligned.  ORT_ERR_INVALID for bad arguments, a box outside
+ * the cube, a source on another device, a misaligned device source or a context in the och::octree pool layout;
+ * ORT_ERR_CAPACITY for a result beyond the 2^29 - 1 compact ids; ORT_ERR_CUDA when device memory runs out.  After any
+ * failure the previous mirror is still installed.  Returns once the new mirror is installed (as ort_build_voxels).  A
+ * host table attached to ctx no longer describes the mirror afterwards. */
+int ort_write_voxels(ort_ctx* ctx, int x0, int y0, int z0, const void* voxels, int elem_bytes,
+                     int nx, int ny, int nz, size_t* n_nodes, uint32_t* level_offsets);
 /* Copy n rows of the device mirror, starting at compact id first (1-based), to nodes8 (host or device). */
 int ort_read_nodes(ort_ctx* ctx, uint32_t first, size_t n, uint32_t* nodes8);
-/* Device bytes the last successful ort_build_voxels allocated: its temporaries plus a new mirror if it had to grow one
- * (nothing is freed before the build ends, so this is its peak on top of what the context held). */
+/* Device bytes the last successful ort_build_voxels or ort_write_voxels allocated: its temporaries plus a new mirror if it
+ * had to grow one (nothing is freed before the call ends, so this is its peak on top of what the context held). */
 uint64_t ort_build_bytes(const ort_ctx* ctx);
 
 /* Replaces: n calls of at(x, y, z) (och_h_octree.h:239-258; och::octree::at, och_octree.cpp:141-160) on the DAG

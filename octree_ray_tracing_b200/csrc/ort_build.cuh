@@ -93,61 +93,93 @@ __device__ __forceinline__ unsigned block_sum(unsigned v)
 	return s;           // valid in thread 0
 }
 
-// Leaf level: count the non-empty cells (sizes the level's table).
-__global__ void build_count_leaf_kernel(BuildInput in, BuildLevel L, unsigned long long* count)
+// ---- content sources ------------------------------------------------------------------------------------------------
+// The kernels below are shared with the box write (ort_write.cuh) through a content source `Src`:
+//   items()            the items one bottom-up pass inserts (a level's cells here)
+//   entry(i)           the table entry that stands for item i (its representative value, != kBuildEmpty)
+//   content(e, w)      the 8 words of entry e, recomputed from immutable inputs
+//   store(i, id)       record item i's temporary id (0 = empty content)
+//   rep(t)             the entry of temporary id t (top-down)
+//   child(e, c)        word c of entry e's content (top-down, levels above the leaf level)
+
+// The builder's source: level L of the dense grid, its child grid C (levels above the leaf level).
+struct DenseSrc
 {
-	const size_t n = static_cast<size_t>(L.gx) * L.gy * L.gz;
-	const size_t cell = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-	unsigned ne = 0;
-	if (cell < n)
+	bool leaf;
+	BuildInput in;
+	BuildLevel L, C;
+	__device__ __forceinline__ size_t items() const { return static_cast<size_t>(L.gx) * L.gy * L.gz; }
+	__device__ __forceinline__ uint32_t entry(size_t i) const { return static_cast<uint32_t>(i); }
+	__device__ __forceinline__ void content(uint32_t e, uint32_t w[8]) const
 	{
-		uint32_t x, y, z, w[8];
-		build_decode(static_cast<uint32_t>(cell), L, x, y, z);
-		build_content(true, in, L, x, y, z, w);
+		uint32_t x, y, z;
+		build_decode(e, L, x, y, z);
+		build_content(leaf, in, C, x, y, z, w);
+	}
+	__device__ __forceinline__ void store(size_t i, uint32_t id) const { L.ids[i] = id; }
+	__device__ __forceinline__ uint32_t rep(uint32_t t) const { return L.table[t - 1]; }
+	__device__ __forceinline__ uint32_t child(uint32_t e, int c) const
+	{
+		uint32_t x, y, z;
+		build_decode(e, L, x, y, z);
+		const uint32_t cx = 2 * x + (c & 1), cy = 2 * y + ((c >> 1) & 1), cz = 2 * z + (c >> 2);
+		return (cx < C.gx && cy < C.gy && cz < C.gz) ? C.ids[(static_cast<size_t>(cz) * C.gy + cy) * C.gx + cx] : 0u;
+	}
+};
+
+// Count the items with non-empty content (sizes a level's table).
+template<class Src>
+__global__ void build_count_kernel(Src src, unsigned long long* count)
+{
+	const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+	unsigned ne = 0;
+	if (i < src.items())
+	{
+		uint32_t w[8];
+		src.content(src.entry(i), w);
 		ne = (w[0] | w[1] | w[2] | w[3] | w[4] | w[5] | w[6] | w[7]) != 0u;
 	}
 	const unsigned s = block_sum(ne);
 	if (threadIdx.x == 0 && s) atomicAdd(count, static_cast<unsigned long long>(s));
 }
 
-// Bottom-up pass of one level: insert every non-empty cell, write its temporary id (table slot + 1, 0 = empty).
-// C = the child grid (levels above the leaf level).
-__global__ void build_insert_kernel(bool leaf, BuildInput in, BuildLevel L, BuildLevel C, unsigned long long* nonempty)
+// Bottom-up pass of one level: insert every item with non-empty content into the table (cap = mask + 1 entries), store
+// its temporary id (table slot + 1, 0 = empty); count the non-empty items.
+template<class Src>
+__global__ void build_insert_kernel(Src src, uint32_t* table, uint32_t mask, unsigned long long* nonempty)
 {
-	const size_t n = static_cast<size_t>(L.gx) * L.gy * L.gz;
-	const size_t cell = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+	const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
 	unsigned ne = 0;
-	if (cell < n)
+	if (i < src.items())
 	{
-		uint32_t x, y, z, w[8];
-		build_decode(static_cast<uint32_t>(cell), L, x, y, z);
-		build_content(leaf, in, C, x, y, z, w);
+		uint32_t w[8];
+		const uint32_t me = src.entry(i);
+		src.content(me, w);
 		uint32_t id = 0;
 		if (w[0] | w[1] | w[2] | w[3] | w[4] | w[5] | w[6] | w[7])
 		{
 			ne = 1;
-			uint32_t slot = build_hash(w) & L.mask;
+			uint32_t slot = build_hash(w) & mask;
 			for (;;)
 			{
-				uint32_t e = L.table[slot];
+				uint32_t e = table[slot];
 				if (e == kBuildEmpty)
 				{
-					e = atomicCAS(L.table + slot, kBuildEmpty, static_cast<uint32_t>(cell));
-					if (e == kBuildEmpty) break;                      // claimed: this cell represents its content
+					e = atomicCAS(table + slot, kBuildEmpty, me);
+					if (e == kBuildEmpty) break;                      // claimed: this item represents its content
 				}
 				// taken: the same content?  (the full 32 bytes; equal hashes prove nothing)
-				uint32_t ex, ey, ez, v[8];
-				build_decode(e, L, ex, ey, ez);
-				build_content(leaf, in, C, ex, ey, ez, v);
+				uint32_t v[8];
+				src.content(e, v);
 				bool same = true;
 #pragma unroll
 				for (int c = 0; c < 8; ++c) same &= v[c] == w[c];
 				if (same) break;
-				slot = (slot + 1) & L.mask;
+				slot = (slot + 1) & mask;
 			}
 			id = slot + 1;
 		}
-		L.ids[cell] = id;
+		src.store(i, id);
 	}
 	const unsigned s = block_sum(ne);
 	if (threadIdx.x == 0 && s) atomicAdd(nonempty, static_cast<unsigned long long>(s));
@@ -163,16 +195,12 @@ __global__ void build_count_table_kernel(const uint32_t* table, size_t cap, unsi
 
 // Top-down, step 1: the temporary id of child slot s = 8 i + c of frontier node i (ch[s]); first occurrence of each
 // distinct child (first[t - 1], indexed by the child level's table slot).
-__global__ void build_children_kernel(const uint32_t* frontier, size_t n_slots, BuildLevel L, BuildLevel C, uint32_t* ch, uint32_t* first)
+template<class Src>
+__global__ void build_children_kernel(const uint32_t* frontier, size_t n_slots, Src src, uint32_t* ch, uint32_t* first)
 {
 	const size_t s = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
 	if (s >= n_slots) return;
-	const uint32_t rep = L.table[frontier[s >> 3] - 1];
-	uint32_t x, y, z;
-	build_decode(rep, L, x, y, z);
-	const int c = static_cast<int>(s & 7);
-	const uint32_t cx = 2 * x + (c & 1), cy = 2 * y + ((c >> 1) & 1), cz = 2 * z + (c >> 2);
-	const uint32_t t = (cx < C.gx && cy < C.gy && cz < C.gz) ? C.ids[(static_cast<size_t>(cz) * C.gy + cy) * C.gx + cx] : 0u;
+	const uint32_t t = src.child(src.rep(frontier[s >> 3]), static_cast<int>(s & 7));
 	ch[s] = t;
 	if (t) atomicMin(first + (t - 1), static_cast<uint32_t>(s));
 }
@@ -187,7 +215,8 @@ __global__ void build_flags_kernel(const uint32_t* ch, const uint32_t* first, si
 }
 
 // step 3 (after the exclusive scan of the flags, pos): the level's rows with final child ids, the next frontier.
-// rows = the level's first row in the output; next_base = final id of the next level's first node.
+// rows = the level's first row in the output; next_base = final id of the next level's first node.  (rows may be ch
+// itself: slot s reads ch[s] before it writes rows[s], and no other slot reads it.)
 __global__ void build_rows_kernel(const uint32_t* ch, const uint32_t* first, const uint32_t* pos, size_t n_slots, uint32_t next_base,
                                   uint32_t* rows, uint32_t* next_frontier)
 {
@@ -205,14 +234,14 @@ __global__ void build_rows_kernel(const uint32_t* ch, const uint32_t* first, con
 	rows[s] = id;
 }
 
-// The leaf level's rows: the voxels of each frontier node's representative cell.
-__global__ void build_leaf_rows_kernel(const uint32_t* frontier, size_t n, BuildInput in, BuildLevel L, uint32_t* rows)
+// The leaf level's rows: the content of each frontier node's representative.
+template<class Src>
+__global__ void build_leaf_rows_kernel(const uint32_t* frontier, size_t n, Src src, uint32_t* rows)
 {
 	const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
 	if (i >= n) return;
-	uint32_t x, y, z, w[8];
-	build_decode(L.table[frontier[i] - 1], L, x, y, z);
-	build_content(true, in, L, x, y, z, w);
+	uint32_t w[8];
+	src.content(src.rep(frontier[i]), w);
 	uint4* o = reinterpret_cast<uint4*>(rows + 8 * i);
 	o[0] = make_uint4(w[0], w[1], w[2], w[3]);
 	o[1] = make_uint4(w[4], w[5], w[6], w[7]);

@@ -113,7 +113,7 @@ struct ort_ctx
 	uint64_t beam_seen_seq = 0;
 	bool frame_call_nested = false;
 	uint64_t beam_builds = 0;
-	uint64_t build_bytes = 0;           // device bytes the last successful ort_build_voxels allocated (its peak)
+	uint64_t build_bytes = 0;           // device bytes the last successful ort_build_voxels or ort_write_voxels allocated (its peak)
 
 	unsigned long long* d_counters = nullptr; // work counters of the persistent kernels: a ring, one per launch (kCounterRing)
 	unsigned next_counter = 0;
@@ -252,6 +252,7 @@ inline void beam_invalidate(ort_ctx* c)
 
 #include "ort_kernels.cuh"
 #include "ort_build.cuh"
+#include "ort_write.cuh"
 #include "ort_query.cuh"
 
 static_assert(ort::kBeamFineLevel == 8, "ort_ctx holds the beam grids of levels 0 .. 8");
@@ -883,6 +884,77 @@ inline size_t pow2_at_least(size_t v)
 	return p;
 }
 
+// A new mirror allocated by a build or write, freed unless it was installed.
+struct NewMirror
+{
+	uint32_t* p = nullptr;
+	~NewMirror() { cudaFree(p); }
+};
+
+// Install `total` compact rows (level l from id base[l]) as the mirror, as ort_upload_full does: every launch in flight
+// reads the array that is replaced, so the device is synchronised first.  The rows are the n_parts device buffers
+// `parts` (part_rows[i] rows each) in order; they go to fresh.p when out_cap != 0 (a new mirror of out_cap rows; a part
+// that already lies there is not copied), else over the current array.  temp_bytes: the call's other allocations.
+int install_mirror(ort_ctx* c, NewMirror& fresh, size_t out_cap, const uint32_t* const* parts, const size_t* part_rows, int n_parts,
+                   size_t total, const size_t* base, uint64_t temp_bytes, size_t* n_out, uint32_t* level_offsets)
+{
+	const int D = c->depth;
+	ORT_CUDA(c, cudaDeviceSynchronize());
+	uint32_t* dst = out_cap ? fresh.p : c->d_nodes;
+	size_t at = 0;
+	for (int i = 0; i < n_parts; ++i)
+	{
+		if (part_rows[i] && parts[i] != dst + 8 * at)
+			ORT_CUDA(c, cudaMemcpyAsync(dst + 8 * at, parts[i], part_rows[i] * 32, cudaMemcpyDeviceToDevice, c->stream));
+		at += part_rows[i];
+	}
+	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
+	if (out_cap)
+	{
+		cudaFree(c->d_nodes);
+		c->d_nodes = fresh.p;
+		c->cap_nodes = static_cast<uint32_t>(out_cap);
+		fresh.p = nullptr;                                         // (owned by the context now)
+	}
+	c->n_nodes = static_cast<uint32_t>(total);
+	c->root = total ? 1u : 0u;
+	c->index_base = 1;
+	c->has_root = total != 0;
+	c->miss_t = __builtin_inff();
+	beam_invalidate(c);
+	c->build_bytes = temp_bytes + out_cap * 32;
+	if (n_out) *n_out = total;
+	if (level_offsets)
+	{
+		for (int l = 1; l <= D; ++l) level_offsets[l - 1] = static_cast<uint32_t>(base[l]);
+		level_offsets[D] = static_cast<uint32_t>(total + 1);
+	}
+	return ORT_OK;
+}
+
+// The `count` voxels of a builder or write source on this context's device: `voxels` itself when it is device memory
+// there (checked: this device, aligned to its element size), else a copy in `tmp` enqueued on the context's stream.
+int device_voxels(ort_ctx* c, const char* what, const void* voxels, int elem_bytes, size_t count, BuildTemps& tmp, const void** src)
+{
+	cudaPointerAttributes a;
+	const bool dev = cudaPointerGetAttributes(&a, voxels) == cudaSuccess && (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged);
+	cudaGetLastError();
+	if (dev && a.type == cudaMemoryTypeDevice && a.device != c->device)
+		return ort_fail(c, ORT_ERR_INVALID, "%s: the voxels live on device %d, the context on device %d", what, a.device, c->device);
+	if (dev && (reinterpret_cast<uintptr_t>(voxels) & static_cast<uintptr_t>(elem_bytes - 1)))
+		return ort_fail(c, ORT_ERR_INVALID, "%s: a device source of %d-byte elements must be %d-byte aligned", what, elem_bytes, elem_bytes);
+	*src = voxels;
+	if (!dev)
+	{
+		const size_t bytes = count * elem_bytes;
+		void* d = nullptr;
+		ORT_CUDA(c, tmp.alloc(reinterpret_cast<uint8_t**>(&d), bytes));
+		ORT_CUDA(c, cudaMemcpyAsync(d, voxels, bytes, cudaMemcpyDefault, c->stream));
+		*src = d;
+	}
+	return ORT_OK;
+}
+
 int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, uint32_t ny, uint32_t nz, size_t* n_out, uint32_t* level_offsets)
 {
 	const int D = c->depth;
@@ -890,24 +962,9 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 	BuildTemps tmp;
 
 	// the input, on this device
-	const void* src = voxels;
-	{
-		cudaPointerAttributes a;
-		const bool dev = cudaPointerGetAttributes(&a, voxels) == cudaSuccess && (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged);
-		cudaGetLastError();
-		if (dev && a.type == cudaMemoryTypeDevice && a.device != c->device)
-			return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: the voxels live on device %d, the context on device %d", a.device, c->device);
-		if (dev && (reinterpret_cast<uintptr_t>(voxels) & static_cast<uintptr_t>(elem_bytes - 1)))
-			return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: a device source of %d-byte elements must be %d-byte aligned", elem_bytes, elem_bytes);
-		if (!dev)
-		{
-			const size_t bytes = static_cast<size_t>(nx) * ny * nz * elem_bytes;
-			void* d = nullptr;
-			ORT_CUDA(c, tmp.alloc(reinterpret_cast<uint8_t**>(&d), bytes));
-			ORT_CUDA(c, cudaMemcpyAsync(d, voxels, bytes, cudaMemcpyDefault, st));
-			src = d;
-		}
-	}
+	const void* src = nullptr;
+	const int rc = device_voxels(c, "ort_build_voxels", voxels, elem_bytes, static_cast<size_t>(nx) * ny * nz, tmp, &src);
+	if (rc != ORT_OK) return rc;
 	const ort::BuildInput in{ src, elem_bytes, nx, ny, nz };
 
 	// level grids, clipped to the input's extent: level l has cells of side 2^(D-l+1) voxels
@@ -928,7 +985,7 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 	unsigned long long h_cnt[2 * (ort::kBuildMaxDepth + 1)] = {};
 
 	// bottom-up: a level's distinct contents are at most its non-empty cells, which are at most the level below's
-	ort::build_count_leaf_kernel<<<blocks_for(static_cast<size_t>(lv[D].gx) * lv[D].gy * lv[D].gz), 256, 0, st>>>(in, lv[D], d_cnt);
+	ort::build_count_kernel<<<blocks_for(static_cast<size_t>(lv[D].gx) * lv[D].gy * lv[D].gz), 256, 0, st>>>(ort::DenseSrc{ true, in, lv[D], lv[D] }, d_cnt);
 	++c->launches;
 	ORT_CUDA(c, cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
 	ORT_CUDA(c, cudaStreamSynchronize(st));
@@ -940,7 +997,7 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 		ORT_CUDA(c, tmp.alloc(&lv[l].table, cap[l]));
 		lv[l].mask = static_cast<uint32_t>(cap[l] - 1);
 		ORT_CUDA(c, cudaMemsetAsync(lv[l].table, 0xFF, cap[l] * 4, st));
-		ort::build_insert_kernel<<<blocks_for(cells), 256, 0, st>>>(l == D, in, lv[l], l == D ? lv[l] : lv[l + 1], d_cnt + l);
+		ort::build_insert_kernel<<<blocks_for(cells), 256, 0, st>>>(ort::DenseSrc{ l == D, in, lv[l], l == D ? lv[l] : lv[l + 1] }, lv[l].table, lv[l].mask, d_cnt + l);
 		ort::build_count_table_kernel<<<blocks_for(cap[l]), 256, 0, st>>>(lv[l].table, cap[l], d_cnt + D + 1 + l);
 		c->launches += 2;
 		ORT_CUDA(c, cudaGetLastError());
@@ -966,7 +1023,7 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 	// the output rows: straight into a new mirror when the current one is too small, else a temporary copied over
 	uint32_t* out = nullptr;
 	size_t out_cap = 0;
-	struct NewMirror { uint32_t* p = nullptr; ~NewMirror() { cudaFree(p); } } fresh;
+	NewMirror fresh;
 	if (total > c->cap_nodes)
 	{
 		out_cap = std::min<size_t>(total + total / 4 + 4096, ort::kIdMask);      // head-room for the deltas that follow, as ort_upload_full
@@ -996,7 +1053,7 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 		{
 			const size_t slots = 8 * n_lvl[l];
 			ORT_CUDA(c, cudaMemsetAsync(first, 0xFF, cap[l + 1] * 4, st));
-			ort::build_children_kernel<<<blocks_for(slots), 256, 0, st>>>(frontier[l], slots, lv[l], lv[l + 1], ch, first);
+			ort::build_children_kernel<<<blocks_for(slots), 256, 0, st>>>(frontier[l], slots, ort::DenseSrc{ false, in, lv[l], lv[l + 1] }, ch, first);
 			ort::build_flags_kernel<<<blocks_for(slots), 256, 0, st>>>(ch, first, slots, pos);
 			c->launches += 2;
 			ort::scan_exclusive(pos, slots, scratch, st, c->launches);
@@ -1005,40 +1062,220 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 			++c->launches;
 			ORT_CUDA(c, cudaGetLastError());
 		}
-		ort::build_leaf_rows_kernel<<<blocks_for(n_lvl[D]), 256, 0, st>>>(frontier[D], n_lvl[D], in, lv[D], out + 8 * (base[D] - 1));
+		ort::build_leaf_rows_kernel<<<blocks_for(n_lvl[D]), 256, 0, st>>>(frontier[D], n_lvl[D], ort::DenseSrc{ true, in, lv[D], lv[D] }, out + 8 * (base[D] - 1));
 		++c->launches;
 		ORT_CUDA(c, cudaGetLastError());
 	}
 	ORT_CUDA(c, cudaStreamSynchronize(st));
+	const uint32_t* part = out;
+	return install_mirror(c, fresh, out_cap, &part, &total, 1, total, base, tmp.bytes, n_out, level_offsets);
+}
 
-	// install, as ort_upload_full does: every launch in flight reads the array that is replaced
-	ORT_CUDA(c, cudaDeviceSynchronize());
-	if (out_cap)
+// ------------------------------------------------------------------------------------------------
+// a dense box of voxels written into the device DAG (ort_write.cuh, DESIGN section 15)
+// ------------------------------------------------------------------------------------------------
+
+constexpr int kWriteMaxExtent = 2048;         // voxels per axis of one write: the builder's depth-11 envelope
+constexpr int kWriteMaxDepth = 16;
+
+// Scratch of the top-down passes (child slots, their scan, the scan's total), grown on demand.
+struct TopDown
+{
+	uint32_t *ch = nullptr, *pos = nullptr, *scan = nullptr, *last = nullptr;
+	size_t cap = 0;
+};
+
+// One top-down step over the 8 n child slots of `frontier` (src.rep / src.child, ort_build.cuh): the first occurrence of
+// each distinct child (first: first_words words, indexed by child t - 1), the next frontier in order of first occurrence
+// (allocated in tmp, n_next entries) and, where rows is not null, the slots' final child ids next_base + rank.
+template<class Src>
+int top_down_step(ort_ctx* c, BuildTemps& tmp, TopDown& td, const Src& src, const uint32_t* frontier, size_t n, uint32_t* first, size_t first_words,
+                  uint32_t next_base, uint32_t* rows, uint32_t** next, size_t* n_next)
+{
+	cudaStream_t st = c->stream;
+	const size_t slots = 8 * n;
+	*n_next = 0;
+	if (!n) return ORT_OK;
+	if (!td.last) ORT_CUDA(c, tmp.alloc(&td.last, 2));
+	if (slots > td.cap)
 	{
-		cudaFree(c->d_nodes);
-		c->d_nodes = out;
-		c->cap_nodes = static_cast<uint32_t>(out_cap);
-		fresh.p = nullptr;                                         // (owned by the context now)
+		ORT_CUDA(c, tmp.alloc(&td.ch, slots));
+		ORT_CUDA(c, tmp.alloc(&td.pos, slots));
+		ORT_CUDA(c, tmp.alloc(&td.scan, ort::scan_scratch_words(slots)));
+		td.cap = slots;
 	}
-	else if (total)
-	{
-		ORT_CUDA(c, cudaMemcpyAsync(c->d_nodes, out, total * 32, cudaMemcpyDeviceToDevice, st));
-		ORT_CUDA(c, cudaStreamSynchronize(st));
-	}
-	c->n_nodes = static_cast<uint32_t>(total);
-	c->root = total ? 1u : 0u;
-	c->index_base = 1;
-	c->has_root = total != 0;
-	c->miss_t = __builtin_inff();
-	beam_invalidate(c);
-	c->build_bytes = tmp.bytes + out_cap * 32;
-	if (n_out) *n_out = total;
-	if (level_offsets)
-	{
-		for (int l = 1; l <= D; ++l) level_offsets[l - 1] = static_cast<uint32_t>(base[l]);
-		level_offsets[D] = static_cast<uint32_t>(total + 1);
-	}
+	ORT_CUDA(c, cudaMemsetAsync(first, 0xFF, first_words * 4, st));
+	ort::build_children_kernel<<<blocks_for(slots), 256, 0, st>>>(frontier, slots, src, td.ch, first);
+	ort::build_flags_kernel<<<blocks_for(slots), 256, 0, st>>>(td.ch, first, slots, td.pos);
+	c->launches += 2;
+	ORT_CUDA(c, cudaMemcpyAsync(td.last, td.pos + slots - 1, 4, cudaMemcpyDeviceToDevice, st));      // the last flag ...
+	ort::scan_exclusive(td.pos, slots, td.scan, st, c->launches);
+	ORT_CUDA(c, cudaMemcpyAsync(td.last + 1, td.pos + slots - 1, 4, cudaMemcpyDeviceToDevice, st));  // ... plus its rank: the count
+	uint32_t h[2] = {};
+	ORT_CUDA(c, cudaMemcpyAsync(h, td.last, 8, cudaMemcpyDeviceToHost, st));
+	ORT_CUDA(c, cudaStreamSynchronize(st));
+	*n_next = static_cast<size_t>(h[0]) + h[1];
+	ORT_CUDA(c, tmp.alloc(next, *n_next));
+	ort::build_rows_kernel<<<blocks_for(slots), 256, 0, st>>>(td.ch, first, td.pos, slots, next_base, rows ? rows : td.ch, *next);
+	++c->launches;
+	ORT_CUDA(c, cudaGetLastError());
 	return ORT_OK;
+}
+
+int write_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* voxels, int elem_bytes, uint32_t nx, uint32_t ny, uint32_t nz,
+                 size_t* n_out, uint32_t* level_offsets)
+{
+	const int D = c->depth;
+	cudaStream_t st = c->stream;
+	BuildTemps tmp;
+	TopDown td;
+
+	const void* src = nullptr;
+	int rc = device_voxels(c, "ort_write_voxels", voxels, elem_bytes, static_cast<size_t>(nx) * ny * nz, tmp, &src);
+	if (rc != ORT_OK) return rc;
+	const ort::BuildInput in{ src, elem_bytes, nx, ny, nz };
+	const ort::WriteDag g{ c->d_nodes - 8, c->has_root ? c->n_nodes + 1 : 0u };
+	const uint32_t old_root = c->has_root && c->root - 1u < g.lim - 1u ? c->root : 0u;
+	const size_t n_ids = c->has_root ? c->n_nodes : 0;         // old ids 1 .. n_ids
+
+	// R_l (the touched cells: origin ro, extent re) and G_l (the children of R_{l-1}; G_1 = R_1 = the root cell)
+	ort::WriteGrid G[kWriteMaxDepth + 2] = {};
+	uint32_t ro[kWriteMaxDepth + 2][3] = {}, re[kWriteMaxDepth + 2][3] = {};
+	const uint32_t b0[3] = { x0, y0, z0 }, b1[3] = { x0 + nx - 1, y0 + ny - 1, z0 + nz - 1 };
+	for (int l = 1; l <= D; ++l)
+	{
+		for (int a = 0; a < 3; ++a)
+		{
+			ro[l][a] = b0[a] >> (D - l + 1);
+			re[l][a] = (b1[a] >> (D - l + 1)) - ro[l][a] + 1;
+		}
+		ort::WriteGrid& w = G[l];
+		w.ox = l == 1 ? 0u : 2 * ro[l - 1][0]; w.gx = l == 1 ? 1u : 2 * re[l - 1][0];
+		w.oy = l == 1 ? 0u : 2 * ro[l - 1][1]; w.gy = l == 1 ? 1u : 2 * re[l - 1][1];
+		w.oz = l == 1 ? 0u : 2 * ro[l - 1][2]; w.gz = l == 1 ? 1u : 2 * re[l - 1][2];
+		const size_t cells = static_cast<size_t>(w.gx) * w.gy * w.gz;
+		ORT_CUDA(c, tmp.alloc(&w.ids, cells));
+		ORT_CUDA(c, tmp.alloc(&w.old_at, cells));
+	}
+
+	// old DAG, top-down: the distinct old ids reachable at each level; the old node at every cell of each G_l
+	uint32_t* old[kWriteMaxDepth + 2] = {};
+	size_t n_old[kWriteMaxDepth + 2] = {};
+	if (old_root)
+	{
+		ORT_CUDA(c, tmp.alloc(&old[1], 1));
+		ORT_CUDA(c, cudaMemcpyAsync(old[1], &old_root, 4, cudaMemcpyHostToDevice, st));
+		n_old[1] = 1;
+		uint32_t* first = nullptr;
+		ORT_CUDA(c, tmp.alloc(&first, n_ids));
+		for (int l = 1; l < D && n_old[l]; ++l)
+			if ((rc = top_down_step(c, tmp, td, ort::OldSrc{ g }, old[l], n_old[l], first, n_ids, 0u, nullptr, &old[l + 1], &n_old[l + 1])) != ORT_OK)
+				return rc;
+	}
+	ORT_CUDA(c, cudaMemcpyAsync(G[1].old_at, &old_root, 4, cudaMemcpyHostToDevice, st));
+	for (int l = 2; l <= D; ++l)
+	{
+		ort::write_old_at_kernel<<<blocks_for(static_cast<size_t>(G[l].gx) * G[l].gy * G[l].gz), 256, 0, st>>>(G[l - 1], G[l], g);
+		++c->launches;
+	}
+	ORT_CUDA(c, cudaGetLastError());
+
+	// bottom-up: T_l holds the reachable old nodes of level l and the touched cells of R_l
+	uint32_t* canon = nullptr;
+	ORT_CUDA(c, tmp.alloc(&canon, n_ids + 1));
+	unsigned long long* d_cnt = nullptr;                        // [l] non-empty items of level l, [0] discarded
+	ORT_CUDA(c, tmp.alloc(&d_cnt, D + 1));
+	ORT_CUDA(c, cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long) * (D + 1), st));
+	ort::WriteSrc S[kWriteMaxDepth + 2] = {};
+	size_t cap[kWriteMaxDepth + 2] = {};
+	for (int l = D; l >= 1; --l)
+	{
+		uint32_t* mapped = nullptr;
+		ORT_CUDA(c, tmp.alloc(&mapped, 8 * n_old[l]));
+		if (n_old[l])
+		{
+			ort::write_map_kernel<<<blocks_for(8 * n_old[l]), 256, 0, st>>>(old[l], n_old[l], g, canon, l == D, mapped);
+			++c->launches;
+		}
+		ort::WriteSrc& s = S[l];
+		s.leaf = l == D;
+		s.in = in;
+		s.bx = x0; s.by = y0; s.bz = z0;
+		s.G = G[l];
+		s.C = l == D ? G[l] : G[l + 1];
+		s.rx = ro[l][0] - G[l].ox; s.ry = ro[l][1] - G[l].oy; s.rz = ro[l][2] - G[l].oz;
+		s.rgx = re[l][0]; s.rgy = re[l][1]; s.rgz = re[l][2];
+		s.g = g;
+		s.old = old[l];
+		s.n_old = static_cast<uint32_t>(n_old[l]);
+		s.mapped = mapped;
+		s.canon = canon;
+		const size_t items = n_old[l] + static_cast<size_t>(s.rgx) * s.rgy * s.rgz;
+		ort::build_count_kernel<<<blocks_for(items), 256, 0, st>>>(s, d_cnt + l);
+		++c->launches;
+		ORT_CUDA(c, cudaGetLastError());
+		unsigned long long h_cnt = 0;
+		ORT_CUDA(c, cudaMemcpyAsync(&h_cnt, d_cnt + l, sizeof h_cnt, cudaMemcpyDeviceToHost, st));
+		ORT_CUDA(c, cudaStreamSynchronize(st));
+		// load factor <= 1/2; past 2^31 entries (a 2048^3 box over a large mirror) up to 3/4, so that slot + 1 fits 32 bits
+		cap[l] = std::min<size_t>(pow2_at_least(2 * static_cast<size_t>(h_cnt)), size_t(1) << 31);
+		uint32_t* table = nullptr;
+		ORT_CUDA(c, tmp.alloc(&table, cap[l]));
+		ORT_CUDA(c, cudaMemsetAsync(table, 0xFF, cap[l] * 4, st));
+		s.table = table;
+		ort::build_insert_kernel<<<blocks_for(items), 256, 0, st>>>(s, table, static_cast<uint32_t>(cap[l] - 1), d_cnt);
+		ort::write_fill_kernel<<<blocks_for(static_cast<size_t>(G[l].gx) * G[l].gy * G[l].gz), 256, 0, st>>>(G[l], s.rx, s.ry, s.rz, s.rgx, s.rgy, s.rgz, canon);
+		c->launches += 2;
+		ORT_CUDA(c, cudaGetLastError());
+	}
+	uint32_t h_root = 0;
+	ORT_CUDA(c, cudaMemcpyAsync(&h_root, G[1].ids, 4, cudaMemcpyDeviceToHost, st));
+	ORT_CUDA(c, cudaStreamSynchronize(st));
+
+	// top-down numbering from the new root, as the builder's
+	size_t n_lvl[kWriteMaxDepth + 2] = {}, base[kWriteMaxDepth + 2] = {};
+	uint32_t* frontier[kWriteMaxDepth + 2] = {};
+	uint32_t* rows[kWriteMaxDepth + 2] = {};
+	size_t total = 0;
+	for (int l = 1; l <= D + 1; ++l) base[l] = 1;
+	if (h_root)
+	{
+		size_t max_cap = 0;
+		for (int l = 2; l <= D; ++l) max_cap = std::max(max_cap, cap[l]);
+		uint32_t* first = nullptr;
+		ORT_CUDA(c, tmp.alloc(&first, max_cap));
+		ORT_CUDA(c, tmp.alloc(&frontier[1], 1));
+		ORT_CUDA(c, cudaMemcpyAsync(frontier[1], G[1].ids, 4, cudaMemcpyDeviceToDevice, st));
+		n_lvl[1] = 1;
+		for (int l = 1; l < D; ++l)
+		{
+			base[l + 1] = base[l] + n_lvl[l];
+			ORT_CUDA(c, tmp.alloc(&rows[l], 8 * n_lvl[l]));
+			if ((rc = top_down_step(c, tmp, td, S[l], frontier[l], n_lvl[l], first, cap[l + 1], static_cast<uint32_t>(base[l + 1]), rows[l],
+			                        &frontier[l + 1], &n_lvl[l + 1])) != ORT_OK)
+				return rc;
+			if (base[l + 1] - 1 + n_lvl[l + 1] > ort::kIdMask)
+				return ort_fail(c, ORT_ERR_CAPACITY, "ort_write_voxels: the resulting DAG has more than the %u compact ids allow", ort::kIdMask);
+		}
+		ORT_CUDA(c, tmp.alloc(&rows[D], 8 * n_lvl[D]));
+		ort::build_leaf_rows_kernel<<<blocks_for(n_lvl[D]), 256, 0, st>>>(frontier[D], n_lvl[D], S[D], rows[D]);
+		++c->launches;
+		ORT_CUDA(c, cudaGetLastError());
+		total = base[D] - 1 + n_lvl[D];
+	}
+	ORT_CUDA(c, cudaStreamSynchronize(st));
+
+	// install: grown with ort_upload_full's head-room when the current array is too small
+	NewMirror fresh;
+	size_t out_cap = 0;
+	if (total > c->cap_nodes)
+	{
+		out_cap = std::min<size_t>(total + total / 4 + 4096, ort::kIdMask);
+		ORT_CUDA(c, cudaMalloc(&fresh.p, out_cap * 32));
+	}
+	const uint32_t* parts[kWriteMaxDepth + 1] = {};
+	for (int l = 1; l <= D; ++l) parts[l - 1] = rows[l];
+	return install_mirror(c, fresh, out_cap, parts, n_lvl + 1, D, total, base, tmp.bytes, n_out, level_offsets);
 }
 
 }  // namespace
@@ -1057,6 +1294,26 @@ int ort_build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, int nx, int
 		                voxels, elem_bytes, nx, ny, nz, dim);
 	DeviceGuard g(c->device);
 	const int rc = build_voxels(c, voxels, elem_bytes, static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz), n_nodes, level_offsets);
+	if (rc != ORT_OK) cudaGetLastError();       // (an allocation that failed leaves its error behind for the next check)
+	return rc;
+}
+
+int ort_write_voxels(ort_ctx* c, int x0, int y0, int z0, const void* voxels, int elem_bytes, int nx, int ny, int nz, size_t* n_nodes, uint32_t* level_offsets)
+{
+	enter(c);
+	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_write_voxels: null context");
+	if (c->index_base != 1)
+		return ort_fail(c, ORT_ERR_INVALID, "ort_write_voxels: the context holds an och::octree pool, not a DAG");
+	const long long dim = 1ll << c->depth;
+	const auto axis_ok = [dim](int o, int e) { return o >= 0 && e >= 1 && e <= kWriteMaxExtent && static_cast<long long>(o) + e <= dim; };
+	if (!axis_ok(x0, nx) || !axis_ok(y0, ny) || !axis_ok(z0, nz))
+		return ort_fail(c, ORT_ERR_INVALID, "ort_write_voxels: box origin (%d, %d, %d) extent (%d, %d, %d) is not inside the cube of %lld voxels a side "
+		                "with 1..%d per axis", x0, y0, z0, nx, ny, nz, dim, kWriteMaxExtent);
+	if (!voxels || (elem_bytes != 1 && elem_bytes != 4))
+		return ort_fail(c, ORT_ERR_INVALID, "ort_write_voxels: bad arguments (voxels=%p elem_bytes=%d)", voxels, elem_bytes);
+	DeviceGuard g(c->device);
+	const int rc = write_voxels(c, static_cast<uint32_t>(x0), static_cast<uint32_t>(y0), static_cast<uint32_t>(z0), voxels, elem_bytes,
+	                            static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz), n_nodes, level_offsets);
 	if (rc != ORT_OK) cudaGetLastError();       // (an allocation that failed leaves its error behind for the next check)
 	return rc;
 }

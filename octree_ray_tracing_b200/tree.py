@@ -114,34 +114,54 @@ class TraceContext:
         assert a.shape[0] == i.size
         self._ck(self.L.ort_upload_delta(self.h, _p(i), _p(a), i.size, root))
 
+    def _voxel_source(self, grid, what: str) -> int:
+        """Check a dense voxel grid for the library (see upload_voxels) and return its element size; a CUDA tensor's
+        producer is waited for, since the library reads it on its own stream."""
+        if isinstance(grid, np.ndarray):
+            if grid.dtype not in (np.uint8, np.int32, np.uint32):
+                raise TypeError(f"{what}: dtype {grid.dtype} (uint8, int32 or uint32 required)")
+            if grid.ndim != 3 or not grid.flags.c_contiguous:
+                raise ValueError(f"{what}: a C-contiguous 3-D array of shape (nz, ny, nx) is required")
+            return grid.dtype.itemsize
+        if hasattr(grid, "data_ptr"):
+            import torch
+            if grid.dtype not in (torch.uint8, torch.int32, torch.uint32):
+                raise TypeError(f"{what}: dtype {grid.dtype} (uint8, int32 or uint32 required)")
+            if grid.dim() != 3 or not grid.is_contiguous():
+                raise ValueError(f"{what}: a contiguous 3-D tensor of shape (nz, ny, nx) is required")
+            if grid.is_cuda:
+                if grid.device.index != self.device:
+                    raise ValueError(f"{what}: the tensor is on {grid.device}, the context on cuda:{self.device}")
+                torch.cuda.current_stream(grid.device).synchronize()      # the library reads it on its own stream
+            return grid.element_size()
+        raise TypeError(f"{what}: numpy array or torch tensor required, got {type(grid).__name__}")
+
     def upload_voxels(self, grid):
         """Build the DAG of a dense voxel grid on this context's GPU and install it as the mirror (ort_build_voxels).
         grid: C-contiguous 3-D numpy array or torch tensor (CPU or CUDA) of shape (nz, ny, nx), dtype uint8, int32 or
         uint32 (read as unsigned); grid[z, y, x] is voxel (x, y, z), 0 = empty.  Returns (n_nodes, level_offsets):
         the mirror then holds what HOctree.flatten() gives for a table holding these voxels."""
-        if isinstance(grid, np.ndarray):
-            if grid.dtype not in (np.uint8, np.int32, np.uint32):
-                raise TypeError(f"upload_voxels: dtype {grid.dtype} (uint8, int32 or uint32 required)")
-            if grid.ndim != 3 or not grid.flags.c_contiguous:
-                raise ValueError("upload_voxels: a C-contiguous 3-D array of shape (nz, ny, nx) is required")
-            elem = grid.dtype.itemsize
-        elif hasattr(grid, "data_ptr"):
-            import torch
-            if grid.dtype not in (torch.uint8, torch.int32, torch.uint32):
-                raise TypeError(f"upload_voxels: dtype {grid.dtype} (uint8, int32 or uint32 required)")
-            if grid.dim() != 3 or not grid.is_contiguous():
-                raise ValueError("upload_voxels: a contiguous 3-D tensor of shape (nz, ny, nx) is required")
-            if grid.is_cuda:
-                if grid.device.index != self.device:
-                    raise ValueError(f"upload_voxels: the tensor is on {grid.device}, the context on cuda:{self.device}")
-                torch.cuda.current_stream(grid.device).synchronize()      # the builder reads it on its own stream
-            elem = grid.element_size()
-        else:
-            raise TypeError(f"upload_voxels: numpy array or torch tensor required, got {type(grid).__name__}")
+        elem = self._voxel_source(grid, "upload_voxels")
         nz, ny, nx = (int(s) for s in grid.shape)
         n = C.c_size_t(0)
         lo = np.zeros(self.depth + 1, np.uint32)
         self._ck(self.L.ort_build_voxels(self.h, _p(grid), elem, nx, ny, nz, C.byref(n), _p(lo)))
+        return n.value, lo
+
+    def write_voxels(self, origin, grid):
+        """Write a dense box of voxels into the DAG on this context's GPU and install the result as the mirror
+        (ort_write_voxels).  origin: (x0, y0, z0); grid: as for upload_voxels, shape (nz, ny, nx) with at most 2048 per
+        axis -- read_voxels(origin, extent)'s output is taken as it is.  Voxel (x0 + i, y0 + j, z0 + k) becomes
+        grid[k, j, i] (0 erases); every voxel outside the box keeps its value.  The box must lie inside the cube.
+        Returns (n_nodes, level_offsets): the mirror then holds what HOctree.flatten() gives for a table holding the
+        resulting voxels.  As after upload_voxels, an HOctree attached to this context no longer describes the mirror
+        and must attach() again before its next sync."""
+        x0, y0, z0 = (int(v) for v in origin)
+        elem = self._voxel_source(grid, "write_voxels")
+        nz, ny, nx = (int(s) for s in grid.shape)
+        n = C.c_size_t(0)
+        lo = np.zeros(self.depth + 1, np.uint32)
+        self._ck(self.L.ort_write_voxels(self.h, x0, y0, z0, _p(grid), elem, nx, ny, nz, C.byref(n), _p(lo)))
         return n.value, lo
 
     def read_nodes(self, first: int = 1, n: int | None = None) -> np.ndarray:
