@@ -119,6 +119,33 @@ int ort_build_voxels(ort_ctx* ctx, const void* voxels, int elem_bytes, int nx, i
  * host table attached to ctx no longer describes the mirror afterwards. */
 int ort_write_voxels(ort_ctx* ctx, int x0, int y0, int z0, const void* voxels, int elem_bytes,
                      int nx, int ny, int nz, size_t* n_nodes, uint32_t* level_offsets);
+/* Patch the box [x0, x0+nx) x [y0, y0+ny) x [z0, z0+nz) of voxels into the DAG on ctx's GPU in place, at a cost that
+ * grows with the box (cells it cuts x depth), not with the scene.  Same voxel contract as ort_write_voxels (layout,
+ * 1- or 4-byte elements, host or device source, 0 erases, every voxel outside the box keeps what ort_voxels_at returned),
+ * with at most 512 voxels per axis; bigger boxes go through ort_write_voxels or several patches.
+ * Mirror contract (unlike ort_write_voxels, the result is not ort_tree_flatten's form):
+ *   - rows 1 .. n_old (n_old = ort_node_count before the call) are not modified.  New rows are appended as ids
+ *     n_old+1 .. n_old+*n_added (n_added optional), the root is replaced and ort_node_count grows by *n_added.
+ *   - no duplicates: no appended row has the content of a row the patch index holds at the same level, and no two
+ *     appended rows of one level are equal.  The patch index holds the rows reachable from the root when it was built
+ *     (by the first patch after the mirror changed by any other call) plus every row appended since.  So when the
+ *     reachable DAG had no duplicates, it has none afterwards: its reachable node count is ort_tree_flatten's n.
+ *   - deterministic numbering: new ids are assigned level by level from the leaf level up to the root level; within a
+ *     level in the raster order (x fastest, then y, then z) of the first cell of the level that the box cuts and that
+ *     has each new content.  Where several index rows hold the same content, the smallest id is used.  The same
+ *     patches on the same mirror give byte-identical mirrors on any GPU, so replicas stay identical without rows sent.
+ *   - a content of all zeros is id 0 and no row: a scene that becomes empty has root 0, and its rows stay.
+ *   Garbage rows accumulate over a long session; ort_write_voxels of any box returns the mirror to ort_tree_flatten's form.
+ * Frames queued before the call (async launches, defer_sync host frames, work on a caller's stream) trace the old scene:
+ * they read rows <= n_old only.  The call does not wait for the device unless the mirror must grow (reallocated as in
+ * ort_upload_full) or the index is built or grown; it ends with one small readback on ort_stream(ctx).
+ * ORT_ERR_INVALID for bad arguments, a box outside the cube or wider than 512, a source on another device, a misaligned
+ * device source or the och::octree pool layout; ORT_ERR_CAPACITY when an appended id would pass 2^29 - 1 (rows written
+ * past n_old are then simply unused); ORT_ERR_CUDA when device memory runs out.  After any failure the rows, root,
+ * ort_node_count and later frames are unchanged.  ort_build_bytes is not changed.  A host table attached to ctx no
+ * longer describes the mirror afterwards. */
+int ort_patch_voxels(ort_ctx* ctx, int x0, int y0, int z0, const void* voxels, int elem_bytes,
+                     int nx, int ny, int nz, size_t* n_added);
 /* Copy n rows of the device mirror, starting at compact id first (1-based), to nodes8 (host or device). */
 int ort_read_nodes(ort_ctx* ctx, uint32_t first, size_t n, uint32_t* nodes8);
 /* Device bytes the last successful ort_build_voxels or ort_write_voxels allocated: its temporaries plus a new mirror if it

@@ -40,6 +40,7 @@ _SIGS = {
     "ort_build_voxels": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t), _vp]),
     "ort_read_nodes": (C.c_int, [_vp, C.c_uint32, C.c_size_t, _vp]),
     "ort_write_voxels": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t), _vp]),
+    "ort_patch_voxels": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "ort_build_bytes": (C.c_uint64, [_vp]),
     "ort_voxels_at": (C.c_int, [_vp, _vp, C.c_size_t, _vp]),
     "ort_read_voxels": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp]),

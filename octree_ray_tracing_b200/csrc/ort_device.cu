@@ -115,6 +115,14 @@ struct ort_ctx
 	uint64_t beam_builds = 0;
 	uint64_t build_bytes = 0;           // device bytes the last successful ort_build_voxels or ort_write_voxels allocated (its peak)
 
+	// ort_patch_voxels (ort_patch.cuh): the patch index, one table of row ids per level 1 .. depth, valid while no other
+	// route has changed the rows since it was built; pidx_rows[l] bounds its entries.  And the per-call scratch.
+	uint32_t* d_pidx[17] = {};
+	size_t   pidx_cap[17] = {};
+	size_t   pidx_rows[17] = {};
+	bool     pidx_valid = false;
+	void*    d_patch = nullptr;  size_t d_patch_bytes = 0;
+
 	unsigned long long* d_counters = nullptr; // work counters of the persistent kernels: a ring, one per launch (kCounterRing)
 	unsigned next_counter = 0;
 	int max_blocks_rays = 0, max_blocks_frame = 0;
@@ -241,11 +249,13 @@ void band_map_release(BandMap& m)
 	m = BandMap{};
 }
 
-// the DAG changed: every beam grid is out of date (rebuilt by the next frame launch that wants one)
+// the DAG changed: every beam grid is out of date (rebuilt by the next frame launch that wants one), and so is the patch
+// index (rebuilt by the next ort_patch_voxels)
 inline void beam_invalidate(ort_ctx* c)
 {
 	for (bool& v : c->beam_valid) v = false;
 	c->beam_dag_age = 0;
+	c->pidx_valid = false;
 }
 
 }  // namespace
@@ -253,6 +263,7 @@ inline void beam_invalidate(ort_ctx* c)
 #include "ort_kernels.cuh"
 #include "ort_build.cuh"
 #include "ort_write.cuh"
+#include "ort_patch.cuh"
 #include "ort_query.cuh"
 
 static_assert(ort::kBeamFineLevel == 8, "ort_ctx holds the beam grids of levels 0 .. 8");
@@ -678,6 +689,8 @@ int ort_destroy(ort_ctx* c)
 	cudaFree(c->d_palette);
 	cudaFree(c->d_counters);
 	cudaFree(c->d_stage);
+	cudaFree(c->d_patch);
+	for (uint32_t* t : c->d_pidx) cudaFree(t);
 	for (BandMap& m : c->band_maps) band_map_release(m);
 	cudaFree(c->d_beam_tmp);
 	for (int k = 0; k <= ort::kBeamFineLevel; ++k) { cudaFree(c->d_beam_skip[k][0]); cudaFree(c->d_beam_skip[k][1]); }
@@ -932,9 +945,9 @@ int install_mirror(ort_ctx* c, NewMirror& fresh, size_t out_cap, const uint32_t*
 	return ORT_OK;
 }
 
-// The `count` voxels of a builder or write source on this context's device: `voxels` itself when it is device memory
-// there (checked: this device, aligned to its element size), else a copy in `tmp` enqueued on the context's stream.
-int device_voxels(ort_ctx* c, const char* what, const void* voxels, int elem_bytes, size_t count, BuildTemps& tmp, const void** src)
+// Whether a voxel source is device memory; a device source must be on this context's device and aligned to its
+// element size (ORT_ERR_INVALID otherwise).
+int voxel_source_kind(ort_ctx* c, const char* what, const void* voxels, int elem_bytes, bool* dev_out)
 {
 	cudaPointerAttributes a;
 	const bool dev = cudaPointerGetAttributes(&a, voxels) == cudaSuccess && (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged);
@@ -943,6 +956,17 @@ int device_voxels(ort_ctx* c, const char* what, const void* voxels, int elem_byt
 		return ort_fail(c, ORT_ERR_INVALID, "%s: the voxels live on device %d, the context on device %d", what, a.device, c->device);
 	if (dev && (reinterpret_cast<uintptr_t>(voxels) & static_cast<uintptr_t>(elem_bytes - 1)))
 		return ort_fail(c, ORT_ERR_INVALID, "%s: a device source of %d-byte elements must be %d-byte aligned", what, elem_bytes, elem_bytes);
+	*dev_out = dev;
+	return ORT_OK;
+}
+
+// The `count` voxels of a builder or write source on this context's device: `voxels` itself when it is device memory
+// there (checked: this device, aligned to its element size), else a copy in `tmp` enqueued on the context's stream.
+int device_voxels(ort_ctx* c, const char* what, const void* voxels, int elem_bytes, size_t count, BuildTemps& tmp, const void** src)
+{
+	bool dev = false;
+	const int rc = voxel_source_kind(c, what, voxels, elem_bytes, &dev);
+	if (rc != ORT_OK) return rc;
 	*src = voxels;
 	if (!dev)
 	{
@@ -1496,6 +1520,272 @@ int ort_read_voxels(ort_ctx* c, int x0, int y0, int z0, int nx, int ny, int nz, 
 	ORT_CUDA(c, cudaStreamSynchronize(c->copy_stream));
 	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
 	return ORT_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// a dense box of voxels patched into the device DAG, append-only (ort_patch.cuh, DESIGN section 16)
+// ------------------------------------------------------------------------------------------------
+
+namespace {
+
+constexpr int kPatchMaxExtent = 512;          // voxels per axis of one patch: bounds its scratch and reserved rows
+
+// Room in the mirror for ids up to `rows` (the caller clips that to kIdMask).  Growing reallocates the array every launch
+// in flight reads, as ort_upload_full does, so it waits for the whole device first; rows 1 .. n_nodes are kept.
+int patch_reserve(ort_ctx* c, size_t rows, size_t bound)
+{
+	if (rows <= c->cap_nodes) return ORT_OK;
+	const size_t n = c->n_nodes;
+	const size_t want = std::min<size_t>(n + n / 4 + 4096 + bound, ort::kIdMask);
+	ORT_CUDA(c, cudaDeviceSynchronize());
+	NewMirror fresh;
+	ORT_CUDA(c, cudaMalloc(&fresh.p, want * 32));
+	if (n) ORT_CUDA(c, cudaMemcpyAsync(fresh.p, c->d_nodes, n * 32, cudaMemcpyDeviceToDevice, c->stream));
+	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
+	cudaFree(c->d_nodes);
+	c->d_nodes = fresh.p;
+	c->cap_nodes = static_cast<uint32_t>(want);
+	fresh.p = nullptr;
+	return ORT_OK;
+}
+
+// A level's index table of at least `cap` entries, emptied (the previous table is dropped).
+int patch_index_table(ort_ctx* c, int l, size_t cap)
+{
+	if (c->pidx_cap[l] < cap)
+	{
+		cudaFree(c->d_pidx[l]);
+		c->d_pidx[l] = nullptr;
+		c->pidx_cap[l] = 0;
+		ORT_CUDA(c, cudaMalloc(&c->d_pidx[l], cap * 4));
+		c->pidx_cap[l] = cap;
+	}
+	ORT_CUDA(c, cudaMemsetAsync(c->d_pidx[l], 0xFF, c->pidx_cap[l] * 4, c->stream));
+	return ORT_OK;
+}
+
+// The patch index of the current rows: the ids reachable at each level from the root (ort_write_voxels' first step),
+// each level's table sized for them plus `cells[l]` appended rows at a load of at most 1/2.
+int patch_index_build(ort_ctx* c, const ort::WriteDag& g, uint32_t old_root, const size_t* cells)
+{
+	const int D = c->depth;
+	cudaStream_t st = c->stream;
+	BuildTemps tmp;
+	TopDown td;
+	uint32_t* ids[kWriteMaxDepth + 2] = {};
+	size_t n[kWriteMaxDepth + 2] = {};
+	if (old_root)
+	{
+		ORT_CUDA(c, tmp.alloc(&ids[1], 1));
+		ORT_CUDA(c, cudaMemcpyAsync(ids[1], &old_root, 4, cudaMemcpyHostToDevice, st));
+		n[1] = 1;
+		uint32_t* first = nullptr;
+		ORT_CUDA(c, tmp.alloc(&first, c->n_nodes));
+		int rc;
+		for (int l = 1; l < D && n[l]; ++l)
+			if ((rc = top_down_step(c, tmp, td, ort::OldSrc{ g }, ids[l], n[l], first, c->n_nodes, 0u, nullptr, &ids[l + 1], &n[l + 1])) != ORT_OK)
+				return rc;
+	}
+	for (int l = 1; l <= D; ++l)
+	{
+		const int rc = patch_index_table(c, l, pow2_at_least(2 * (n[l] + cells[l])));
+		if (rc != ORT_OK) return rc;
+		if (n[l])
+		{
+			ort::patch_index_build_kernel<<<blocks_for(n[l]), 256, 0, st>>>(ids[l], n[l], ort::PatchIndex{ c->d_pidx[l], static_cast<uint32_t>(c->pidx_cap[l] - 1) }, g.nodes_m1);
+			++c->launches;
+		}
+		c->pidx_rows[l] = n[l];
+	}
+	ORT_CUDA(c, cudaGetLastError());
+	ORT_CUDA(c, cudaStreamSynchronize(st));
+	c->pidx_valid = true;
+	return ORT_OK;
+}
+
+// Grow (rehash) each level's table whose load would pass 3/4 with `cells[l]` more rows.
+int patch_index_grow(ort_ctx* c, const uint32_t* nodes_m1, const size_t* cells)
+{
+	for (int l = 1; l <= c->depth; ++l)
+	{
+		const size_t need = c->pidx_rows[l] + cells[l];
+		if (4 * need <= 3 * c->pidx_cap[l]) continue;
+		const size_t cap = pow2_at_least(2 * need);
+		uint32_t* t = nullptr;
+		ORT_CUDA(c, cudaMalloc(&t, cap * 4));
+		const cudaError_t e = cudaMemsetAsync(t, 0xFF, cap * 4, c->stream);
+		if (e != cudaSuccess) { cudaFree(t); ORT_CUDA(c, e); }
+		if (c->pidx_cap[l])
+		{
+			ort::patch_index_rehash_kernel<<<blocks_for(c->pidx_cap[l]), 256, 0, c->stream>>>(c->d_pidx[l], c->pidx_cap[l], ort::PatchIndex{ t, static_cast<uint32_t>(cap - 1) }, nodes_m1);
+			++c->launches;
+		}
+		const cudaError_t k = cudaGetLastError();
+		if (k != cudaSuccess) { cudaFree(t); ORT_CUDA(c, k); }
+		cudaFree(c->d_pidx[l]);                 // (waits for the rehash)
+		c->d_pidx[l] = t;
+		c->pidx_cap[l] = cap;
+	}
+	return ORT_OK;
+}
+
+int patch_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* voxels, int elem_bytes, uint32_t nx, uint32_t ny, uint32_t nz,
+                 size_t* n_added)
+{
+	const int D = c->depth;
+	cudaStream_t st = c->stream;
+	bool dev = false;
+	int rc = voxel_source_kind(c, "ort_patch_voxels", voxels, elem_bytes, &dev);
+	if (rc != ORT_OK) return rc;
+
+	// R_l: the cells of level l the box cuts (origin ro, extent re); their count bounds the rows level l appends
+	uint32_t ro[kWriteMaxDepth + 2][3] = {}, re[kWriteMaxDepth + 2][3] = {};
+	size_t cells[kWriteMaxDepth + 2] = {}, bound = 0, max_cells = 0, max_cap = 0;
+	const uint32_t b0[3] = { x0, y0, z0 }, b1[3] = { x0 + nx - 1, y0 + ny - 1, z0 + nz - 1 };
+	for (int l = 1; l <= D; ++l)
+	{
+		for (int a = 0; a < 3; ++a)
+		{
+			ro[l][a] = b0[a] >> (D - l + 1);
+			re[l][a] = (b1[a] >> (D - l + 1)) - ro[l][a] + 1;
+		}
+		cells[l] = static_cast<size_t>(re[l][0]) * re[l][1] * re[l][2];
+		bound += cells[l];
+		max_cells = std::max(max_cells, cells[l]);
+		max_cap = std::max(max_cap, pow2_at_least(2 * cells[l]));
+	}
+
+	// rows for every id the patch may append (past the id limit the call is refused, so those are never needed)
+	const uint32_t n_old = c->n_nodes;
+	if ((rc = patch_reserve(c, std::min<size_t>(static_cast<size_t>(n_old) + bound, ort::kIdMask), bound)) != ORT_OK) return rc;
+	const ort::WriteDag g{ c->d_nodes - 8, c->has_root ? n_old + 1 : 0u };
+	const uint32_t old_root = c->has_root && c->root - 1u < g.lim - 1u ? c->root : 0u;
+	if (!c->pidx_valid)
+		rc = patch_index_build(c, g, old_root, cells);
+	else
+		rc = patch_index_grow(c, g.nodes_m1, cells);
+	if (rc != ORT_OK) return rc;
+
+	// scratch (words): first ids per level + root | non-empty counter | R_l's ids and old_at | local table + first
+	// occurrence | hits | flags and their scan
+	const auto words = [](size_t n) { return align_up(n, 64); };
+	const size_t w_state = words(D + 2), w_cnt = words(2), w_tf = words(2 * max_cap), w_hit = words(max_cells), w_flag = words(max_cells + 1);
+	size_t total = w_state + w_cnt + w_tf + w_hit + w_flag + words(ort::scan_scratch_words(max_cells + 1));
+	for (int l = 1; l <= D; ++l) total += 2 * words(cells[l]);
+	if (total * 4 > c->d_patch_bytes)
+	{
+		cudaFree(c->d_patch);                   // (waits for the previous patch)
+		c->d_patch = nullptr;
+		c->d_patch_bytes = 0;
+		ORT_CUDA(c, cudaMalloc(&c->d_patch, total * 4));
+		c->d_patch_bytes = total * 4;
+	}
+	uint32_t* w = static_cast<uint32_t*>(c->d_patch);
+	uint32_t* state = w;                        // state[l]: level l's first new id (state[0]: one past the last); state[D + 1]: root
+	w += w_state;
+	unsigned long long* d_cnt = reinterpret_cast<unsigned long long*>(w);
+	w += w_cnt;
+	ort::WriteGrid R[kWriteMaxDepth + 2] = {};
+	for (int l = 1; l <= D; ++l)
+	{
+		R[l].ox = ro[l][0]; R[l].oy = ro[l][1]; R[l].oz = ro[l][2];
+		R[l].gx = re[l][0]; R[l].gy = re[l][1]; R[l].gz = re[l][2];
+		R[l].ids = w; w += words(cells[l]);
+		R[l].old_at = w; w += words(cells[l]);
+	}
+	uint32_t* tf = w; w += w_tf;
+	uint32_t* hit = w; w += w_hit;
+	uint32_t* flag = w; w += w_flag;
+	uint32_t* scan = w;
+
+	// the source on the device: host sources through a staging slot
+	const void* src = voxels;
+	int slot = -1;
+	if (!dev)
+	{
+		const size_t bytes = static_cast<size_t>(nx) * ny * nz * elem_bytes;
+		if ((rc = ensure_dstage(c, 2 * align_up(bytes, 256))) != ORT_OK) return rc;
+		char* base = nullptr;
+		slot = query_slot(c, &base);
+		ORT_CUDA(c, cudaMemcpyAsync(base, voxels, bytes, cudaMemcpyHostToDevice, st));
+		src = base;
+	}
+	const ort::BuildInput in{ src, elem_bytes, nx, ny, nz };
+
+	// old nodes under R_l, top-down
+	ort::patch_begin_kernel<<<1, 1, 0, st>>>(R[1].old_at, old_root, state + D, n_old);
+	++c->launches;
+	for (int l = 2; l <= D; ++l)
+	{
+		ort::write_old_at_kernel<<<blocks_for(cells[l]), 256, 0, st>>>(R[l - 1], R[l], g);
+		++c->launches;
+	}
+	// bottom-up: intern R_l, probe the index with each new content's first cell, append the misses
+	for (int l = D; l >= 1; --l)
+	{
+		const ort::PatchSrc s{ l == D, in, x0, y0, z0, R[l], l == D ? R[l] : R[l + 1], g };
+		const size_t cap = pow2_at_least(2 * cells[l]);
+		ORT_CUDA(c, cudaMemsetAsync(tf, 0xFF, 2 * cap * 4, st));
+		ort::build_insert_kernel<<<blocks_for(cells[l]), 256, 0, st>>>(s, tf, static_cast<uint32_t>(cap - 1), d_cnt);
+		ort::patch_first_kernel<<<blocks_for(cells[l]), 256, 0, st>>>(R[l].ids, cells[l], tf + cap);
+		ort::patch_probe_kernel<<<blocks_for(cells[l] + 1), 256, 0, st>>>(s, tf + cap, ort::PatchIndex{ c->d_pidx[l], static_cast<uint32_t>(c->pidx_cap[l] - 1) }, hit, flag);
+		c->launches += 3;
+		ort::scan_exclusive(flag, cells[l] + 1, scan, st, c->launches);
+		ort::patch_rows_kernel<<<blocks_for(cells[l]), 256, 0, st>>>(s, tf + cap, hit, flag, state + l, c->cap_nodes, c->d_nodes - 8,
+		                                                            l == 1 ? state + D + 1 : nullptr);
+		++c->launches;
+		ORT_CUDA(c, cudaGetLastError());
+	}
+	// the appended rows enter the index (unless the call is refused below)
+	ort::PatchIndexSet set{};
+	set.depth = D;
+	for (int l = 1; l <= D; ++l) set.ix[l] = ort::PatchIndex{ c->d_pidx[l], static_cast<uint32_t>(c->pidx_cap[l] - 1) };
+	ort::patch_index_append_kernel<<<blocks_for(bound), 256, 0, st>>>(state, set, g.nodes_m1);
+	++c->launches;
+	ORT_CUDA(c, cudaGetLastError());
+	if (slot >= 0 && (rc = query_slot_done(c, slot, nullptr, nullptr, 0)) != ORT_OK) return rc;
+
+	// the one readback: first ids per level, root
+	uint32_t h[kWriteMaxDepth + 2] = {};
+	ORT_CUDA(c, cudaMemcpyAsync(h, state, (D + 2) * 4, cudaMemcpyDeviceToHost, st));
+	ORT_CUDA(c, cudaStreamSynchronize(st));
+	const uint32_t n_new = h[0] - 1;
+	if (n_new > ort::kIdMask)
+		return ort_fail(c, ORT_ERR_CAPACITY, "ort_patch_voxels: the patch would append ids past the %u compact ids allow (%u rows before it)", ort::kIdMask, n_old);
+	for (int l = 1; l <= D; ++l) c->pidx_rows[l] += h[l - 1] - h[l];
+	c->n_nodes = n_new;
+	c->root = h[D + 1];
+	c->has_root = c->root != 0;
+	beam_invalidate(c);
+	c->pidx_valid = true;                       // (the index now holds the appended rows too)
+	if (n_added) *n_added = n_new - n_old;
+	return ORT_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ort_patch_voxels(ort_ctx* c, int x0, int y0, int z0, const void* voxels, int elem_bytes, int nx, int ny, int nz, size_t* n_added)
+{
+	enter(c);
+	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_patch_voxels: null context");
+	if (c->index_base != 1)
+		return ort_fail(c, ORT_ERR_INVALID, "ort_patch_voxels: the context holds an och::octree pool, not a DAG");
+	const long long dim = 1ll << c->depth;
+	const auto axis_ok = [dim](int o, int e) { return o >= 0 && e >= 1 && e <= kPatchMaxExtent && static_cast<long long>(o) + e <= dim; };
+	if (!axis_ok(x0, nx) || !axis_ok(y0, ny) || !axis_ok(z0, nz))
+		return ort_fail(c, ORT_ERR_INVALID, "ort_patch_voxels: box origin (%d, %d, %d) extent (%d, %d, %d) is not inside the cube of %lld voxels a side "
+		                "with 1..%d per axis", x0, y0, z0, nx, ny, nz, dim, kPatchMaxExtent);
+	if (!voxels || (elem_bytes != 1 && elem_bytes != 4))
+		return ort_fail(c, ORT_ERR_INVALID, "ort_patch_voxels: bad arguments (voxels=%p elem_bytes=%d)", voxels, elem_bytes);
+	DeviceGuard g(c->device);
+	const int rc = patch_voxels(c, static_cast<uint32_t>(x0), static_cast<uint32_t>(y0), static_cast<uint32_t>(z0), voxels, elem_bytes,
+	                            static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz), n_added);
+	if (rc != ORT_OK) cudaGetLastError();       // (an allocation that failed leaves its error behind for the next check)
+	return rc;
 }
 
 }  // extern "C"

@@ -164,6 +164,25 @@ class TraceContext:
         self._ck(self.L.ort_write_voxels(self.h, x0, y0, z0, _p(grid), elem, nx, ny, nz, C.byref(n), _p(lo)))
         return n.value, lo
 
+    def patch_voxels(self, origin, grid) -> int:
+        """Patch a dense box of voxels into the DAG on this context's GPU in place (ort_patch_voxels): the same sources
+        and voxel rules as write_voxels, at most 512 per axis, at a cost that grows with the box, not the scene.  Rows
+        already in the mirror stay as they are; the changed nodes are appended (no content the mirror's reachable rows
+        or earlier patches already hold is appended again) and the root is replaced.  Returns the number of rows
+        appended.  compact() returns the mirror to HOctree.flatten()'s form."""
+        x0, y0, z0 = (int(v) for v in origin)
+        elem = self._voxel_source(grid, "patch_voxels")
+        nz, ny, nx = (int(s) for s in grid.shape)
+        n = C.c_size_t(0)
+        self._ck(self.L.ort_patch_voxels(self.h, x0, y0, z0, _p(grid), elem, nx, ny, nz, C.byref(n)))
+        return n.value
+
+    def compact(self):
+        """Drop the rows no longer reachable (left behind by patch_voxels): voxel (0, 0, 0) is written back unchanged
+        with write_voxels, which installs the flatten() form of the same voxels.  Returns write_voxels' result."""
+        v = self.voxels_at(np.zeros((1, 3), np.int32))
+        return self.write_voxels((0, 0, 0), v.reshape(1, 1, 1))
+
     def read_nodes(self, first: int = 1, n: int | None = None) -> np.ndarray:
         """Rows first .. first + n - 1 (compact ids, 1-based) of the device mirror as an (n, 8) uint32 array."""
         if n is None:
