@@ -6,6 +6,7 @@
 // table (ort_host_tree.cpp) stays the owner; edits arrive as (id, node) deltas and are scattered.
 #include "ort_internal.h"
 #include "ort_rcp_table.h"
+#include "ort_trace.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -117,9 +118,9 @@ struct ort_ctx
 
 	// ort_patch_voxels (ort_patch.cuh): the patch index, one table of row ids per level 1 .. depth, valid while no other
 	// route has changed the rows since it was built; pidx_rows[l] bounds its entries.  And the per-call scratch.
-	uint32_t* d_pidx[17] = {};
-	size_t   pidx_cap[17] = {};
-	size_t   pidx_rows[17] = {};
+	uint32_t* d_pidx[ort::kMaxDepth + 1] = {};
+	size_t   pidx_cap[ort::kMaxDepth + 1] = {};
+	size_t   pidx_rows[ort::kMaxDepth + 1] = {};
 	bool     pidx_valid = false;
 	void*    d_patch = nullptr;  size_t d_patch_bytes = 0;
 
@@ -256,6 +257,21 @@ inline void beam_invalidate(ort_ctx* c)
 	for (bool& v : c->beam_valid) v = false;
 	c->beam_dag_age = 0;
 	c->pidx_valid = false;
+}
+
+// Rows of a mirror array grown to hold `rows` ids: head-room for the deltas (and `extra` for the patch) that follow,
+// clipped to the compact ids, which are 29-bit (FastWalker: 3 bits of each stack entry carry the child index).
+inline size_t mirror_capacity(size_t rows, size_t extra = 0) { return std::min<size_t>(rows + rows / 4 + 4096 + extra, ort::kIdMask); }
+
+// The mirror now holds compact rows 1 .. n (h_octree layout) whose root is `root` (0: no tree).
+inline void set_mirror(ort_ctx* c, uint32_t n, uint32_t root)
+{
+	c->n_nodes = n;
+	c->root = root;
+	c->index_base = 1;
+	c->has_root = root != 0;
+	c->miss_t = __builtin_inff();
+	beam_invalidate(c);
 }
 
 }  // namespace
@@ -754,9 +770,7 @@ int ort_upload_full(ort_ctx* c, const uint32_t* nodes8, size_t n, uint32_t root)
 	ORT_CUDA(c, cudaDeviceSynchronize());
 	if (n > c->cap_nodes)
 	{
-		// grow with head-room for the deltas that will follow
-		size_t want = n + n / 4 + 4096;
-		if (want > ort::kIdMask) want = ort::kIdMask;   // compact ids are 29-bit (FastWalker: 3 bits of each stack entry carry the child index)
+		const size_t want = mirror_capacity(n);
 		cudaFree(c->d_nodes);
 		c->d_nodes = nullptr;
 		c->cap_nodes = 0;
@@ -766,12 +780,7 @@ int ort_upload_full(ort_ctx* c, const uint32_t* nodes8, size_t n, uint32_t root)
 	if (n)
 		ORT_CUDA(c, cudaMemcpyAsync(c->d_nodes, nodes8, n * 32, cudaMemcpyDefault, c->stream));
 	ORT_CUDA(c, cudaStreamSynchronize(c->stream));   // the source may be reused by the caller right away
-	c->n_nodes = static_cast<uint32_t>(n);
-	c->root = root;
-	c->index_base = 1;
-	c->has_root = root != 0;
-	c->miss_t = __builtin_inff();
-	beam_invalidate(c);
+	set_mirror(c, static_cast<uint32_t>(n), root);
 	return ORT_OK;
 }
 
@@ -897,23 +906,58 @@ inline size_t pow2_at_least(size_t v)
 	return p;
 }
 
-// A new mirror allocated by a build or write, freed unless it was installed.
+// Entries of an open-addressing table that holds n keys at a load of at most 1/2.
+inline size_t table_cap(size_t n) { return pow2_at_least(2 * n); }
+
+// Copy `bytes` of device results to the host on the context's stream and wait for them.
+int read_back(ort_ctx* c, void* host, const void* dev, size_t bytes)
+{
+	ORT_CUDA(c, cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, c->stream));
+	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
+	return ORT_OK;
+}
+
+// The current mirror as a write or patch reads it, and its root: 0 when there is no tree or the root lies past the rows.
+ort::WriteDag old_dag(const ort_ctx* c, uint32_t* root)
+{
+	const ort::WriteDag g{ c->d_nodes - 8, c->has_root ? c->n_nodes + 1 : 0u };
+	*root = c->has_root && c->root - 1u < g.lim - 1u ? c->root : 0u;
+	return g;
+}
+
+// A new mirror array of cap rows, allocated by a build, write or patch; freed unless it was installed.
 struct NewMirror
 {
 	uint32_t* p = nullptr;
+	size_t cap = 0;
 	~NewMirror() { cudaFree(p); }
+	// allocated when the context's array is too small for `rows` ids (else p stays null)
+	cudaError_t grow(const ort_ctx* c, size_t rows)
+	{
+		if (rows <= c->cap_nodes) return cudaSuccess;
+		cap = mirror_capacity(rows);
+		return cudaMalloc(&p, cap * 32);
+	}
+	// replaces the context's array; no launch may still read that one
+	void install(ort_ctx* c)
+	{
+		cudaFree(c->d_nodes);
+		c->d_nodes = p;
+		c->cap_nodes = static_cast<uint32_t>(cap);
+		p = nullptr;
+	}
 };
 
 // Install `total` compact rows (level l from id base[l]) as the mirror, as ort_upload_full does: every launch in flight
 // reads the array that is replaced, so the device is synchronised first.  The rows are the n_parts device buffers
-// `parts` (part_rows[i] rows each) in order; they go to fresh.p when out_cap != 0 (a new mirror of out_cap rows; a part
-// that already lies there is not copied), else over the current array.  temp_bytes: the call's other allocations.
-int install_mirror(ort_ctx* c, NewMirror& fresh, size_t out_cap, const uint32_t* const* parts, const size_t* part_rows, int n_parts,
+// `parts` (part_rows[i] rows each) in order; they go to fresh.p when it was allocated (a part that already lies there is
+// not copied), else over the current array.  temp_bytes: the call's other allocations.
+int install_mirror(ort_ctx* c, NewMirror& fresh, const uint32_t* const* parts, const size_t* part_rows, int n_parts,
                    size_t total, const size_t* base, uint64_t temp_bytes, size_t* n_out, uint32_t* level_offsets)
 {
 	const int D = c->depth;
 	ORT_CUDA(c, cudaDeviceSynchronize());
-	uint32_t* dst = out_cap ? fresh.p : c->d_nodes;
+	uint32_t* dst = fresh.p ? fresh.p : c->d_nodes;
 	size_t at = 0;
 	for (int i = 0; i < n_parts; ++i)
 	{
@@ -922,20 +966,9 @@ int install_mirror(ort_ctx* c, NewMirror& fresh, size_t out_cap, const uint32_t*
 		at += part_rows[i];
 	}
 	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
-	if (out_cap)
-	{
-		cudaFree(c->d_nodes);
-		c->d_nodes = fresh.p;
-		c->cap_nodes = static_cast<uint32_t>(out_cap);
-		fresh.p = nullptr;                                         // (owned by the context now)
-	}
-	c->n_nodes = static_cast<uint32_t>(total);
-	c->root = total ? 1u : 0u;
-	c->index_base = 1;
-	c->has_root = total != 0;
-	c->miss_t = __builtin_inff();
-	beam_invalidate(c);
-	c->build_bytes = temp_bytes + out_cap * 32;
+	if (fresh.p) fresh.install(c);
+	set_mirror(c, static_cast<uint32_t>(total), total ? 1u : 0u);
+	c->build_bytes = temp_bytes + fresh.cap * 32;
 	if (n_out) *n_out = total;
 	if (level_offsets)
 	{
@@ -979,6 +1012,23 @@ int device_voxels(ort_ctx* c, const char* what, const void* voxels, int elem_byt
 	return ORT_OK;
 }
 
+// The first occurrence of each distinct child among the `slots` child slots of `frontier` (src.rep / src.child,
+// ort_build.cuh): first (first_words words, indexed by child t - 1) and the slots' flags, scanned into ranks in pos.
+// last_flag, where not null, receives the last flag before the scan.
+template<class Src>
+int first_occurrences(ort_ctx* c, const Src& src, const uint32_t* frontier, size_t slots, uint32_t* ch, uint32_t* first, size_t first_words,
+                      uint32_t* pos, uint32_t* scan, uint32_t* last_flag)
+{
+	cudaStream_t st = c->stream;
+	ORT_CUDA(c, cudaMemsetAsync(first, 0xFF, first_words * 4, st));
+	ort::build_children_kernel<<<blocks_for(slots), 256, 0, st>>>(frontier, slots, src, ch, first);
+	ort::build_flags_kernel<<<blocks_for(slots), 256, 0, st>>>(ch, first, slots, pos);
+	c->launches += 2;
+	if (last_flag) ORT_CUDA(c, cudaMemcpyAsync(last_flag, pos + slots - 1, 4, cudaMemcpyDeviceToDevice, st));
+	ort::scan_exclusive(pos, slots, scan, st, c->launches);
+	return ORT_OK;
+}
+
 int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, uint32_t ny, uint32_t nz, size_t* n_out, uint32_t* level_offsets)
 {
 	const int D = c->depth;
@@ -987,7 +1037,7 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 
 	// the input, on this device
 	const void* src = nullptr;
-	const int rc = device_voxels(c, "ort_build_voxels", voxels, elem_bytes, static_cast<size_t>(nx) * ny * nz, tmp, &src);
+	int rc = device_voxels(c, "ort_build_voxels", voxels, elem_bytes, static_cast<size_t>(nx) * ny * nz, tmp, &src);
 	if (rc != ORT_OK) return rc;
 	const ort::BuildInput in{ src, elem_bytes, nx, ny, nz };
 
@@ -1011,13 +1061,12 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 	// bottom-up: a level's distinct contents are at most its non-empty cells, which are at most the level below's
 	ort::build_count_kernel<<<blocks_for(static_cast<size_t>(lv[D].gx) * lv[D].gy * lv[D].gz), 256, 0, st>>>(ort::DenseSrc{ true, in, lv[D], lv[D] }, d_cnt);
 	++c->launches;
-	ORT_CUDA(c, cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-	ORT_CUDA(c, cudaStreamSynchronize(st));
+	if ((rc = read_back(c, h_cnt, d_cnt, sizeof(unsigned long long))) != ORT_OK) return rc;
 	size_t bound = static_cast<size_t>(h_cnt[0]);
 	for (int l = D; l >= 1; --l)
 	{
 		const size_t cells = static_cast<size_t>(lv[l].gx) * lv[l].gy * lv[l].gz;
-		cap[l] = pow2_at_least(2 * std::min(bound, cells));      // load factor <= 1/2
+		cap[l] = table_cap(std::min(bound, cells));
 		ORT_CUDA(c, tmp.alloc(&lv[l].table, cap[l]));
 		lv[l].mask = static_cast<uint32_t>(cap[l] - 1);
 		ORT_CUDA(c, cudaMemsetAsync(lv[l].table, 0xFF, cap[l] * 4, st));
@@ -1025,12 +1074,10 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 		ort::build_count_table_kernel<<<blocks_for(cap[l]), 256, 0, st>>>(lv[l].table, cap[l], d_cnt + D + 1 + l);
 		c->launches += 2;
 		ORT_CUDA(c, cudaGetLastError());
-		ORT_CUDA(c, cudaMemcpyAsync(h_cnt + l, d_cnt + l, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-		ORT_CUDA(c, cudaStreamSynchronize(st));
+		if ((rc = read_back(c, h_cnt + l, d_cnt + l, sizeof(unsigned long long))) != ORT_OK) return rc;
 		bound = static_cast<size_t>(h_cnt[l]);
 	}
-	ORT_CUDA(c, cudaMemcpyAsync(h_cnt + D + 1, d_cnt + D + 1, sizeof(unsigned long long) * (D + 1), cudaMemcpyDeviceToHost, st));
-	ORT_CUDA(c, cudaStreamSynchronize(st));
+	if ((rc = read_back(c, h_cnt + D + 1, d_cnt + D + 1, sizeof(unsigned long long) * (D + 1))) != ORT_OK) return rc;
 
 	// final ids: level l holds ids base[l] .. base[l] + n[l] - 1
 	size_t n_lvl[ort::kBuildMaxDepth + 2] = {}, base[ort::kBuildMaxDepth + 2] = {};
@@ -1045,16 +1092,10 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 		return ort_fail(c, ORT_ERR_CAPACITY, "ort_build_voxels: the grid's DAG has %zu nodes, more than the %u compact ids allow", total, ort::kIdMask);
 
 	// the output rows: straight into a new mirror when the current one is too small, else a temporary copied over
-	uint32_t* out = nullptr;
-	size_t out_cap = 0;
 	NewMirror fresh;
-	if (total > c->cap_nodes)
-	{
-		out_cap = std::min<size_t>(total + total / 4 + 4096, ort::kIdMask);      // head-room for the deltas that follow, as ort_upload_full
-		ORT_CUDA(c, cudaMalloc(&fresh.p, out_cap * 32));
-		out = fresh.p;
-	}
-	else if (total)
+	ORT_CUDA(c, fresh.grow(c, total));
+	uint32_t* out = fresh.p;
+	if (!out && total)
 		ORT_CUDA(c, tmp.alloc(&out, total * 8));
 
 	if (total)
@@ -1076,11 +1117,8 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 		for (int l = 1; l < D; ++l)
 		{
 			const size_t slots = 8 * n_lvl[l];
-			ORT_CUDA(c, cudaMemsetAsync(first, 0xFF, cap[l + 1] * 4, st));
-			ort::build_children_kernel<<<blocks_for(slots), 256, 0, st>>>(frontier[l], slots, ort::DenseSrc{ false, in, lv[l], lv[l + 1] }, ch, first);
-			ort::build_flags_kernel<<<blocks_for(slots), 256, 0, st>>>(ch, first, slots, pos);
-			c->launches += 2;
-			ort::scan_exclusive(pos, slots, scratch, st, c->launches);
+			if ((rc = first_occurrences(c, ort::DenseSrc{ false, in, lv[l], lv[l + 1] }, frontier[l], slots, ch, first, cap[l + 1], pos, scratch, nullptr)) != ORT_OK)
+				return rc;
 			ort::build_rows_kernel<<<blocks_for(slots), 256, 0, st>>>(ch, first, pos, slots, static_cast<uint32_t>(base[l + 1]),
 			                                                          out + 8 * (base[l] - 1), frontier[l + 1]);
 			++c->launches;
@@ -1092,7 +1130,7 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 	}
 	ORT_CUDA(c, cudaStreamSynchronize(st));
 	const uint32_t* part = out;
-	return install_mirror(c, fresh, out_cap, &part, &total, 1, total, base, tmp.bytes, n_out, level_offsets);
+	return install_mirror(c, fresh, &part, &total, 1, total, base, tmp.bytes, n_out, level_offsets);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1100,7 +1138,6 @@ int build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, uint32_t nx, ui
 // ------------------------------------------------------------------------------------------------
 
 constexpr int kWriteMaxExtent = 2048;         // voxels per axis of one write: the builder's depth-11 envelope
-constexpr int kWriteMaxDepth = 16;
 
 // Scratch of the top-down passes (child slots, their scan, the scan's total), grown on demand.
 struct TopDown
@@ -1109,9 +1146,8 @@ struct TopDown
 	size_t cap = 0;
 };
 
-// One top-down step over the 8 n child slots of `frontier` (src.rep / src.child, ort_build.cuh): the first occurrence of
-// each distinct child (first: first_words words, indexed by child t - 1), the next frontier in order of first occurrence
-// (allocated in tmp, n_next entries) and, where rows is not null, the slots' final child ids next_base + rank.
+// One top-down step over the 8 n child slots of `frontier` (first_occurrences), then the next frontier in order of first
+// occurrence (allocated in tmp, n_next entries) and, where rows is not null, the slots' final child ids next_base + rank.
 template<class Src>
 int top_down_step(ort_ctx* c, BuildTemps& tmp, TopDown& td, const Src& src, const uint32_t* frontier, size_t n, uint32_t* first, size_t first_words,
                   uint32_t next_base, uint32_t* rows, uint32_t** next, size_t* n_next)
@@ -1128,16 +1164,11 @@ int top_down_step(ort_ctx* c, BuildTemps& tmp, TopDown& td, const Src& src, cons
 		ORT_CUDA(c, tmp.alloc(&td.scan, ort::scan_scratch_words(slots)));
 		td.cap = slots;
 	}
-	ORT_CUDA(c, cudaMemsetAsync(first, 0xFF, first_words * 4, st));
-	ort::build_children_kernel<<<blocks_for(slots), 256, 0, st>>>(frontier, slots, src, td.ch, first);
-	ort::build_flags_kernel<<<blocks_for(slots), 256, 0, st>>>(td.ch, first, slots, td.pos);
-	c->launches += 2;
-	ORT_CUDA(c, cudaMemcpyAsync(td.last, td.pos + slots - 1, 4, cudaMemcpyDeviceToDevice, st));      // the last flag ...
-	ort::scan_exclusive(td.pos, slots, td.scan, st, c->launches);
+	int rc = first_occurrences(c, src, frontier, slots, td.ch, first, first_words, td.pos, td.scan, td.last);      // the last flag ...
+	if (rc != ORT_OK) return rc;
 	ORT_CUDA(c, cudaMemcpyAsync(td.last + 1, td.pos + slots - 1, 4, cudaMemcpyDeviceToDevice, st));  // ... plus its rank: the count
 	uint32_t h[2] = {};
-	ORT_CUDA(c, cudaMemcpyAsync(h, td.last, 8, cudaMemcpyDeviceToHost, st));
-	ORT_CUDA(c, cudaStreamSynchronize(st));
+	if ((rc = read_back(c, h, td.last, 8)) != ORT_OK) return rc;
 	*n_next = static_cast<size_t>(h[0]) + h[1];
 	ORT_CUDA(c, tmp.alloc(next, *n_next));
 	ort::build_rows_kernel<<<blocks_for(slots), 256, 0, st>>>(td.ch, first, td.pos, slots, next_base, rows ? rows : td.ch, *next);
@@ -1146,8 +1177,45 @@ int top_down_step(ort_ctx* c, BuildTemps& tmp, TopDown& td, const Src& src, cons
 	return ORT_OK;
 }
 
-int write_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* voxels, int elem_bytes, uint32_t nx, uint32_t ny, uint32_t nz,
-                 size_t* n_out, uint32_t* level_offsets)
+// The distinct old ids reachable at each level l from the old root (old_dag), top-down: ids[l] (in tmp), n[l] of them.
+int reachable_ids(ort_ctx* c, BuildTemps& tmp, TopDown& td, const ort::WriteDag& g, uint32_t root, uint32_t** ids, size_t* n)
+{
+	if (!root) return ORT_OK;
+	ORT_CUDA(c, tmp.alloc(&ids[1], 1));
+	ORT_CUDA(c, cudaMemcpyAsync(ids[1], &root, 4, cudaMemcpyHostToDevice, c->stream));
+	n[1] = 1;
+	uint32_t* first = nullptr;
+	ORT_CUDA(c, tmp.alloc(&first, c->n_nodes));
+	int rc;
+	for (int l = 1; l < c->depth && n[l]; ++l)
+		if ((rc = top_down_step(c, tmp, td, ort::OldSrc{ g }, ids[l], n[l], first, c->n_nodes, 0u, nullptr, &ids[l + 1], &n[l + 1])) != ORT_OK)
+			return rc;
+	return ORT_OK;
+}
+
+// R_l, the cells of level l = 1 .. depth that a box cuts: a box of cells (origin and extent in cells of the level, no
+// buffers), cells[l] of them; sum and max over the levels.
+struct BoxCells
+{
+	ort::WriteGrid R[ort::kMaxDepth + 2] = {};
+	size_t cells[ort::kMaxDepth + 2] = {}, sum = 0, max = 0;
+	BoxCells(int D, const ort::QueryBox& b)
+	{
+		for (int l = 1; l <= D; ++l)
+		{
+			const int s = D - l + 1;
+			ort::WriteGrid& r = R[l];
+			r.ox = b.x0 >> s; r.gx = ((b.x0 + b.nx - 1) >> s) - r.ox + 1;
+			r.oy = b.y0 >> s; r.gy = ((b.y0 + b.ny - 1) >> s) - r.oy + 1;
+			r.oz = b.z0 >> s; r.gz = ((b.z0 + b.nz - 1) >> s) - r.oz + 1;
+			cells[l] = static_cast<size_t>(r.gx) * r.gy * r.gz;
+			sum += cells[l];
+			max = std::max(max, cells[l]);
+		}
+	}
+};
+
+int write_voxels(ort_ctx* c, const ort::QueryBox& b, const void* voxels, int elem_bytes, size_t* n_out, uint32_t* level_offsets)
 {
 	const int D = c->depth;
 	cudaStream_t st = c->stream;
@@ -1155,47 +1223,32 @@ int write_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* 
 	TopDown td;
 
 	const void* src = nullptr;
-	int rc = device_voxels(c, "ort_write_voxels", voxels, elem_bytes, static_cast<size_t>(nx) * ny * nz, tmp, &src);
+	int rc = device_voxels(c, "ort_write_voxels", voxels, elem_bytes, static_cast<size_t>(b.nx) * b.ny * b.nz, tmp, &src);
 	if (rc != ORT_OK) return rc;
-	const ort::BuildInput in{ src, elem_bytes, nx, ny, nz };
-	const ort::WriteDag g{ c->d_nodes - 8, c->has_root ? c->n_nodes + 1 : 0u };
-	const uint32_t old_root = c->has_root && c->root - 1u < g.lim - 1u ? c->root : 0u;
+	const ort::BuildInput in{ src, elem_bytes, b.nx, b.ny, b.nz };
+	uint32_t old_root = 0;
+	const ort::WriteDag g = old_dag(c, &old_root);
 	const size_t n_ids = c->has_root ? c->n_nodes : 0;         // old ids 1 .. n_ids
 
-	// R_l (the touched cells: origin ro, extent re) and G_l (the children of R_{l-1}; G_1 = R_1 = the root cell)
-	ort::WriteGrid G[kWriteMaxDepth + 2] = {};
-	uint32_t ro[kWriteMaxDepth + 2][3] = {}, re[kWriteMaxDepth + 2][3] = {};
-	const uint32_t b0[3] = { x0, y0, z0 }, b1[3] = { x0 + nx - 1, y0 + ny - 1, z0 + nz - 1 };
+	// G_l: the children of R_{l-1}; G_1 = R_1 = the root cell
+	const BoxCells box(D, b);
+	ort::WriteGrid G[ort::kMaxDepth + 2] = {};
 	for (int l = 1; l <= D; ++l)
 	{
-		for (int a = 0; a < 3; ++a)
-		{
-			ro[l][a] = b0[a] >> (D - l + 1);
-			re[l][a] = (b1[a] >> (D - l + 1)) - ro[l][a] + 1;
-		}
 		ort::WriteGrid& w = G[l];
-		w.ox = l == 1 ? 0u : 2 * ro[l - 1][0]; w.gx = l == 1 ? 1u : 2 * re[l - 1][0];
-		w.oy = l == 1 ? 0u : 2 * ro[l - 1][1]; w.gy = l == 1 ? 1u : 2 * re[l - 1][1];
-		w.oz = l == 1 ? 0u : 2 * ro[l - 1][2]; w.gz = l == 1 ? 1u : 2 * re[l - 1][2];
+		const ort::WriteGrid& p = box.R[l - 1];
+		w.ox = l == 1 ? 0u : 2 * p.ox; w.gx = l == 1 ? 1u : 2 * p.gx;
+		w.oy = l == 1 ? 0u : 2 * p.oy; w.gy = l == 1 ? 1u : 2 * p.gy;
+		w.oz = l == 1 ? 0u : 2 * p.oz; w.gz = l == 1 ? 1u : 2 * p.gz;
 		const size_t cells = static_cast<size_t>(w.gx) * w.gy * w.gz;
 		ORT_CUDA(c, tmp.alloc(&w.ids, cells));
 		ORT_CUDA(c, tmp.alloc(&w.old_at, cells));
 	}
 
 	// old DAG, top-down: the distinct old ids reachable at each level; the old node at every cell of each G_l
-	uint32_t* old[kWriteMaxDepth + 2] = {};
-	size_t n_old[kWriteMaxDepth + 2] = {};
-	if (old_root)
-	{
-		ORT_CUDA(c, tmp.alloc(&old[1], 1));
-		ORT_CUDA(c, cudaMemcpyAsync(old[1], &old_root, 4, cudaMemcpyHostToDevice, st));
-		n_old[1] = 1;
-		uint32_t* first = nullptr;
-		ORT_CUDA(c, tmp.alloc(&first, n_ids));
-		for (int l = 1; l < D && n_old[l]; ++l)
-			if ((rc = top_down_step(c, tmp, td, ort::OldSrc{ g }, old[l], n_old[l], first, n_ids, 0u, nullptr, &old[l + 1], &n_old[l + 1])) != ORT_OK)
-				return rc;
-	}
+	uint32_t* old[ort::kMaxDepth + 2] = {};
+	size_t n_old[ort::kMaxDepth + 2] = {};
+	if ((rc = reachable_ids(c, tmp, td, g, old_root, old, n_old)) != ORT_OK) return rc;
 	ORT_CUDA(c, cudaMemcpyAsync(G[1].old_at, &old_root, 4, cudaMemcpyHostToDevice, st));
 	for (int l = 2; l <= D; ++l)
 	{
@@ -1210,8 +1263,8 @@ int write_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* 
 	unsigned long long* d_cnt = nullptr;                        // [l] non-empty items of level l, [0] discarded
 	ORT_CUDA(c, tmp.alloc(&d_cnt, D + 1));
 	ORT_CUDA(c, cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long) * (D + 1), st));
-	ort::WriteSrc S[kWriteMaxDepth + 2] = {};
-	size_t cap[kWriteMaxDepth + 2] = {};
+	ort::WriteSrc S[ort::kMaxDepth + 2] = {};
+	size_t cap[ort::kMaxDepth + 2] = {};
 	for (int l = D; l >= 1; --l)
 	{
 		uint32_t* mapped = nullptr;
@@ -1224,25 +1277,24 @@ int write_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* 
 		ort::WriteSrc& s = S[l];
 		s.leaf = l == D;
 		s.in = in;
-		s.bx = x0; s.by = y0; s.bz = z0;
+		s.bx = b.x0; s.by = b.y0; s.bz = b.z0;
 		s.G = G[l];
 		s.C = l == D ? G[l] : G[l + 1];
-		s.rx = ro[l][0] - G[l].ox; s.ry = ro[l][1] - G[l].oy; s.rz = ro[l][2] - G[l].oz;
-		s.rgx = re[l][0]; s.rgy = re[l][1]; s.rgz = re[l][2];
+		s.rx = box.R[l].ox - G[l].ox; s.ry = box.R[l].oy - G[l].oy; s.rz = box.R[l].oz - G[l].oz;
+		s.rgx = box.R[l].gx; s.rgy = box.R[l].gy; s.rgz = box.R[l].gz;
 		s.g = g;
 		s.old = old[l];
 		s.n_old = static_cast<uint32_t>(n_old[l]);
 		s.mapped = mapped;
 		s.canon = canon;
-		const size_t items = n_old[l] + static_cast<size_t>(s.rgx) * s.rgy * s.rgz;
+		const size_t items = n_old[l] + box.cells[l];
 		ort::build_count_kernel<<<blocks_for(items), 256, 0, st>>>(s, d_cnt + l);
 		++c->launches;
 		ORT_CUDA(c, cudaGetLastError());
 		unsigned long long h_cnt = 0;
-		ORT_CUDA(c, cudaMemcpyAsync(&h_cnt, d_cnt + l, sizeof h_cnt, cudaMemcpyDeviceToHost, st));
-		ORT_CUDA(c, cudaStreamSynchronize(st));
-		// load factor <= 1/2; past 2^31 entries (a 2048^3 box over a large mirror) up to 3/4, so that slot + 1 fits 32 bits
-		cap[l] = std::min<size_t>(pow2_at_least(2 * static_cast<size_t>(h_cnt)), size_t(1) << 31);
+		if ((rc = read_back(c, &h_cnt, d_cnt + l, sizeof h_cnt)) != ORT_OK) return rc;
+		// past 2^31 entries (a 2048^3 box over a large mirror) the load goes up to 3/4, so that slot + 1 fits 32 bits
+		cap[l] = std::min<size_t>(table_cap(static_cast<size_t>(h_cnt)), size_t(1) << 31);
 		uint32_t* table = nullptr;
 		ORT_CUDA(c, tmp.alloc(&table, cap[l]));
 		ORT_CUDA(c, cudaMemsetAsync(table, 0xFF, cap[l] * 4, st));
@@ -1253,13 +1305,12 @@ int write_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* 
 		ORT_CUDA(c, cudaGetLastError());
 	}
 	uint32_t h_root = 0;
-	ORT_CUDA(c, cudaMemcpyAsync(&h_root, G[1].ids, 4, cudaMemcpyDeviceToHost, st));
-	ORT_CUDA(c, cudaStreamSynchronize(st));
+	if ((rc = read_back(c, &h_root, G[1].ids, 4)) != ORT_OK) return rc;
 
 	// top-down numbering from the new root, as the builder's
-	size_t n_lvl[kWriteMaxDepth + 2] = {}, base[kWriteMaxDepth + 2] = {};
-	uint32_t* frontier[kWriteMaxDepth + 2] = {};
-	uint32_t* rows[kWriteMaxDepth + 2] = {};
+	size_t n_lvl[ort::kMaxDepth + 2] = {}, base[ort::kMaxDepth + 2] = {};
+	uint32_t* frontier[ort::kMaxDepth + 2] = {};
+	uint32_t* rows[ort::kMaxDepth + 2] = {};
 	size_t total = 0;
 	for (int l = 1; l <= D + 1; ++l) base[l] = 1;
 	if (h_root)
@@ -1289,17 +1340,49 @@ int write_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* 
 	}
 	ORT_CUDA(c, cudaStreamSynchronize(st));
 
-	// install: grown with ort_upload_full's head-room when the current array is too small
+	// install, into a new array when the current one is too small
 	NewMirror fresh;
-	size_t out_cap = 0;
-	if (total > c->cap_nodes)
-	{
-		out_cap = std::min<size_t>(total + total / 4 + 4096, ort::kIdMask);
-		ORT_CUDA(c, cudaMalloc(&fresh.p, out_cap * 32));
-	}
-	const uint32_t* parts[kWriteMaxDepth + 1] = {};
+	ORT_CUDA(c, fresh.grow(c, total));
+	const uint32_t* parts[ort::kMaxDepth + 1] = {};
 	for (int l = 1; l <= D; ++l) parts[l - 1] = rows[l];
-	return install_mirror(c, fresh, out_cap, parts, n_lvl + 1, D, total, base, tmp.bytes, n_out, level_offsets);
+	return install_mirror(c, fresh, parts, n_lvl + 1, D, total, base, tmp.bytes, n_out, level_offsets);
+}
+
+// A public call that builds or edits the mirror from a voxel source: `run` on the context's device.  A failed call
+// leaves no CUDA error behind (an allocation that failed leaves its error for the next check).
+template<class Run>
+int mirror_call(ort_ctx* c, const char* what, const void* voxels, int elem_bytes, Run&& run)
+{
+	enter(c);
+	if (!c) return ort_fail(c, ORT_ERR_INVALID, "%s: null context", what);
+	if (!voxels || (elem_bytes != 1 && elem_bytes != 4))
+		return ort_fail(c, ORT_ERR_INVALID, "%s: bad arguments (voxels=%p elem_bytes=%d)", what, voxels, elem_bytes);
+	DeviceGuard g(c->device);
+	const int rc = run();
+	if (rc != ORT_OK) cudaGetLastError();
+	return rc;
+}
+
+// The box argument of a voxel call, ORT_ERR_INVALID unless it lies inside the cube with 1 .. max_extent voxels per axis
+// (max_extent 0: the cube's side).
+int voxel_box(ort_ctx* c, const char* what, int x0, int y0, int z0, int nx, int ny, int nz, int max_extent, ort::QueryBox* box)
+{
+	const long long dim = 1ll << c->depth, lim = max_extent ? std::min<long long>(max_extent, dim) : dim;
+	const auto axis_ok = [&](int o, int e) { return o >= 0 && e >= 1 && e <= lim && static_cast<long long>(o) + e <= dim; };
+	if (!axis_ok(x0, nx) || !axis_ok(y0, ny) || !axis_ok(z0, nz))
+		return ort_fail(c, ORT_ERR_INVALID, "%s: box origin (%d, %d, %d) extent (%d, %d, %d) is not inside the cube of %lld voxels a side "
+		                "with 1..%lld per axis", what, x0, y0, z0, nx, ny, nz, dim, lim);
+	*box = ort::QueryBox{ static_cast<uint32_t>(x0), static_cast<uint32_t>(y0), static_cast<uint32_t>(z0),
+	                      static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz) };
+	return ORT_OK;
+}
+
+// The box of a write or patch, which edit a DAG, not an och::octree pool.
+int edit_box(ort_ctx* c, const char* what, int x0, int y0, int z0, int nx, int ny, int nz, int max_extent, ort::QueryBox* box)
+{
+	if (c->index_base != 1)
+		return ort_fail(c, ORT_ERR_INVALID, "%s: the context holds an och::octree pool, not a DAG", what);
+	return voxel_box(c, what, x0, y0, z0, nx, ny, nz, max_extent, box);
 }
 
 }  // namespace
@@ -1308,38 +1391,23 @@ extern "C" {
 
 int ort_build_voxels(ort_ctx* c, const void* voxels, int elem_bytes, int nx, int ny, int nz, size_t* n_nodes, uint32_t* level_offsets)
 {
-	enter(c);
-	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: null context");
-	if (c->depth > ort::kBuildMaxDepth)
-		return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: context depth %d; the builder takes depth <= %d", c->depth, ort::kBuildMaxDepth);
-	const int dim = 1 << c->depth;
-	if (!voxels || (elem_bytes != 1 && elem_bytes != 4) || nx < 1 || ny < 1 || nz < 1 || nx > dim || ny > dim || nz > dim)
-		return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: bad arguments (voxels=%p elem_bytes=%d extent %d x %d x %d, 1..%d per axis)",
-		                voxels, elem_bytes, nx, ny, nz, dim);
-	DeviceGuard g(c->device);
-	const int rc = build_voxels(c, voxels, elem_bytes, static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz), n_nodes, level_offsets);
-	if (rc != ORT_OK) cudaGetLastError();       // (an allocation that failed leaves its error behind for the next check)
-	return rc;
+	return mirror_call(c, "ort_build_voxels", voxels, elem_bytes, [&] {
+		if (c->depth > ort::kBuildMaxDepth)
+			return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: context depth %d; the builder takes depth <= %d", c->depth, ort::kBuildMaxDepth);
+		const int dim = 1 << c->depth;
+		if (nx < 1 || ny < 1 || nz < 1 || nx > dim || ny > dim || nz > dim)
+			return ort_fail(c, ORT_ERR_INVALID, "ort_build_voxels: bad extent %d x %d x %d, 1..%d per axis", nx, ny, nz, dim);
+		return build_voxels(c, voxels, elem_bytes, static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz), n_nodes, level_offsets);
+	});
 }
 
 int ort_write_voxels(ort_ctx* c, int x0, int y0, int z0, const void* voxels, int elem_bytes, int nx, int ny, int nz, size_t* n_nodes, uint32_t* level_offsets)
 {
-	enter(c);
-	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_write_voxels: null context");
-	if (c->index_base != 1)
-		return ort_fail(c, ORT_ERR_INVALID, "ort_write_voxels: the context holds an och::octree pool, not a DAG");
-	const long long dim = 1ll << c->depth;
-	const auto axis_ok = [dim](int o, int e) { return o >= 0 && e >= 1 && e <= kWriteMaxExtent && static_cast<long long>(o) + e <= dim; };
-	if (!axis_ok(x0, nx) || !axis_ok(y0, ny) || !axis_ok(z0, nz))
-		return ort_fail(c, ORT_ERR_INVALID, "ort_write_voxels: box origin (%d, %d, %d) extent (%d, %d, %d) is not inside the cube of %lld voxels a side "
-		                "with 1..%d per axis", x0, y0, z0, nx, ny, nz, dim, kWriteMaxExtent);
-	if (!voxels || (elem_bytes != 1 && elem_bytes != 4))
-		return ort_fail(c, ORT_ERR_INVALID, "ort_write_voxels: bad arguments (voxels=%p elem_bytes=%d)", voxels, elem_bytes);
-	DeviceGuard g(c->device);
-	const int rc = write_voxels(c, static_cast<uint32_t>(x0), static_cast<uint32_t>(y0), static_cast<uint32_t>(z0), voxels, elem_bytes,
-	                            static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz), n_nodes, level_offsets);
-	if (rc != ORT_OK) cudaGetLastError();       // (an allocation that failed leaves its error behind for the next check)
-	return rc;
+	return mirror_call(c, "ort_write_voxels", voxels, elem_bytes, [&] {
+		ort::QueryBox box;
+		const int rc = edit_box(c, "ort_write_voxels", x0, y0, z0, nx, ny, nz, kWriteMaxExtent, &box);
+		return rc != ORT_OK ? rc : write_voxels(c, box, voxels, elem_bytes, n_nodes, level_offsets);
+	});
 }
 
 int ort_read_nodes(ort_ctx* c, uint32_t first, size_t n, uint32_t* nodes8)
@@ -1471,18 +1539,14 @@ int ort_read_voxels(ort_ctx* c, int x0, int y0, int z0, int nx, int ny, int nz, 
 {
 	enter(c);
 	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_read_voxels: null context");
-	const long long dim = 1ll << c->depth;
-	const auto axis_ok = [dim](int o, int e) { return o >= 0 && e >= 1 && static_cast<long long>(o) + e <= dim; };
-	if (!axis_ok(x0, nx) || !axis_ok(y0, ny) || !axis_ok(z0, nz))
-		return ort_fail(c, ORT_ERR_INVALID, "ort_read_voxels: box origin (%d, %d, %d) extent (%d, %d, %d) is not inside the cube of %lld voxels a side",
-		                x0, y0, z0, nx, ny, nz, dim);
+	ort::QueryBox box;
+	int rc = voxel_box(c, "ort_read_voxels", x0, y0, z0, nx, ny, nz, 0, &box);
+	if (rc != ORT_OK) return rc;
 	if (!out) return ort_fail(c, ORT_ERR_INVALID, "ort_read_voxels: null buffer");
 	DeviceGuard g(c->device);
 	const bool out_dev = is_device_ptr(out);
 	if (out_dev && (reinterpret_cast<uintptr_t>(out) & 3u))
 		return ort_fail(c, ORT_ERR_INVALID, "ort_read_voxels: a device output must be 4-byte aligned");
-	const ort::QueryBox box{ static_cast<uint32_t>(x0), static_cast<uint32_t>(y0), static_cast<uint32_t>(z0),
-	                         static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz) };
 	if (out_dev) return launch_read_voxels(c, box, out);                      // enqueue only
 
 	// host output: whole output rows (nx voxels) through the staging slots, at most kQueryStageBytes at a time -- whole
@@ -1491,8 +1555,7 @@ int ort_read_voxels(ort_ctx* c, int x0, int y0, int z0, int nx, int ny, int nz, 
 	const size_t chunk_rows = std::max<size_t>(1, kQueryStageBytes / row_bytes);
 	const size_t slice_rows = static_cast<size_t>(ny);
 	const size_t total_rows = slice_rows * static_cast<size_t>(nz);
-	int rc = ensure_dstage(c, 2 * align_up(std::min(chunk_rows, total_rows) * row_bytes, 256));
-	if (rc != ORT_OK) return rc;
+	if ((rc = ensure_dstage(c, 2 * align_up(std::min(chunk_rows, total_rows) * row_bytes, 256))) != ORT_OK) return rc;
 	for (size_t r0 = 0; r0 < total_rows;)
 	{
 		const uint32_t z = static_cast<uint32_t>(r0 / slice_rows), y = static_cast<uint32_t>(r0 % slice_rows);
@@ -1532,22 +1595,21 @@ namespace {
 
 constexpr int kPatchMaxExtent = 512;          // voxels per axis of one patch: bounds its scratch and reserved rows
 
+inline ort::PatchIndex patch_index(const ort_ctx* c, int l) { return ort::PatchIndex{ c->d_pidx[l], static_cast<uint32_t>(c->pidx_cap[l] - 1) }; }
+
 // Room in the mirror for ids up to `rows` (the caller clips that to kIdMask).  Growing reallocates the array every launch
 // in flight reads, as ort_upload_full does, so it waits for the whole device first; rows 1 .. n_nodes are kept.
 int patch_reserve(ort_ctx* c, size_t rows, size_t bound)
 {
 	if (rows <= c->cap_nodes) return ORT_OK;
 	const size_t n = c->n_nodes;
-	const size_t want = std::min<size_t>(n + n / 4 + 4096 + bound, ort::kIdMask);
-	ORT_CUDA(c, cudaDeviceSynchronize());
 	NewMirror fresh;
-	ORT_CUDA(c, cudaMalloc(&fresh.p, want * 32));
+	fresh.cap = mirror_capacity(n, bound);
+	ORT_CUDA(c, cudaDeviceSynchronize());
+	ORT_CUDA(c, cudaMalloc(&fresh.p, fresh.cap * 32));
 	if (n) ORT_CUDA(c, cudaMemcpyAsync(fresh.p, c->d_nodes, n * 32, cudaMemcpyDeviceToDevice, c->stream));
 	ORT_CUDA(c, cudaStreamSynchronize(c->stream));
-	cudaFree(c->d_nodes);
-	c->d_nodes = fresh.p;
-	c->cap_nodes = static_cast<uint32_t>(want);
-	fresh.p = nullptr;
+	fresh.install(c);
 	return ORT_OK;
 }
 
@@ -1566,35 +1628,24 @@ int patch_index_table(ort_ctx* c, int l, size_t cap)
 	return ORT_OK;
 }
 
-// The patch index of the current rows: the ids reachable at each level from the root (ort_write_voxels' first step),
-// each level's table sized for them plus `cells[l]` appended rows at a load of at most 1/2.
+// The patch index of the current rows: the ids reachable at each level from the root, each level's table sized for them
+// plus `cells[l]` appended rows.
 int patch_index_build(ort_ctx* c, const ort::WriteDag& g, uint32_t old_root, const size_t* cells)
 {
 	const int D = c->depth;
 	cudaStream_t st = c->stream;
 	BuildTemps tmp;
 	TopDown td;
-	uint32_t* ids[kWriteMaxDepth + 2] = {};
-	size_t n[kWriteMaxDepth + 2] = {};
-	if (old_root)
-	{
-		ORT_CUDA(c, tmp.alloc(&ids[1], 1));
-		ORT_CUDA(c, cudaMemcpyAsync(ids[1], &old_root, 4, cudaMemcpyHostToDevice, st));
-		n[1] = 1;
-		uint32_t* first = nullptr;
-		ORT_CUDA(c, tmp.alloc(&first, c->n_nodes));
-		int rc;
-		for (int l = 1; l < D && n[l]; ++l)
-			if ((rc = top_down_step(c, tmp, td, ort::OldSrc{ g }, ids[l], n[l], first, c->n_nodes, 0u, nullptr, &ids[l + 1], &n[l + 1])) != ORT_OK)
-				return rc;
-	}
+	uint32_t* ids[ort::kMaxDepth + 2] = {};
+	size_t n[ort::kMaxDepth + 2] = {};
+	int rc = reachable_ids(c, tmp, td, g, old_root, ids, n);
+	if (rc != ORT_OK) return rc;
 	for (int l = 1; l <= D; ++l)
 	{
-		const int rc = patch_index_table(c, l, pow2_at_least(2 * (n[l] + cells[l])));
-		if (rc != ORT_OK) return rc;
+		if ((rc = patch_index_table(c, l, table_cap(n[l] + cells[l]))) != ORT_OK) return rc;
 		if (n[l])
 		{
-			ort::patch_index_build_kernel<<<blocks_for(n[l]), 256, 0, st>>>(ids[l], n[l], ort::PatchIndex{ c->d_pidx[l], static_cast<uint32_t>(c->pidx_cap[l] - 1) }, g.nodes_m1);
+			ort::patch_index_build_kernel<<<blocks_for(n[l]), 256, 0, st>>>(ids[l], n[l], patch_index(c, l), g.nodes_m1);
 			++c->launches;
 		}
 		c->pidx_rows[l] = n[l];
@@ -1612,7 +1663,7 @@ int patch_index_grow(ort_ctx* c, const uint32_t* nodes_m1, const size_t* cells)
 	{
 		const size_t need = c->pidx_rows[l] + cells[l];
 		if (4 * need <= 3 * c->pidx_cap[l]) continue;
-		const size_t cap = pow2_at_least(2 * need);
+		const size_t cap = table_cap(need);
 		uint32_t* t = nullptr;
 		ORT_CUDA(c, cudaMalloc(&t, cap * 4));
 		const cudaError_t e = cudaMemsetAsync(t, 0xFF, cap * 4, c->stream);
@@ -1631,8 +1682,7 @@ int patch_index_grow(ort_ctx* c, const uint32_t* nodes_m1, const size_t* cells)
 	return ORT_OK;
 }
 
-int patch_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* voxels, int elem_bytes, uint32_t nx, uint32_t ny, uint32_t nz,
-                 size_t* n_added)
+int patch_voxels(ort_ctx* c, const ort::QueryBox& b, const void* voxels, int elem_bytes, size_t* n_added)
 {
 	const int D = c->depth;
 	cudaStream_t st = c->stream;
@@ -1640,40 +1690,26 @@ int patch_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* 
 	int rc = voxel_source_kind(c, "ort_patch_voxels", voxels, elem_bytes, &dev);
 	if (rc != ORT_OK) return rc;
 
-	// R_l: the cells of level l the box cuts (origin ro, extent re); their count bounds the rows level l appends
-	uint32_t ro[kWriteMaxDepth + 2][3] = {}, re[kWriteMaxDepth + 2][3] = {};
-	size_t cells[kWriteMaxDepth + 2] = {}, bound = 0, max_cells = 0, max_cap = 0;
-	const uint32_t b0[3] = { x0, y0, z0 }, b1[3] = { x0 + nx - 1, y0 + ny - 1, z0 + nz - 1 };
-	for (int l = 1; l <= D; ++l)
-	{
-		for (int a = 0; a < 3; ++a)
-		{
-			ro[l][a] = b0[a] >> (D - l + 1);
-			re[l][a] = (b1[a] >> (D - l + 1)) - ro[l][a] + 1;
-		}
-		cells[l] = static_cast<size_t>(re[l][0]) * re[l][1] * re[l][2];
-		bound += cells[l];
-		max_cells = std::max(max_cells, cells[l]);
-		max_cap = std::max(max_cap, pow2_at_least(2 * cells[l]));
-	}
+	// R_l: the cells of level l the box cuts; their count bounds the rows level l appends
+	const BoxCells box(D, b);
 
 	// rows for every id the patch may append (past the id limit the call is refused, so those are never needed)
 	const uint32_t n_old = c->n_nodes;
-	if ((rc = patch_reserve(c, std::min<size_t>(static_cast<size_t>(n_old) + bound, ort::kIdMask), bound)) != ORT_OK) return rc;
-	const ort::WriteDag g{ c->d_nodes - 8, c->has_root ? n_old + 1 : 0u };
-	const uint32_t old_root = c->has_root && c->root - 1u < g.lim - 1u ? c->root : 0u;
+	if ((rc = patch_reserve(c, std::min<size_t>(static_cast<size_t>(n_old) + box.sum, ort::kIdMask), box.sum)) != ORT_OK) return rc;
+	uint32_t old_root = 0;
+	const ort::WriteDag g = old_dag(c, &old_root);
 	if (!c->pidx_valid)
-		rc = patch_index_build(c, g, old_root, cells);
+		rc = patch_index_build(c, g, old_root, box.cells);
 	else
-		rc = patch_index_grow(c, g.nodes_m1, cells);
+		rc = patch_index_grow(c, g.nodes_m1, box.cells);
 	if (rc != ORT_OK) return rc;
 
 	// scratch (words): first ids per level + root | non-empty counter | R_l's ids and old_at | local table + first
 	// occurrence | hits | flags and their scan
 	const auto words = [](size_t n) { return align_up(n, 64); };
-	const size_t w_state = words(D + 2), w_cnt = words(2), w_tf = words(2 * max_cap), w_hit = words(max_cells), w_flag = words(max_cells + 1);
-	size_t total = w_state + w_cnt + w_tf + w_hit + w_flag + words(ort::scan_scratch_words(max_cells + 1));
-	for (int l = 1; l <= D; ++l) total += 2 * words(cells[l]);
+	const size_t w_state = words(D + 2), w_cnt = words(2), w_tf = words(2 * table_cap(box.max)), w_hit = words(box.max), w_flag = words(box.max + 1);
+	size_t total = w_state + w_cnt + w_tf + w_hit + w_flag + words(ort::scan_scratch_words(box.max + 1));
+	for (int l = 1; l <= D; ++l) total += 2 * words(box.cells[l]);
 	if (total * 4 > c->d_patch_bytes)
 	{
 		cudaFree(c->d_patch);                   // (waits for the previous patch)
@@ -1687,13 +1723,12 @@ int patch_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* 
 	w += w_state;
 	unsigned long long* d_cnt = reinterpret_cast<unsigned long long*>(w);
 	w += w_cnt;
-	ort::WriteGrid R[kWriteMaxDepth + 2] = {};
+	ort::WriteGrid R[ort::kMaxDepth + 2] = {};
 	for (int l = 1; l <= D; ++l)
 	{
-		R[l].ox = ro[l][0]; R[l].oy = ro[l][1]; R[l].oz = ro[l][2];
-		R[l].gx = re[l][0]; R[l].gy = re[l][1]; R[l].gz = re[l][2];
-		R[l].ids = w; w += words(cells[l]);
-		R[l].old_at = w; w += words(cells[l]);
+		R[l] = box.R[l];
+		R[l].ids = w; w += words(box.cells[l]);
+		R[l].old_at = w; w += words(box.cells[l]);
 	}
 	uint32_t* tf = w; w += w_tf;
 	uint32_t* hit = w; w += w_hit;
@@ -1705,52 +1740,51 @@ int patch_voxels(ort_ctx* c, uint32_t x0, uint32_t y0, uint32_t z0, const void* 
 	int slot = -1;
 	if (!dev)
 	{
-		const size_t bytes = static_cast<size_t>(nx) * ny * nz * elem_bytes;
+		const size_t bytes = static_cast<size_t>(b.nx) * b.ny * b.nz * elem_bytes;
 		if ((rc = ensure_dstage(c, 2 * align_up(bytes, 256))) != ORT_OK) return rc;
 		char* base = nullptr;
 		slot = query_slot(c, &base);
 		ORT_CUDA(c, cudaMemcpyAsync(base, voxels, bytes, cudaMemcpyHostToDevice, st));
 		src = base;
 	}
-	const ort::BuildInput in{ src, elem_bytes, nx, ny, nz };
+	const ort::BuildInput in{ src, elem_bytes, b.nx, b.ny, b.nz };
 
 	// old nodes under R_l, top-down
 	ort::patch_begin_kernel<<<1, 1, 0, st>>>(R[1].old_at, old_root, state + D, n_old);
 	++c->launches;
 	for (int l = 2; l <= D; ++l)
 	{
-		ort::write_old_at_kernel<<<blocks_for(cells[l]), 256, 0, st>>>(R[l - 1], R[l], g);
+		ort::write_old_at_kernel<<<blocks_for(box.cells[l]), 256, 0, st>>>(R[l - 1], R[l], g);
 		++c->launches;
 	}
 	// bottom-up: intern R_l, probe the index with each new content's first cell, append the misses
 	for (int l = D; l >= 1; --l)
 	{
-		const ort::PatchSrc s{ l == D, in, x0, y0, z0, R[l], l == D ? R[l] : R[l + 1], g };
-		const size_t cap = pow2_at_least(2 * cells[l]);
+		const size_t cells = box.cells[l], cap = table_cap(cells);
+		const ort::PatchSrc s{ l == D, in, b.x0, b.y0, b.z0, R[l], l == D ? R[l] : R[l + 1], g };
 		ORT_CUDA(c, cudaMemsetAsync(tf, 0xFF, 2 * cap * 4, st));
-		ort::build_insert_kernel<<<blocks_for(cells[l]), 256, 0, st>>>(s, tf, static_cast<uint32_t>(cap - 1), d_cnt);
-		ort::patch_first_kernel<<<blocks_for(cells[l]), 256, 0, st>>>(R[l].ids, cells[l], tf + cap);
-		ort::patch_probe_kernel<<<blocks_for(cells[l] + 1), 256, 0, st>>>(s, tf + cap, ort::PatchIndex{ c->d_pidx[l], static_cast<uint32_t>(c->pidx_cap[l] - 1) }, hit, flag);
+		ort::build_insert_kernel<<<blocks_for(cells), 256, 0, st>>>(s, tf, static_cast<uint32_t>(cap - 1), d_cnt);
+		ort::patch_first_kernel<<<blocks_for(cells), 256, 0, st>>>(R[l].ids, cells, tf + cap);
+		ort::patch_probe_kernel<<<blocks_for(cells + 1), 256, 0, st>>>(s, tf + cap, patch_index(c, l), hit, flag);
 		c->launches += 3;
-		ort::scan_exclusive(flag, cells[l] + 1, scan, st, c->launches);
-		ort::patch_rows_kernel<<<blocks_for(cells[l]), 256, 0, st>>>(s, tf + cap, hit, flag, state + l, c->cap_nodes, c->d_nodes - 8,
-		                                                            l == 1 ? state + D + 1 : nullptr);
+		ort::scan_exclusive(flag, cells + 1, scan, st, c->launches);
+		ort::patch_rows_kernel<<<blocks_for(cells), 256, 0, st>>>(s, tf + cap, hit, flag, state + l, c->cap_nodes, c->d_nodes - 8,
+		                                                         l == 1 ? state + D + 1 : nullptr);
 		++c->launches;
 		ORT_CUDA(c, cudaGetLastError());
 	}
 	// the appended rows enter the index (unless the call is refused below)
 	ort::PatchIndexSet set{};
 	set.depth = D;
-	for (int l = 1; l <= D; ++l) set.ix[l] = ort::PatchIndex{ c->d_pidx[l], static_cast<uint32_t>(c->pidx_cap[l] - 1) };
-	ort::patch_index_append_kernel<<<blocks_for(bound), 256, 0, st>>>(state, set, g.nodes_m1);
+	for (int l = 1; l <= D; ++l) set.ix[l] = patch_index(c, l);
+	ort::patch_index_append_kernel<<<blocks_for(box.sum), 256, 0, st>>>(state, set, g.nodes_m1);
 	++c->launches;
 	ORT_CUDA(c, cudaGetLastError());
 	if (slot >= 0 && (rc = query_slot_done(c, slot, nullptr, nullptr, 0)) != ORT_OK) return rc;
 
 	// the one readback: first ids per level, root
-	uint32_t h[kWriteMaxDepth + 2] = {};
-	ORT_CUDA(c, cudaMemcpyAsync(h, state, (D + 2) * 4, cudaMemcpyDeviceToHost, st));
-	ORT_CUDA(c, cudaStreamSynchronize(st));
+	uint32_t h[ort::kMaxDepth + 2] = {};
+	if ((rc = read_back(c, h, state, (D + 2) * 4)) != ORT_OK) return rc;
 	const uint32_t n_new = h[0] - 1;
 	if (n_new > ort::kIdMask)
 		return ort_fail(c, ORT_ERR_CAPACITY, "ort_patch_voxels: the patch would append ids past the %u compact ids allow (%u rows before it)", ort::kIdMask, n_old);
@@ -1770,22 +1804,11 @@ extern "C" {
 
 int ort_patch_voxels(ort_ctx* c, int x0, int y0, int z0, const void* voxels, int elem_bytes, int nx, int ny, int nz, size_t* n_added)
 {
-	enter(c);
-	if (!c) return ort_fail(c, ORT_ERR_INVALID, "ort_patch_voxels: null context");
-	if (c->index_base != 1)
-		return ort_fail(c, ORT_ERR_INVALID, "ort_patch_voxels: the context holds an och::octree pool, not a DAG");
-	const long long dim = 1ll << c->depth;
-	const auto axis_ok = [dim](int o, int e) { return o >= 0 && e >= 1 && e <= kPatchMaxExtent && static_cast<long long>(o) + e <= dim; };
-	if (!axis_ok(x0, nx) || !axis_ok(y0, ny) || !axis_ok(z0, nz))
-		return ort_fail(c, ORT_ERR_INVALID, "ort_patch_voxels: box origin (%d, %d, %d) extent (%d, %d, %d) is not inside the cube of %lld voxels a side "
-		                "with 1..%d per axis", x0, y0, z0, nx, ny, nz, dim, kPatchMaxExtent);
-	if (!voxels || (elem_bytes != 1 && elem_bytes != 4))
-		return ort_fail(c, ORT_ERR_INVALID, "ort_patch_voxels: bad arguments (voxels=%p elem_bytes=%d)", voxels, elem_bytes);
-	DeviceGuard g(c->device);
-	const int rc = patch_voxels(c, static_cast<uint32_t>(x0), static_cast<uint32_t>(y0), static_cast<uint32_t>(z0), voxels, elem_bytes,
-	                            static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz), n_added);
-	if (rc != ORT_OK) cudaGetLastError();       // (an allocation that failed leaves its error behind for the next check)
-	return rc;
+	return mirror_call(c, "ort_patch_voxels", voxels, elem_bytes, [&] {
+		ort::QueryBox box;
+		const int rc = edit_box(c, "ort_patch_voxels", x0, y0, z0, nx, ny, nz, kPatchMaxExtent, &box);
+		return rc != ORT_OK ? rc : patch_voxels(c, box, voxels, elem_bytes, n_added);
+	});
 }
 
 }  // extern "C"

@@ -96,11 +96,9 @@ __global__ void patch_index_rehash_kernel(const uint32_t* old_table, size_t old_
 	if (e != kBuildEmpty) patch_index_insert(ix, nodes_m1, e);
 }
 
-constexpr int kPatchMaxDepth = 16;
-
 struct PatchIndexSet
 {
-	PatchIndex ix[kPatchMaxDepth + 1];          // level 1 .. depth
+	PatchIndex ix[kMaxDepth + 1];               // level 1 .. depth
 	int depth;
 };
 
